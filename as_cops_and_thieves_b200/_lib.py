@@ -13,9 +13,10 @@ import numpy as np
 
 from . import build as _build
 
-CAT_ABI_VERSION = 5
+CAT_ABI_VERSION = 6
 CAT_MAX_AGENTS = 8
 CAT_MAX_RAYS = 128
+CAT_MAX_MAPS = 8
 CAT_WALL_SLOTS = 4
 CAT_NEAR_SLOTS = 4
 
@@ -84,7 +85,8 @@ class CatStateView(C.Structure):
 
 #: every symbol ``include/cat_b200.h`` declares
 EXPORTS = (
-    "cat_abi_version", "cat_last_error", "cat_env_create", "cat_env_destroy", "cat_env_info",
+    "cat_abi_version", "cat_last_error", "cat_env_create", "cat_env_create_multi", "cat_env_destroy", "cat_env_info",
+    "cat_env_map_info",
     "cat_env_record_layout", "cat_env_packed_record_layout", "cat_env_overflow_counts", "cat_ray_lists_host",
     "cat_env_set_seed", "cat_env_state_bytes", "cat_env_init_state", "cat_env_reset", "cat_env_step", "cat_env_step_host", "cat_env_observe",
     "cat_env_get_state", "cat_env_set_state", "cat_gae", "cat_adv_normalize",
@@ -115,8 +117,11 @@ def load():
     L.cat_last_error.restype = C.c_char_p
     L.cat_env_create.argtypes = [C.POINTER(CatMapDesc), C.POINTER(CatParams), C.c_int32, C.c_int64, C.c_int32,
                                  C.POINTER(C.c_void_p)]
+    L.cat_env_create_multi.argtypes = [C.POINTER(CatMapDesc), C.c_int32, C.POINTER(C.c_int32), C.POINTER(CatParams), C.c_int64,
+                                       C.c_int32, C.POINTER(C.c_void_p)]
     L.cat_env_destroy.argtypes = [C.c_void_p]
     L.cat_env_info.argtypes = [C.c_void_p, C.POINTER(CatEnvInfo)]
+    L.cat_env_map_info.argtypes = [C.c_void_p, C.c_int32, C.POINTER(CatEnvInfo)]
     L.cat_env_set_seed.argtypes = [C.c_void_p, C.c_uint64]
     L.cat_env_state_bytes.restype = C.c_size_t
     L.cat_env_state_bytes.argtypes = [C.c_void_p]

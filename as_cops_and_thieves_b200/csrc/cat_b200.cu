@@ -105,24 +105,33 @@ static void ray_lists_release(SharedRayLists* sh) {
   delete sh;
 }
 
+// One map of an environment: its staged blob, its view lists and its share of the (cell, ray) lists.  Map m owns the
+// worlds [world_begin, world_begin + n_worlds) of the environment.
+struct EnvMap {
+  unsigned char* blob_dev = nullptr;
+  int blob_bytes = 0;
+  int32_t* view_off_dev = nullptr;
+  uint16_t* view_edges_dev = nullptr;
+  SharedRayLists* ray_lists = nullptr;   // shared with the other environments of this map on this device
+  int world_begin = 0, n_worlds = 0;
+  int n_hulls = 0, n_edges = 0;
+};
+
 struct CatEnv {
   std::vector<std::pair<int, LaunchShape>> shape_cache;   // launch shape per world count (the chunked host path asks every step)
   WorldKernel kernel = nullptr;        // every output the ABI offers
   WorldKernel kernel_record = nullptr; // record output only (launches that ask for nothing else)
   int device = 0;
   int n_worlds = 0;
-  unsigned char* blob_dev = nullptr;
-  int32_t* view_off_dev = nullptr;
-  uint16_t* view_edges_dev = nullptr;
-  SharedRayLists* ray_lists = nullptr;   // shared with the other environments of this map on this device
+  std::vector<EnvMap> maps;            // 1 .. CAT_MAX_MAPS, in world order
   unsigned long long* overflow_dev = nullptr;
   CatRecordLayout rec{}, rec_packed{};
-  KParams kp{};
+  KParams kp{};                        // with the map table of a full-environment launch
   CatEnvInfo info{};
   int smem_bytes = 0;
   int grid = 0;
   int threads = kThreads;
-  int blob_bytes = 0, max_optin = 0, n_sm = 0;
+  int blob_bytes = 0, max_optin = 0, n_sm = 0;   // blob_bytes: the largest of the maps' blobs
   // chunked host path: a second stream for the device-to-host copies and one event per chunk
   cudaStream_t copy_stream = nullptr;
   std::vector<cudaEvent_t> chunk_events;
@@ -130,15 +139,20 @@ struct CatEnv {
 };
 
 // the kernel instantiation an environment runs (fixed at creation): agents / rays as compile-time constants for the
-// shipped shape, the any-shape instantiation otherwise (CAT_GENERIC_KERNEL=1 at creation forces it: test knob)
-static WorldKernel pick_world_kernel(int A, int R, bool lists, bool extras) {
+// shipped shape, the any-shape instantiation otherwise (CAT_GENERIC_KERNEL=1 at creation forces it: test knob); the
+// mixed-map instantiations (multi) for an environment of several maps
+template <bool TM>
+static WorldKernel pick_world_kernel_t(int A, int R, bool lists, bool extras) {
   const char* e = getenv("CAT_GENERIC_KERNEL");
   const bool generic = e && e[0] == '1';
   if (A == 3 && R == 90 && !generic) {
-    if (lists) return extras ? cat_world_kernel<3, 90, true, true> : cat_world_kernel<3, 90, true, false>;
-    return cat_world_kernel<3, 90, false, true>;
+    if (lists) return extras ? cat_world_kernel<3, 90, true, true, TM> : cat_world_kernel<3, 90, true, false, TM>;
+    return cat_world_kernel<3, 90, false, true, TM>;
   }
-  return cat_world_kernel<0, 0, false, true>;
+  return cat_world_kernel<0, 0, false, true, TM>;
+}
+static WorldKernel pick_world_kernel(int A, int R, bool lists, bool extras, bool multi) {
+  return multi ? pick_world_kernel_t<true>(A, R, lists, extras) : pick_world_kernel_t<false>(A, R, lists, extras);
 }
 
 static bool pick_launch_shape(CatEnv* env, int n_worlds, LaunchShape* out) {
@@ -165,6 +179,47 @@ static bool pick_launch_shape(CatEnv* env, int n_worlds, LaunchShape* out) {
   if (const char* e = getenv("CAT_MAX_GRID")) { const int v = atoi(e); if (v >= 1 && v < out->grid) out->grid = v; }   // tuning knob
   if (best_score >= 0 && env->shape_cache.size() < 64) env->shape_cache.emplace_back(n_worlds, *out);
   return best_score >= 0;
+}
+
+// Fill the map table of a launch that steps the worlds [w0, w1) of the environment with `grid` CTAs of `wpc` warps and
+// return the grid to launch.  The CTAs are split between the maps with worlds in the range: a one-wave grid (a warp for
+// every world) gives each map the CTAs its worlds need, so every map's share stays one wave; a persistent grid is split
+// in proportion to the worlds, at least one CTA per map (raised to one CTA per map if it is smaller).  With one map the
+// grid is returned unchanged.
+static int fill_map_table(const CatEnv* env, KParams& k, int w0, int w1, int grid, int wpc) {
+  int len[CAT_MAX_MAPS], ctas[CAT_MAX_MAPS];
+  int n = 0;
+  for (const EnvMap& m : env->maps) {
+    const int b = std::max(w0, m.world_begin), e = std::min(w1, m.world_begin + m.n_worlds);
+    if (b >= e) continue;
+    MapSlice& sl = k.maps[n];
+    sl.blob = m.blob_dev; sl.blob_bytes = m.blob_bytes; sl.world_begin = b; sl.world_end = e;
+    len[n++] = e - b;
+  }
+  k.n_maps = n;
+  k.world_begin = w0; k.world_end = w1;
+  const long long total = (long long)w1 - w0;
+  if ((long long)grid * wpc >= total) {
+    grid = 0;
+    for (int i = 0; i < n; ++i) { ctas[i] = (len[i] + wpc - 1) / wpc; grid += ctas[i]; }
+  } else {
+    grid = std::max(grid, n);
+    int used = 0;
+    for (int i = 0; i < n; ++i) { ctas[i] = std::max(1, (int)((long long)grid * len[i] / total)); used += ctas[i]; }
+    while (used > grid) {          // the minimum of one CTA pushed the sum over: take from the map with the most
+      int j = 0;
+      for (int i = 1; i < n; ++i) if (ctas[i] > ctas[j]) j = i;
+      --ctas[j]; --used;
+    }
+    while (used < grid) {          // rounding left CTAs over: give each to the map with the most worlds per CTA
+      int j = 0;
+      for (int i = 1; i < n; ++i) if ((long long)len[i] * ctas[j] > (long long)len[j] * ctas[i]) j = i;
+      ++ctas[j]; ++used;
+    }
+  }
+  int c = 0;
+  for (int i = 0; i < n; ++i) { k.maps[i].cta_begin = c; c += ctas[i]; }
+  return grid;
 }
 
 // Launch with programmatic stream serialisation: the kernel's CTAs may be scheduled while the previous kernel in the
@@ -199,12 +254,9 @@ int cat_debug_stats(unsigned long long* out8, int reset) {
 int cat_abi_version(void) { return CAT_ABI_VERSION; }
 const char* cat_last_error(void) { return g_last_error.c_str(); }
 
-int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds, int64_t gid0, int32_t device,
-                   CatEnv** out) {
-  if (!map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
-  *out = nullptr;
+// Everything cat_env_create checks of one map, before any CUDA call (testable without a device).
+static int check_map(const CatMapDesc* map, const CatParams* pr) {
   const int A = map->n_cops + map->n_thieves, R = pr->n_rays, H = map->n_hulls, E = map->n_edges;
-  if (n_worlds < 1) return fail(CAT_ERR_INVALID, "n_worlds must be >= 1");
   if (map->n_cops < 1 || map->n_thieves < 1) return fail(CAT_ERR_INVALID, "need at least one cop and one thief");
   if (A > CAT_MAX_AGENTS) return fail(CAT_ERR_LIMIT, "too many agents (CAT_MAX_AGENTS)");
   if (R < 2 || R > CAT_MAX_RAYS) return fail(CAT_ERR_LIMIT, "n_rays out of range (2..CAT_MAX_RAYS)");
@@ -217,7 +269,14 @@ int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds,
   if (!(pr->dt > 0.0)) return fail(CAT_ERR_INVALID, "dt must be > 0");
   const int P = A * (A - 1) / 2;
   if (P > 32) return fail(CAT_ERR_LIMIT, "too many agent pairs for one warp");
+  return CAT_OK;
+}
 
+// The shared-memory blob of one map (BlobHeader + arrays).  The header's global-memory table pointers are left zero:
+// the caller fills them in once the tables are on the device.
+static std::vector<unsigned char> build_blob(const CatMapDesc* map, const CatParams* pr) {
+  const int A = map->n_cops + map->n_thieves, R = pr->n_rays, H = map->n_hulls, E = map->n_edges;
+  const int ncell = map->nx * map->ny;
   // ---- blob
   const int nreg = map->region_off[A];
   BlobHeader hd{};
@@ -306,6 +365,82 @@ int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds,
     for (int i = 0; i < 2 * A; ++i) ip[i] = (float)map->init_pos[i];
   }
 
+  return blob;
+}
+
+// The per-(cell, ray) candidate lists of one map on one device: found in the cache or built, uploaded and cached.
+static int acquire_ray_lists(const CatMapDesc* map, const CatParams* pr, int device, SharedRayLists** out) {
+  const int R = pr->n_rays, H = map->n_hulls, E = map->n_edges;
+  const double rsum = pr->wall_radius + pr->ray_radius;
+  // key: everything build_ray_lists reads
+  std::vector<unsigned char> key;
+  auto put = [&key](const void* p, size_t n) { const unsigned char* b = static_cast<const unsigned char*>(p); key.insert(key.end(), b, b + n); };
+  const char* knob_cells = getenv("CAT_RAY_LIST_CELLS");
+  const char* knob_min = getenv("CAT_RAY_LIST_MIN_CELL");
+  const double head[6] = {(double)device, (double)R, pr->ray_length, rsum, pr->ray_list_cell,
+                          (knob_cells ? atof(knob_cells) : 0.0) * 4096.0 + (knob_min ? atof(knob_min) : 0.0)};
+  put(head, sizeof(head));
+  put(&H, sizeof(H)); put(&E, sizeof(E));
+  put(map->hull_off, sizeof(int32_t) * (H + 1));
+  put(map->vert, sizeof(double) * 2 * E);
+  put(map->normal, sizeof(double) * 2 * E);
+  put(map->hull_bb, sizeof(double) * 4 * H);
+  std::lock_guard<std::mutex> lock(g_ray_lists_mutex);
+  SharedRayLists* sh = nullptr;
+  for (SharedRayLists* c : g_ray_lists)
+    if (c->key == key) { sh = c; break; }
+  if (!sh) {
+    RayLists rl;
+    build_ray_lists(map, R, pr->ray_length, rsum, pr->ray_list_cell, &rl);
+    sh = new SharedRayLists();
+    sh->key.swap(key);
+    sh->g = rl.g; sh->slot_words = rl.slots.size(); sh->ovf_words = rl.ovf.size();
+    cudaError_t e1 = cudaMalloc(&sh->slots_dev, rl.slots.size() * 4);
+    cudaError_t e2 = e1 == cudaSuccess ? cudaMalloc(&sh->ovf_dev, rl.ovf.size() * 4) : e1;
+    if (e2 == cudaSuccess) e2 = cudaMemcpy(sh->slots_dev, rl.slots.data(), rl.slots.size() * 4, cudaMemcpyHostToDevice);
+    if (e2 == cudaSuccess) e2 = cudaMemcpy(sh->ovf_dev, rl.ovf.data(), rl.ovf.size() * 4, cudaMemcpyHostToDevice);
+    if (e2 != cudaSuccess) {
+      if (sh->slots_dev) cudaFree(sh->slots_dev);
+      if (sh->ovf_dev) cudaFree(sh->ovf_dev);
+      delete sh;
+      return fail(CAT_ERR_CUDA, std::string("ray lists: ") + cudaGetErrorString(e2));
+    }
+    g_ray_lists.push_back(sh);
+  }
+  ++sh->refs;
+  *out = sh;
+  return CAT_OK;
+}
+
+int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds, int64_t gid0, int32_t device,
+                   CatEnv** out) {
+  if (!map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
+  return cat_env_create_multi(map, 1, &n_worlds, pr, gid0, device, out);
+}
+
+int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map, const CatParams* pr,
+                         int64_t gid0, int32_t device, CatEnv** out) {
+  if (!maps || !worlds_per_map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
+  *out = nullptr;
+  if (n_maps < 1) return fail(CAT_ERR_INVALID, "n_maps must be >= 1");
+  if (n_maps > CAT_MAX_MAPS) return fail(CAT_ERR_LIMIT, "too many maps (CAT_MAX_MAPS)");
+  long long total = 0;
+  for (int m = 0; m < n_maps; ++m) {
+    if (worlds_per_map[m] < 1) return fail(CAT_ERR_INVALID, "n_worlds must be >= 1");
+    const int rc = check_map(&maps[m], pr);
+    if (rc != CAT_OK) return rc;
+    if (maps[m].n_cops != maps[0].n_cops || maps[m].n_thieves != maps[0].n_thieves)
+      return fail(CAT_ERR_INVALID, "every map of an environment needs the same numbers of cops and thieves");
+    total += worlds_per_map[m];
+  }
+  if (total > 0x7FFFFFFFll) return fail(CAT_ERR_LIMIT, "too many worlds");
+  const CatMapDesc* map = &maps[0];   // agents, rays and constants are the same for every map
+  const int n_worlds = (int)total;
+  const int A = map->n_cops + map->n_thieves, R = pr->n_rays;
+  const int P = A * (A - 1) / 2;
+  std::vector<std::vector<unsigned char>> blobs;
+  for (int m = 0; m < n_maps; ++m) blobs.push_back(build_blob(&maps[m], pr));
+
   CatEnv* env = new CatEnv();
   env->device = device;
   env->n_worlds = n_worlds;
@@ -317,81 +452,68 @@ int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds,
     cudaError_t _e = (expr);                                                                                \
     if (_e != cudaSuccess) { cat_env_destroy(env); return fail(CAT_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(_e)); } \
   } while (0)
-  CREATE_TRY(cudaMalloc(&env->blob_dev, blob_bytes), "cudaMalloc(map blob)");
-  CREATE_TRY(cudaMemcpy(env->blob_dev, blob.data(), blob_bytes, cudaMemcpyHostToDevice), "cudaMemcpy(map blob)");
   CREATE_TRY(cudaMalloc(&env->overflow_dev, 2 * sizeof(unsigned long long)), "cudaMalloc(overflow counters)");
   CREATE_TRY(cudaMemset(env->overflow_dev, 0, 2 * sizeof(unsigned long long)), "cudaMemset(overflow counters)");
+  env->maps.resize(n_maps);
+  CatEnvInfo& inf = env->info;
+  int64_t ray_list_bytes = 0;
+  for (int m = 0, w0 = 0; m < n_maps; w0 += worlds_per_map[m], ++m) {
+    const CatMapDesc* md = &maps[m];
+    EnvMap& em = env->maps[m];
+    em.world_begin = w0; em.n_worlds = worlds_per_map[m];
+    em.n_hulls = md->n_hulls; em.n_edges = md->n_edges;
+    std::vector<unsigned char>& blob = blobs[m];
+    BlobHeader hd;
+    memcpy(&hd, blob.data(), sizeof(hd));
+    const int E = md->n_edges, ncell = md->nx * md->ny;
+    // per-cell candidate lists (optional; valid only if they were built for at least this sensor range)
+    // Worth it only when the full scan is long: the lists live in global memory (two dependent loads per sweep,
+    // cold after an L2 flush), and a map of a few dozen edges is scanned in one or two batches anyway.
+    if (md->view_cell_off && md->view_cell_edges && E >= 96 &&
+        md->view_range >= pr->ray_length + pr->wall_radius + pr->ray_radius) {
+      const int n_list = md->view_cell_off[ncell];
+      std::vector<uint16_t> ve((size_t)(n_list > 0 ? n_list : 1));
+      for (int i = 0; i < n_list; ++i) ve[i] = (uint16_t)md->view_cell_edges[i];
+      CREATE_TRY(cudaMalloc(&em.view_off_dev, sizeof(int32_t) * (ncell + 1)), "cudaMalloc(view lists)");
+      CREATE_TRY(cudaMalloc(&em.view_edges_dev, sizeof(uint16_t) * ve.size()), "cudaMalloc(view lists)");
+      CREATE_TRY(cudaMemcpy(em.view_off_dev, md->view_cell_off, sizeof(int32_t) * (ncell + 1), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
+      CREATE_TRY(cudaMemcpy(em.view_edges_dev, ve.data(), sizeof(uint16_t) * ve.size(), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
+      hd.view_off = em.view_off_dev; hd.view_edges = em.view_edges_dev;
+    }
+    // per-(cell, ray) candidate lists of the sensor sweep (ray_lists.h), built from the map description
+    if (!(pr->ray_list_cell < 0.0)) {
+      const int rc = acquire_ray_lists(md, pr, device, &em.ray_lists);
+      if (rc != CAT_OK) { cat_env_destroy(env); return rc; }
+      const SharedRayLists* sh = em.ray_lists;
+      hd.ray_slots = sh->slots_dev; hd.ray_ovf = sh->ovf_dev;
+      hd.ray_slot_count = (unsigned)(sh->slot_words / 4); hd.ray_ovf_words = (unsigned)sh->ovf_words;
+      hd.rg_x0 = sh->g.x0; hd.rg_y0 = sh->g.y0; hd.rg_inv_cell = sh->g.inv_cell; hd.rg_nx = sh->g.nx; hd.rg_ny = sh->g.ny;
+      ray_list_bytes += (int64_t)(sh->slot_words + sh->ovf_words) * 4;
+    }
+    memcpy(blob.data(), &hd, sizeof(hd));
+    em.blob_bytes = (int)blob.size();
+    CREATE_TRY(cudaMalloc(&em.blob_dev, em.blob_bytes), "cudaMalloc(map blob)");
+    CREATE_TRY(cudaMemcpy(em.blob_dev, blob.data(), em.blob_bytes, cudaMemcpyHostToDevice), "cudaMemcpy(map blob)");
+    env->blob_bytes = std::max(env->blob_bytes, em.blob_bytes);
+  }
 
   KParams& k = env->kp;
-  k.blob = env->blob_dev; k.blob_bytes = blob_bytes;
-  // per-cell candidate lists (optional; valid only if they were built for at least this sensor range)
-  // Worth it only when the full scan is long: the lists live in global memory (two dependent loads per sweep,
-  // cold after an L2 flush), and a map of a few dozen edges is scanned in one or two batches anyway.
-  if (map->view_cell_off && map->view_cell_edges && E >= 96 &&
-      map->view_range >= pr->ray_length + pr->wall_radius + pr->ray_radius) {
-    const int n_list = map->view_cell_off[ncell];
-    std::vector<uint16_t> ve((size_t)(n_list > 0 ? n_list : 1));
-    for (int i = 0; i < n_list; ++i) ve[i] = (uint16_t)map->view_cell_edges[i];
-    CREATE_TRY(cudaMalloc(&env->view_off_dev, sizeof(int32_t) * (ncell + 1)), "cudaMalloc(view lists)");
-    CREATE_TRY(cudaMalloc(&env->view_edges_dev, sizeof(uint16_t) * ve.size()), "cudaMalloc(view lists)");
-    CREATE_TRY(cudaMemcpy(env->view_off_dev, map->view_cell_off, sizeof(int32_t) * (ncell + 1), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
-    CREATE_TRY(cudaMemcpy(env->view_edges_dev, ve.data(), sizeof(uint16_t) * ve.size(), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
-    k.view_off = env->view_off_dev; k.view_edges = env->view_edges_dev;
+  {   // map 0's values: what a single-map launch reads (a mixed-map launch reads each map's from its blob header)
+    const EnvMap& em = env->maps[0];
+    k.blob = em.blob_dev; k.blob_bytes = em.blob_bytes;
+    k.view_off = em.view_off_dev; k.view_edges = em.view_edges_dev;
+    if (const SharedRayLists* sh = em.ray_lists) {
+      k.ray_slots = sh->slots_dev; k.ray_ovf = sh->ovf_dev;
+      k.ray_slot_count = (unsigned)(sh->slot_words / 4); k.ray_ovf_words = (unsigned)sh->ovf_words;
+      k.rg_x0 = sh->g.x0; k.rg_y0 = sh->g.y0; k.rg_inv_cell = sh->g.inv_cell; k.rg_nx = sh->g.nx; k.rg_ny = sh->g.ny;
+      inf.ray_list_cells = sh->g.nx * sh->g.ny; inf.ray_list_nx = sh->g.nx; inf.ray_list_ny = sh->g.ny; inf.ray_list_cell = sh->g.cell;
+    }
+    inf.ray_list_bytes = ray_list_bytes;
   }
   k.overflow = env->overflow_dev;
-  // per-(cell, ray) candidate lists of the sensor sweep (ray_lists.h), built here from the map description
-  CatEnvInfo& inf = env->info;
-  if (!(pr->ray_list_cell < 0.0)) {
-    const double rsum = pr->wall_radius + pr->ray_radius;
-    // key: everything build_ray_lists reads
-    std::vector<unsigned char> key;
-    auto put = [&key](const void* p, size_t n) { const unsigned char* b = static_cast<const unsigned char*>(p); key.insert(key.end(), b, b + n); };
-    const char* knob_cells = getenv("CAT_RAY_LIST_CELLS");
-    const char* knob_min = getenv("CAT_RAY_LIST_MIN_CELL");
-    const double head[6] = {(double)device, (double)R, pr->ray_length, rsum, pr->ray_list_cell,
-                            (knob_cells ? atof(knob_cells) : 0.0) * 4096.0 + (knob_min ? atof(knob_min) : 0.0)};
-    put(head, sizeof(head));
-    put(&H, sizeof(H)); put(&E, sizeof(E));
-    put(map->hull_off, sizeof(int32_t) * (H + 1));
-    put(map->vert, sizeof(double) * 2 * E);
-    put(map->normal, sizeof(double) * 2 * E);
-    put(map->hull_bb, sizeof(double) * 4 * H);
-    SharedRayLists* sh = nullptr;
-    {
-      std::lock_guard<std::mutex> lock(g_ray_lists_mutex);
-      for (SharedRayLists* c : g_ray_lists)
-        if (c->key == key) { sh = c; break; }
-      if (!sh) {
-        RayLists rl;
-        build_ray_lists(map, R, pr->ray_length, rsum, pr->ray_list_cell, &rl);
-        sh = new SharedRayLists();
-        sh->key.swap(key);
-        sh->g = rl.g; sh->slot_words = rl.slots.size(); sh->ovf_words = rl.ovf.size();
-        cudaError_t e1 = cudaMalloc(&sh->slots_dev, rl.slots.size() * 4);
-        cudaError_t e2 = e1 == cudaSuccess ? cudaMalloc(&sh->ovf_dev, rl.ovf.size() * 4) : e1;
-        if (e2 == cudaSuccess) e2 = cudaMemcpy(sh->slots_dev, rl.slots.data(), rl.slots.size() * 4, cudaMemcpyHostToDevice);
-        if (e2 == cudaSuccess) e2 = cudaMemcpy(sh->ovf_dev, rl.ovf.data(), rl.ovf.size() * 4, cudaMemcpyHostToDevice);
-        if (e2 != cudaSuccess) {
-          if (sh->slots_dev) cudaFree(sh->slots_dev);
-          if (sh->ovf_dev) cudaFree(sh->ovf_dev);
-          delete sh;
-          cat_env_destroy(env);
-          return fail(CAT_ERR_CUDA, std::string("ray lists: ") + cudaGetErrorString(e2));
-        }
-        g_ray_lists.push_back(sh);
-      }
-      ++sh->refs;
-    }
-    env->ray_lists = sh;
-    k.ray_slots = sh->slots_dev; k.ray_ovf = sh->ovf_dev;
-    k.ray_slot_count = (unsigned)(sh->slot_words / 4); k.ray_ovf_words = (unsigned)sh->ovf_words;
-    k.rg_x0 = sh->g.x0; k.rg_y0 = sh->g.y0; k.rg_inv_cell = sh->g.inv_cell; k.rg_nx = sh->g.nx; k.rg_ny = sh->g.ny;
-    inf.ray_list_cells = sh->g.nx * sh->g.ny; inf.ray_list_nx = sh->g.nx; inf.ray_list_ny = sh->g.ny; inf.ray_list_cell = sh->g.cell;
-    inf.ray_list_bytes = (int64_t)(sh->slot_words + sh->ovf_words) * 4;
-  }
   k.n_worlds = n_worlds; k.gid0 = gid0;
   k.A = A; k.nc = map->n_cops; k.R = R;
-  k.n_edges = E;
+  k.n_edges = map->n_edges;
   k.lay = make_layout(A, R);          // record / scratch / output-record offsets (world_kernel.cuh)
   CatRecordLayout& rc = env->rec;
   rc.off_dist = 0; rc.off_type = k.lay.r_off_type; rc.off_reward = k.lay.r_off_reward;
@@ -418,30 +540,30 @@ int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds,
   int max_optin = 0, n_sm = 0;
   cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
-  const int smem_max = align_up(blob_bytes, 128) + 2 * k.lay.scratch_bytes;
-  if (align_up(blob_bytes, 128) + 2 * k.lay.scratch_bytes > max_optin) {
+  const int smem_max = align_up(env->blob_bytes, 128) + 2 * k.lay.scratch_bytes;
+  if (smem_max > max_optin) {
     cat_env_destroy(env);
     return fail(CAT_ERR_LIMIT, "map does not fit in shared memory (" + std::to_string(smem_max) + " B)");
   }
   // The attribute belongs to the FUNCTION (per device), not to this environment: always raise it to the device
   // maximum, so creating an environment for a smaller map never lowers the cap of one that is still alive.
   cudaFuncAttributes fattr{};
-  env->kernel = pick_world_kernel(A, R, k.ray_slots != nullptr, true);
-  env->kernel_record = pick_world_kernel(A, R, k.ray_slots != nullptr, false);
+  env->kernel = pick_world_kernel(A, R, k.ray_slots != nullptr, true, n_maps > 1);
+  env->kernel_record = pick_world_kernel(A, R, k.ray_slots != nullptr, false, n_maps > 1);
   CREATE_TRY(cudaFuncGetAttributes(&fattr, env->kernel), "cudaFuncGetAttributes");
   max_optin -= (int)fattr.sharedSizeBytes;      // the opt-in limit covers static + dynamic shared memory
   CREATE_TRY(cudaFuncSetAttribute(env->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin), "cudaFuncSetAttribute");
   if (env->kernel_record != env->kernel)
     CREATE_TRY(cudaFuncSetAttribute(env->kernel_record, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin), "cudaFuncSetAttribute");
-  env->blob_bytes = blob_bytes; env->max_optin = max_optin; env->n_sm = n_sm;
+  env->max_optin = max_optin; env->n_sm = n_sm;
   LaunchShape shp;
   if (!pick_launch_shape(env, n_worlds, &shp)) { cat_env_destroy(env); return fail(CAT_ERR_CUDA, "occupancy query failed"); }
-  env->threads = shp.threads; env->smem_bytes = shp.smem; env->grid = shp.grid;
-  k.world_begin = 0; k.world_end = n_worlds;
+  env->threads = shp.threads; env->smem_bytes = shp.smem;
+  env->grid = fill_map_table(env, k, 0, n_worlds, shp.grid, shp.threads / 32);   // the table every full launch uses
 
   inf.n_worlds = n_worlds; inf.n_agents = A; inf.n_cops = map->n_cops; inf.n_thieves = map->n_thieves;
-  inf.n_rays = R; inf.n_hulls = H; inf.n_edges = E; inf.state_dim = k.state_dim; inf.record_words = k.lay.rec_words;
-  inf.map_blob_bytes = blob_bytes; inf.smem_bytes_per_cta = env->smem_bytes; inf.warps_per_cta = env->threads / 32;
+  inf.n_rays = R; inf.n_hulls = map->n_hulls; inf.n_edges = map->n_edges; inf.state_dim = k.state_dim; inf.record_words = k.lay.rec_words;
+  inf.map_blob_bytes = env->blob_bytes; inf.smem_bytes_per_cta = env->smem_bytes; inf.warps_per_cta = env->threads / 32;
   inf.grid = env->grid; inf.n_pairs = P;
 #undef CREATE_TRY
   *out = env;
@@ -451,10 +573,12 @@ int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds,
 int cat_env_destroy(CatEnv* env) {
   if (!env) return CAT_OK;
   DeviceGuard guard(env->device);
-  if (env->blob_dev) cudaFree(env->blob_dev);
-  if (env->view_off_dev) cudaFree(env->view_off_dev);
-  if (env->view_edges_dev) cudaFree(env->view_edges_dev);
-  ray_lists_release(env->ray_lists);
+  for (EnvMap& m : env->maps) {
+    if (m.blob_dev) cudaFree(m.blob_dev);
+    if (m.view_off_dev) cudaFree(m.view_off_dev);
+    if (m.view_edges_dev) cudaFree(m.view_edges_dev);
+    ray_lists_release(m.ray_lists);
+  }
   if (env->overflow_dev) cudaFree(env->overflow_dev);
   for (cudaEvent_t e : env->chunk_events) cudaEventDestroy(e);
   if (env->copies_done) cudaEventDestroy(env->copies_done);
@@ -466,6 +590,22 @@ int cat_env_destroy(CatEnv* env) {
 int cat_env_info(const CatEnv* env, CatEnvInfo* info) {
   if (!env || !info) return fail(CAT_ERR_INVALID, "null argument");
   *info = env->info;
+  return CAT_OK;
+}
+
+int cat_env_map_info(const CatEnv* env, int32_t map, CatEnvInfo* info) {
+  if (!env || !info) return fail(CAT_ERR_INVALID, "null argument");
+  if (map < 0 || map >= (int)env->maps.size()) return fail(CAT_ERR_INVALID, "map index out of range");
+  const EnvMap& m = env->maps[map];
+  CatEnvInfo inf = env->info;
+  inf.n_worlds = m.n_worlds; inf.n_hulls = m.n_hulls; inf.n_edges = m.n_edges; inf.map_blob_bytes = m.blob_bytes;
+  inf.grid = (map + 1 < env->kp.n_maps ? env->kp.maps[map + 1].cta_begin : env->grid) - env->kp.maps[map].cta_begin;
+  inf.ray_list_cells = 0; inf.ray_list_nx = 0; inf.ray_list_ny = 0; inf.ray_list_cell = 0.f; inf.ray_list_bytes = 0;
+  if (const SharedRayLists* sh = m.ray_lists) {
+    inf.ray_list_cells = sh->g.nx * sh->g.ny; inf.ray_list_nx = sh->g.nx; inf.ray_list_ny = sh->g.ny; inf.ray_list_cell = sh->g.cell;
+    inf.ray_list_bytes = (int64_t)(sh->slot_words + sh->ovf_words) * 4;
+  }
+  *info = inf;
   return CAT_OK;
 }
 
@@ -614,8 +754,8 @@ int cat_env_step_host(CatEnv* env, void* state_dev, const uint8_t* host_actions,
     const int w1 = w0 + per < N ? w0 + per : N, n = w1 - w0;
     LaunchShape shp;
     if (!pick_launch_shape(env, n, &shp)) return fail(CAT_ERR_CUDA, "occupancy query failed");
-    k.world_begin = w0; k.world_end = w1;
-    CUDA_TRY(launch_pdl(kernel_for(env, k), shp.grid, shp.threads, (size_t)shp.smem, stream, k));
+    const int grid = fill_map_table(env, k, w0, w1, shp.grid, shp.threads / 32);   // (a chunk may span several maps)
+    CUDA_TRY(launch_pdl(kernel_for(env, k), grid, shp.threads, (size_t)shp.smem, stream, k));
     CUDA_TRY(cudaEventRecord(env->chunk_events[c], stream));
     CUDA_TRY(cudaStreamWaitEvent(env->copy_stream, env->chunk_events[c], 0));
     CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(records_host) + (size_t)w0 * stride, static_cast<const char*>(records_dev) + (size_t)w0 * stride,

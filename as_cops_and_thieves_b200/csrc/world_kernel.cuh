@@ -38,9 +38,21 @@ struct BlobHeader {
   int32_t off_nextn, off_edgehull, off_conoff, off_conlist;
   int32_t off_dir, off_regoff, off_regions, off_initpos;
   int32_t off_batchbb;
-  int32_t pad[3];
+  // the map's tables in global memory (written by the host once they are on the device): with these in the header a
+  // CTA's map is fully described by the blob it stages, so the CTAs of one launch can run different maps
+  int32_t rg_nx, rg_ny;                     // (cell, ray) candidate-list grid (ray_lists.h)
+  uint32_t ray_slot_count;                  // sizes of the two list arrays (checked build only)
+  float rg_x0, rg_y0, rg_inv_cell;
+  uint32_t ray_ovf_words;
+  const uint4* ray_slots;                   // slots [cells * R] of 4 words; nullptr = rasterise
+  const uint32_t* ray_ovf;                  // overflow words of the lists
+  const int32_t* view_off;                  // per grid cell candidate-edge lists (nullptr = scan all edges)
+  const uint16_t* view_edges;
 };
-static_assert(sizeof(BlobHeader) == 96, "header must stay 16-byte sized");
+static_assert(sizeof(BlobHeader) == 144, "header must stay 16-byte sized");
+__device__ __forceinline__ const BlobHeader* blob_header(const unsigned char* blob) {
+  return reinterpret_cast<const BlobHeader*>(blob);
+}
 
 struct MapView {
   const float4* edge;      // vx, vy, nx, ny  (vertex ending the edge, outward normal)
@@ -58,7 +70,7 @@ struct MapView {
   const float2* init_pos;
   int H, nx, ny;
   float gx0, gy0, cell, inv_cell;
-  int n_edges_dbg;
+  int n_edges;
 };
 
 // Word offsets inside a world's packed state record and byte offsets inside a warp's scratch area — ONE definition,
@@ -104,11 +116,26 @@ __host__ __device__ constexpr Layout make_layout(int A, int R) {
   return l;
 }
 
+// inside a function templated on <TM>: a map-dependent value — from the blob header the CTA staged (TM: a mixed-map
+// launch, every CTA may run another map) or from the parameters (a single-map launch, constant-bank operands)
+#define MAPK(blob, f) (TM ? blob_header(blob)->f : k.f)
+
 template <int TA, int TR> struct FixedLayout { static constexpr Layout v = make_layout(TA ? TA : 1, TR ? TR : 1); };
 // inside a function templated on <TA, TR>: the layout value as an immediate (shipped shape) or from the parameters
 #define LAY(f) (TA ? FixedLayout<TA, TR>::v.f : k.lay.f)
 
+// One map's share of a launch: CTAs [cta_begin, next entry's cta_begin or gridDim.x) step the worlds
+// [world_begin, world_end) of the environment, all of them on the map whose blob they stage.
+struct MapSlice {
+  const unsigned char* blob;
+  int blob_bytes;
+  int cta_begin;
+  int world_begin, world_end;
+};
+
 struct KParams {
+  // The map of a single-map launch (the instantiations with TM = false).  A mixed-map launch (TM = true) finds its
+  // CTA's blob in `maps` below and every other map-dependent value in that blob's header (BlobHeader).
   const unsigned char* blob;
   int blob_bytes;
   const int32_t* view_off;      // global memory: per grid cell candidate-edge lists (nullptr = scan all edges)
@@ -157,6 +184,11 @@ struct KParams {
   float* critic_f32;
   uint16_t* obs_bf16;
   uint16_t* critic_bf16;
+  // The launch's maps, by value (no device table, graph-capturable): entries in increasing cta_begin and world order,
+  // together covering [world_begin, world_end).  Read by the TM = true instantiations only; a single-map launch fills
+  // one entry that mirrors the fields above.
+  int n_maps;
+  MapSlice maps[CAT_MAX_MAPS];
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -179,7 +211,7 @@ __device__ __forceinline__ MapView make_view(const unsigned char* blob) {
   m.reg_off = reinterpret_cast<const int32_t*>(blob + h->off_regoff);
   m.regions = reinterpret_cast<const float4*>(blob + h->off_regions);
   m.init_pos = reinterpret_cast<const float2*>(blob + h->off_initpos);
-  m.H = h->n_hulls; m.nx = h->nx; m.ny = h->ny; m.n_edges_dbg = h->n_edges;
+  m.H = h->n_hulls; m.nx = h->nx; m.ny = h->ny; m.n_edges = h->n_edges;
   m.gx0 = h->gx0; m.gy0 = h->gy0; m.cell = h->cell; m.inv_cell = h->inv_cell;
   return m;
 }
@@ -469,7 +501,7 @@ __device__ __noinline__ void raster_batch(const unsigned char* blob, unsigned lo
     if (p < total) {
       int i = i0l + (p - exl);
       if (i >= R) i -= R;
-      CAT_CHECK(i >= 0 && i < R && el >= 0 && el < m.n_edges_dbg);
+      CAT_CHECK(i >= 0 && i < R && el >= 0 && el < m.n_edges);
       const float4 dv = m.dir[i];
       Ray r;
       r.ox = ox; r.oy = oy; r.ux = dv.x; r.uy = dv.y; r.L = L;
@@ -493,6 +525,7 @@ __device__ __noinline__ void raster_batch(const unsigned char* blob, unsigned lo
 // of 32 edges (hulls are stored in Morton order, so a batch is compact) are visited NEAR TO FAR: lane b measures
 // the distance of batch b's bounding box once, a counting rank orders them, and the walk stops at the first batch
 // beyond sensor range; the per-grid-cell static lists (maps.view_lists) shorten the scan when present.
+template <bool TM>
 __device__ __noinline__ void rasterise_agent(const KParams& k, const unsigned char* blob, unsigned char* scratch, int a,
                                              float ox, float oy) {
   // (scalars, not the Warp struct: a struct passed by reference to an out-of-line function would live in local memory)
@@ -501,18 +534,18 @@ __device__ __noinline__ void rasterise_agent(const KParams& k, const unsigned ch
   w.best = reinterpret_cast<unsigned long long*>(scratch + k.lay.s_best);
   w.cand = reinterpret_cast<uint16_t*>(scratch + k.lay.s_cand);
   w.blob = blob; w.lane = threadIdx.x & 31;
-  const int R = k.R, lane = w.lane, E = k.n_edges;
+  const int R = k.R, lane = w.lane, E = MAPK(blob, n_edges);
   const float L = k.ray_len, rsum = k.wall_r + k.ray_r;
   const float range2 = (L + rsum) * (L + rsum);
   int ncand = 0;
   const int nb = (E + 31) >> 5;
   int vq = 0, vq1 = 0;
-  const int vcell = k.view_off ? grid_cell(m, ox, oy) : -1;
+  const int vcell = MAPK(blob, view_off) ? grid_cell(m, ox, oy) : -1;
   const bool use_view = vcell >= 0;
   uint32_t vnext = 0xFFFFu;
   if (use_view) {
-    vq = __ldg(k.view_off + vcell); vq1 = __ldg(k.view_off + vcell + 1);
-    if (vq + lane < vq1) vnext = __ldg(k.view_edges + vq + lane);
+    vq = __ldg(MAPK(blob, view_off) + vcell); vq1 = __ldg(MAPK(blob, view_off) + vcell + 1);
+    if (vq + lane < vq1) vnext = __ldg(MAPK(blob, view_edges) + vq + lane);
   }
   const bool ordered = !use_view && nb <= 32;
   float bdist = CUDART_INF_F;
@@ -536,7 +569,7 @@ __device__ __noinline__ void rasterise_agent(const KParams& k, const unsigned ch
       if (vq >= vq1) break;
       e = vnext == 0xFFFFu ? E : (int)vnext;
       vq += 32;
-      vnext = vq + lane < vq1 ? (uint32_t)__ldg(k.view_edges + vq + lane) : 0xFFFFu;
+      vnext = vq + lane < vq1 ? (uint32_t)__ldg(MAPK(blob, view_edges) + vq + lane) : 0xFFFFu;
     } else {
       if (it >= nb) break;
       int base;
@@ -608,7 +641,7 @@ struct SlotStage { uint32_t phase; bool pending; };
 // arithmetic — started as early as the positions are known so that the L2 / HBM latency hides behind the
 // termination test and the action impulses.  Slot r lands at w.best + 2 r (16-byte stride); the walk later writes
 // ray r's result key over the first half of its own slot.
-template <int TA, int TR>
+template <int TA, int TR, bool TM>
 __device__ __forceinline__ void stage_ray_slots(const KParams& k, const Warp& w, SlotStage& st) {
   const int A = TA ? TA : k.A, R = TR ? TR : k.R, lane = w.lane;
   const float* pos = w.rec;
@@ -616,8 +649,8 @@ __device__ __forceinline__ void stage_ray_slots(const KParams& k, const Warp& w,
   if (st.pending) { mbar_wait(bar, st.phase); st.phase ^= 1u; }
   int base = -1;   // outside the grid: farther than the sensor reach from every wall
   if (lane < A) {
-    const float gx = (pos[2 * lane] - k.rg_x0) * k.rg_inv_cell, gy = (pos[2 * lane + 1] - k.rg_y0) * k.rg_inv_cell;
-    if (gx >= 0.f && gy >= 0.f && gx < (float)k.rg_nx && gy < (float)k.rg_ny) base = ((int)gy * k.rg_nx + (int)gx) * R;
+    const float gx = (pos[2 * lane] - MAPK(w.blob, rg_x0)) * MAPK(w.blob, rg_inv_cell), gy = (pos[2 * lane + 1] - MAPK(w.blob, rg_y0)) * MAPK(w.blob, rg_inv_cell);
+    if (gx >= 0.f && gy >= 0.f && gx < (float)MAPK(w.blob, rg_nx) && gy < (float)MAPK(w.blob, rg_ny)) base = ((int)gy * MAPK(w.blob, rg_nx) + (int)gx) * R;
   }
   const uint32_t inside = __ballot_sync(0xFFFFFFFFu, base >= 0);   // (also orders the previous world's reads of the slot area)
   if (lane == 0) {
@@ -629,10 +662,10 @@ __device__ __forceinline__ void stage_ray_slots(const KParams& k, const Warp& w,
     const int ba = __shfl_sync(0xFFFFFFFFu, base, a);
     uint4* dst = reinterpret_cast<uint4*>(w.best) + a * R;
     if (ba >= 0) {
-      CAT_CHECK((unsigned)(ba + R) <= k.ray_slot_count && (a + 1) * R * 16 <= LAY(nrays_pad) * 16);
+      CAT_CHECK((unsigned)(ba + R) <= MAPK(w.blob, ray_slot_count) && (a + 1) * R * 16 <= LAY(nrays_pad) * 16);
       if (lane == 0)
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                     "l"(k.ray_slots + ba), "r"(R * 16), "r"(bar)
+                     "l"(MAPK(w.blob, ray_slots) + ba), "r"(R * 16), "r"(bar)
                      : "memory");
     } else {
 #pragma unroll 1
@@ -653,7 +686,7 @@ __device__ __forceinline__ void stage_ray_slots(const KParams& k, const Warp& w,
 // winner; if it fails (a grazing fat ray) the list is walked again with the rule applied to every hit.
 //   Hit key = (float bits of s, feature): smaller s first, then smaller feature — the order of the rasteriser's
 // 64-bit atomicMin, so both paths pick the same hit bit for bit.
-template <int TA, int TR>
+template <int TA, int TR, bool TM>
 __device__ __forceinline__ void sweep_lists(const KParams& k, const MapView& m, const Warp& w, SlotStage& st) {
   const int A = TA ? TA : k.A, R = TR ? TR : k.R, nrays = A * R, lane = w.lane;
   const float L = k.ray_len, rsum = k.wall_r + k.ray_r, rs2 = rsum * rsum, inv_L = 1.f / k.ray_len;
@@ -696,15 +729,16 @@ __device__ __forceinline__ void sweep_lists(const KParams& k, const MapView& m, 
     if (cur >= 0) {
       uint32_t ent = e0;
       if (__builtin_expect((int)ent < 0, 0)) {   // link: the list continues in a chunk of the overflow array
-        CAT_CHECK((ent & 0x7FFFFFFFu) + 4u <= k.ray_ovf_words && ((ent & 3u) == 0u));
-        const uint4 c = __ldg(reinterpret_cast<const uint4*>(k.ray_ovf + (ent & 0x7FFFFFFFu)));
+        // (TM: the pointer is read here, on the rare path, so no register holds it across the walk)
+        CAT_CHECK((ent & 0x7FFFFFFFu) + 4u <= MAPK(w.blob, ray_ovf_words) && ((ent & 3u) == 0u));
+        const uint4 c = __ldg(reinterpret_cast<const uint4*>(MAPK(w.blob, ray_ovf) + (ent & 0x7FFFFFFFu)));
         ent = c.x; e1 = c.y; e2 = c.z; e3 = c.w;
       }
       e0 = e1; e1 = e2; e2 = e3; e3 = kRayEnd;
       if (__uint_as_float(bs) < __uint_as_float(ent & 0xFFFF0000u)) fin = true;   // (an empty list: its first entry is the end mark)
       else {
         const uint32_t el = ent & 0xFFFFu;
-        CAT_CHECK((int)el < k.n_edges && cur < nrays);
+        CAT_CHECK((int)el < MAPK(w.blob, n_edges) && cur < nrays);
         Ray r;
         r.ox = ox; r.oy = oy; r.ux = ux; r.uy = uy; r.L = L;
         int kind;
@@ -770,12 +804,12 @@ __device__ __forceinline__ void sweep_lists(const KParams& k, const MapView& m, 
 // candidate lists (sweep_lists, lanes = rays) or, without lists, by rasterising the edges in view into a 1-D depth
 // buffer per agent (rasterise_agent, lanes = edges then (edge, ray) pairs).  Then, lanes = rays: the other agents'
 // circles and the alpha = 0 rules are merged in, and the hit point goes through the float16 chain.
-template <int TA, int TR, bool TL, bool TX>
+template <int TA, int TR, bool TL, bool TX, bool TM>
 __device__ __forceinline__ void observe_world(const KParams& k, const MapView& m, const Warp& w, long long world, bool staged,
                                               SlotStage& st) {
   const int A = TA ? TA : k.A, R = TR ? TR : k.R, lane = w.lane;
-  const bool lists = TL || k.ray_slots != nullptr;   // TL: an instantiation without the rasteriser
-  if (lists && !staged) stage_ray_slots<TA, TR>(k, w, st);
+  const bool lists = TL || MAPK(w.blob, ray_slots) != nullptr;   // TL: an instantiation without the rasteriser
+  if (lists && !staged) stage_ray_slots<TA, TR, TM>(k, w, st);
   const float* pos = w.rec;
   const float* tc = w.rec + LAY(o_tc);
   const uint32_t flags = reinterpret_cast<const uint32_t*>(w.rec)[LAY(o_flags)];
@@ -814,7 +848,7 @@ __device__ __forceinline__ void observe_world(const KParams& k, const MapView& m
   __syncwarp();
   if (lane == 0 && flags) reinterpret_cast<uint32_t*>(w.rec)[LAY(o_flags)] = 0u;   // lists are now valid for these positions
 
-  if (lists) sweep_lists<TA, TR>(k, m, w, st);
+  if (lists) sweep_lists<TA, TR, TM>(k, m, w, st);
   const int kstride = lists ? 2 : 1;   // the list walk leaves ray r's key in the first half of its 16-byte slot
 
   const int nsub = (R + 31) >> 5;
@@ -836,7 +870,7 @@ __device__ __forceinline__ void observe_world(const KParams& k, const MapView& m
       for (int i = lane; i < R; i += 32) w.best[a * R + i] = make_key(L, kNoFeature);
       __syncwarp();
       // ---- (2) rasterise the walls in view
-      rasterise_agent(k, w.blob, reinterpret_cast<unsigned char*>(w.rec), a, ox, oy);
+      rasterise_agent<TM>(k, w.blob, reinterpret_cast<unsigned char*>(w.rec), a, ox, oy);
     }
 
     // the other agents' cached centres relative to this origin, compacted (the candidate queue is free now)
@@ -909,7 +943,7 @@ __device__ __forceinline__ void observe_world(const KParams& k, const MapView& m
           // rewards need the nearest opponent seen by this agent (cop.py:66-70, thief.py:60-63)
           if (type == want) atomicMin(&w.minbits[a], (uint32_t)dbits);
         }
-        CAT_CHECK(r < LAY(nrays) && (feat == kNoFeature || feat >= kAgentTag || (int)(feat >> 1) < k.n_edges));
+        CAT_CHECK(r < LAY(nrays) && (feat == kNoFeature || feat >= kAgentTag || (int)(feat >> 1) < MAPK(w.blob, n_edges)));
         w.rdist[r] = dbits;
         w.rtype[r] = type;
         if (TX && k.hit_point) {
@@ -1524,14 +1558,39 @@ __device__ __forceinline__ void reset_world(const KParams& k, const MapView& m, 
 // shipped map: <3, 90>), or 0 = read them from the parameters (any other configuration: <0, 0>).  TL: the environment
 // has ray lists (the default) — the instantiation carries no rasteriser code at all.  TX = false: a STEP launch that wants the
 // output record only — none of the optional outputs (separate arrays, shared observations, fp32 / bf16 layouts, hit
-// points) and none of the init / reset / observe launch modes is compiled in.
-template <int TA, int TR, bool TL, bool TX>
+// points) and none of the init / reset / observe launch modes is compiled in.  TM: a mixed-map environment — each CTA
+// looks its map up in the launch's map table and reads the map-dependent values from the blob header it staged; the
+// single-map instantiations (TM = false) take them from the parameters, at no register cost (a run-time table lookup
+// in every instantiation raised the spills of three of the four, by up to 148 bytes of loads).
+template <int TA, int TR, bool TL, bool TX, bool TM>
 __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_constant__ KParams k) {
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) unsigned long long mbar;
   __shared__ int next_slot;   // the CTA's world queue (below)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int mode = TX ? k.mode : (int)MODE_STEP;   // the record-only instantiation serves step launches only (kernel_for)
+
+  // The CTA's map: the last entry of the launch's map table whose first CTA is at or below this one (at most
+  // CAT_MAX_MAPS - 1 uniform compares).  Inside its map's share of the launch the CTA numbers itself and its worlds
+  // exactly as a launch of that map alone would.
+  int mi = 0;
+  if (TM) {
+#pragma unroll
+    for (int i = 1; i < CAT_MAX_MAPS; ++i) mi += (i < k.n_maps && (int)blockIdx.x >= k.maps[i].cta_begin) ? 1 : 0;
+  }
+  const unsigned char* map_blob_m = k.maps[mi].blob;
+  const int map_blob_bytes_m = k.maps[mi].blob_bytes;
+  // the CTA's share of the launch: its map's group of CTAs and worlds (TM), or the whole launch — a single-map
+  // instantiation reads these straight from the parameters and special registers, as it always has
+  const unsigned cta_m = blockIdx.x - (unsigned)k.maps[mi].cta_begin;   // (unsigned, like blockIdx.x)
+  const unsigned n_cta_m = (unsigned)((mi + 1 < k.n_maps ? k.maps[mi + 1].cta_begin : (int)gridDim.x) - k.maps[mi].cta_begin);
+  const int world_begin_m = k.maps[mi].world_begin, world_end_m = k.maps[mi].world_end;
+#define MAP_BLOB (TM ? map_blob_m : k.blob)
+#define MAP_BLOB_BYTES (TM ? map_blob_bytes_m : k.blob_bytes)
+#define CTA_IDX (TM ? cta_m : blockIdx.x)
+#define CTA_CNT (TM ? n_cta_m : gridDim.x)
+#define W_BEGIN (TM ? world_begin_m : k.world_begin)
+#define W_END (TM ? world_end_m : k.world_end)
 
   // Stage the map once per CTA: one elected thread issues a TMA bulk copy (cp.async.bulk ->
   // UBLKCP) that completes on an mbarrier; everyone else waits on the barrier's phase.
@@ -1542,11 +1601,11 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
   }
   __syncthreads();
   if (tid == 0) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&mbar)), "r"(k.blob_bytes)
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&mbar)), "r"(MAP_BLOB_BYTES)
                  : "memory");
     asm volatile(
         "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem)),
-        "l"(k.blob), "r"(k.blob_bytes), "r"(smem_u32(&mbar))
+        "l"(MAP_BLOB), "r"(MAP_BLOB_BYTES), "r"(smem_u32(&mbar))
         : "memory");
   }
   // Programmatic dependent launch (the host launches with programmatic stream serialisation): everything above — CTA
@@ -1556,10 +1615,10 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
   asm volatile("griddepcontrol.wait;" ::: "memory");
   // Prefetch this warp's first record while the map copy is in flight (with one world per warp, the usual case
   // at a few thousand worlds, both latencies would otherwise add up on the critical path).
-  const bool one_wave_launch = (long long)gridDim.x * (blockDim.x >> 5) >= k.world_end - k.world_begin;
-  const long long first_world = one_wave_launch ? k.world_begin + (long long)blockIdx.x * (blockDim.x >> 5) + warp
-                                                : k.world_begin + blockIdx.x + (long long)warp * gridDim.x;
-  const bool prefetched = LAY(rec_words) <= 64 && mode != MODE_INIT && first_world < k.world_end;
+  const bool one_wave_launch = (long long)CTA_CNT * (blockDim.x >> 5) >= W_END - W_BEGIN;
+  const long long first_world = one_wave_launch ? W_BEGIN + (long long)CTA_IDX * (blockDim.x >> 5) + warp
+                                                : W_BEGIN + CTA_IDX + (long long)warp * CTA_CNT;
+  const bool prefetched = LAY(rec_words) <= 64 && mode != MODE_INIT && first_world < W_END;
   float pf0 = 0.f, pf1 = 0.f;
   if (prefetched) {
     const float* g = k.state + (size_t)first_world * LAY(rec_words);
@@ -1581,7 +1640,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
   }
   const MapView m = make_view(smem);
 
-  unsigned char* scratch = smem + ((k.blob_bytes + 127) & ~127) + (size_t)warp * LAY(scratch_bytes);
+  unsigned char* scratch = smem + ((MAP_BLOB_BYTES + 127) & ~127) + (size_t)warp * LAY(scratch_bytes);
   Warp w;
   w.rec = reinterpret_cast<float*>(scratch);
   w.rdist = reinterpret_cast<uint16_t*>(scratch + LAY(s_rdist));
@@ -1610,7 +1669,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
   for (int i = lane; i < (LAY(r_bytes) >> 2); i += 32) reinterpret_cast<uint32_t*>(w.rdist)[i] = 0u;
   __syncwarp();
   const int A = TA ? TA : k.A;
-  // Worlds to warps.  CTA c owns the worlds c, c + G, c + 2 G, ... of the launch (G = gridDim.x): every SM gets the same
+  // Worlds to warps.  CTA c owns the worlds c, c + G, c + 2 G, ... of its map's share of the launch (G = that share's CTAs): every SM gets the same
   // number of worlds to within one, whatever the world count — with contiguous blocks of `warps` worlds per CTA and round,
   // 16384 worlds on 148 x 32 warps left 80 SMs with three rounds and 68 with four: the SMs were busy 77 % of the launch
   // (ncu sm__cycles_active / elapsed, profiles/r2_notes.md).  Inside the CTA the warps draw their next world from a
@@ -1627,9 +1686,9 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
 #pragma unroll 1
   for (int slot = warp;; slot = next_world_slot()) {
     if (one_wave && slot >= wpc) break;
-    const long long world = one_wave ? k.world_begin + (long long)blockIdx.x * wpc + slot
-                                     : k.world_begin + blockIdx.x + (long long)slot * gridDim.x;
-    if (world >= k.world_end) break;
+    const long long world = one_wave ? W_BEGIN + (long long)CTA_IDX * wpc + slot
+                                     : W_BEGIN + CTA_IDX + (long long)slot * CTA_CNT;
+    if (world >= W_END) break;
     float* grec = k.state + (size_t)world * LAY(rec_words);
     int32_t* reci = reinterpret_cast<int32_t*>(w.rec);
 
@@ -1660,7 +1719,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
     bool captured = false, timeout = false;
     // the sensor sweep reads the PRE-step positions, which are known now: start fetching the rays' candidate slots
     bool staged = false;
-    if (do_step && (TL || k.ray_slots)) { stage_ray_slots<TA, TR>(k, w, slot_stage); staged = true; }
+    if (do_step && (TL || MAPK(smem, ray_slots))) { stage_ray_slots<TA, TR, TM>(k, w, slot_stage); staged = true; }
     if (do_step) {  // ---------------- base_env.py:354-383 ----------------
       const float* pos = w.rec;
       float* vel = w.rec + LAY(o_vel);
@@ -1710,7 +1769,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
       // is re-spawned in it emits the NEW episode's observation (C-10) and a terminal reward that does not depend
       // on what is seen, so its terminal sensor sweep would be thrown away: skip it.  With one world per warp the
       // launch lasts as long as its slowest warp, and a second sweep made every finishing world that warp.
-      if (!(do_step && (captured || timeout) && k.auto_reset)) observe_world<TA, TR, TL, TX>(k, m, w, world, staged, slot_stage);
+      if (!(do_step && (captured || timeout) && k.auto_reset)) observe_world<TA, TR, TL, TX, TM>(k, m, w, world, staged, slot_stage);
       bool again = false;
       if (do_step) {
         if (lane < A) w.rew[lane] = agent_reward(k, lane, w.minbits[lane], captured, timeout);
@@ -1742,4 +1801,10 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
     __syncwarp();
   }
 }
+#undef MAP_BLOB
+#undef MAP_BLOB_BYTES
+#undef CTA_IDX
+#undef CTA_CNT
+#undef W_BEGIN
+#undef W_END
 

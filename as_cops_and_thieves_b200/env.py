@@ -71,7 +71,7 @@ class _EnvCommon:
 
     metadata = {"render_modes": ["human", "rgb_array"]}  # base_env.py:49
 
-    def _setup_common(self, map: Map, cmap, params: EnvParams) -> None:
+    def _setup_common(self, map: Map, cmap, params: EnvParams, window: Optional[Tuple[float, float]] = None) -> None:
         self.map = map
         self.width, self.height = map.window_dimensions
         self.possible_agents: List[str] = cmap.agent_ids                     # base_env.py:96
@@ -79,7 +79,7 @@ class _EnvCommon:
         obs_space = _agent_observation_space(params.n_rays, params.ray_length)
         self.observation_spaces = {a: obs_space for a in self.possible_agents}  # base_env.py:102-105
         self.action_spaces = {a: spaces.Discrete(4) for a in self.possible_agents}  # entity.py:88-90
-        shared = _shared_observation_space(map.window_dimensions, self.possible_agents, cmap.n_cops,
+        shared = _shared_observation_space(window or map.window_dimensions, self.possible_agents, cmap.n_cops,
                                            params.n_rays, params.ray_length)
         self.shared_observation_spaces = shared                              # base_env.py:113-115
         self._shared_observation_spaces = shared
@@ -105,6 +105,15 @@ class _EnvCommon:
                         sp[f"{other}_{key}"] = s
             flat[aid] = spaces.Dict(sp)
         return spaces.Dict(flat)
+
+
+def split_worlds(num_envs: int, n_maps: int) -> List[int]:
+    """``num_envs`` worlds over ``n_maps`` maps as evenly as possible, the remainder to the first maps."""
+    num_envs, n_maps = int(num_envs), int(n_maps)
+    if n_maps < 1 or num_envs < n_maps:
+        raise ValueError(f"cannot split {num_envs} worlds over {n_maps} maps (at least one world per map)")
+    q, r = divmod(num_envs, n_maps)
+    return [q + (1 if m < r else 0) for m in range(n_maps)]
 
 
 def _make_params(max_step_count: int, time_step: float, physical: Optional[dict], **over) -> EnvParams:
@@ -248,18 +257,48 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
 
     ``agents`` never empties: finished worlds are re-spawned inside the step kernel and report the
     observation of the new episode (SURVEY.md C-10), with the terminal reward / flags of the old one.
+
+    Mixed maps: ``map`` may be a sequence of maps (at most 8, all with the same cops and thieves).  ``num_envs`` is
+    then split over them as evenly as possible (the remainder to the first maps, ``split_worlds``) or given per map;
+    ``spawn_override`` is None or one entry per map, ``cell`` applies to every map.  Map m owns a contiguous block of
+    the worlds (``map_index`` gives the map of each, ``map_names`` their names), one launch steps all of them, and the
+    observation, state and critic layouts are the single-map ones.  ``team_positions`` is bounded by the largest window.
     """
 
-    def __init__(self, map: Map, num_envs: int, *, max_step_count: int = 400, time_step: float = 1 / 60.0,
-                 device: Union[str, torch.device] = "cuda:0", seed: int = 0, gid0: int = 0,
+    def __init__(self, map: Union[Map, Sequence[Map]], num_envs: Union[int, Sequence[int]], *, max_step_count: int = 400,
+                 time_step: float = 1 / 60.0, device: Union[str, torch.device] = "cuda:0", seed: int = 0, gid0: int = 0,
                  physical_params: Optional[dict] = None, stale_shape_cache: bool = True,
-                 spawn_override: Optional[dict] = None, cell: Optional[float] = None, render_mode=None):
+                 spawn_override: Optional[Union[dict, Sequence[Optional[dict]]]] = None, cell: Optional[float] = None,
+                 render_mode=None):
         params = _make_params(max_step_count, time_step, physical_params, auto_reset=1, seed=int(seed),
                               stale_shape_cache=int(stale_shape_cache))
-        self._cmap = compile_map(map, spawn_override=spawn_override, cell=cell)
         self._params = params
-        self._setup_common(map, self._cmap, params)
-        self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True)
+        if isinstance(map, Map):
+            self.maps = [map]
+            self._cmap = compile_map(map, spawn_override=spawn_override, cell=cell)
+            self._cmaps = [self._cmap]
+            self._setup_common(map, self._cmap, params)
+            self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True)
+        else:
+            self.maps = list(map)
+            n = len(self.maps)
+            counts = split_worlds(num_envs, n) if isinstance(num_envs, (int, np.integer)) else [int(c) for c in num_envs]
+            if len(counts) != n:
+                raise ValueError(f"{n} maps need {n} world counts, got {len(counts)}")
+            overrides = [None] * n if spawn_override is None else list(spawn_override)
+            if len(overrides) != n:
+                raise ValueError(f"spawn_override: one entry per map ({n}), got {len(overrides)}")
+            self._cmaps = [compile_map(m, spawn_override=o, cell=cell) for m, o in zip(self.maps, overrides)]
+            self._cmap = self._cmaps[0]
+            if any(c.agent_ids != self._cmap.agent_ids for c in self._cmaps):
+                raise ValueError("every map of a mixed environment needs the same agents")
+            window = (max(m.window_dimensions[0] for m in self.maps), max(m.window_dimensions[1] for m in self.maps))
+            self._setup_common(self.maps[0], self._cmap, params, window=window)
+            self._w = CatWorlds(self._cmaps, counts, device=device, gid0=gid0, params=params, want_f32=True,
+                                want_critic=True)
+            num_envs = sum(counts)
+        self.map_names = [c.name for c in self._cmaps]
+        self.map_index = self._w.map_index
         self.num_envs = int(num_envs)
         self.num_agents = len(self.possible_agents)
         self.agents = self.possible_agents[:]
@@ -322,9 +361,10 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         return self._w.critic_f32
 
     def render(self, world: int = 0):
+        """``rgb_array`` of one world, drawn on that world's own map."""
         from .render import render_rgb
         pos = self._w.get_state()["pos"][world].cpu().numpy()
-        return render_rgb(self._cmap, pos)
+        return render_rgb(self._cmaps[int(self._w.map_index[world])], pos)
 
     def close(self) -> None:
         self._w.close()

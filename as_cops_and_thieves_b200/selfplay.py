@@ -130,16 +130,26 @@ def sample_policy_from_archive(role_archive_path: Path, role_prefix: str, strate
 
 # ------------------------------------------------------------------ batched evaluation (eval_pfsp_agents.py:7-59)
 def evaluate_agents(env, learner, n_episodes: int = 5, cop_prefix: str = "cop", thief_prefix: str = "thief",
-                    greedy: bool = False, max_steps: Optional[int] = None) -> Tuple[float, float]:
+                    greedy: bool = False, max_steps: Optional[int] = None, by_map: bool = False):
     """Play every world until it has finished ``n_episodes`` episodes with the learner's policies frozen;
     return (cop win rate, thief win rate) over all counted episodes.  The winner comes from the step kernel's
-    ``winner`` output (0 cop, 1 thief), the batched form of ``infos[agent]["winner"]``."""
+    ``winner`` output (0 cop, 1 thief), the batched form of ``infos[agent]["winner"]``.
+
+    ``by_map=True`` (for a mixed-map environment) returns ``(cop rate, thief rate, per_map)`` instead, ``per_map``
+    holding one dict per map of the environment — ``{"map", "cop", "thief", "episodes"}`` — from the episodes its
+    worlds finished (``env.map_index``); their ``episodes`` add up to the episodes behind the overall rates."""
     import torch
     N, dev = env.num_envs, env.device
     limit = max_steps or (env.max_step_count + 1) * n_episodes
     finished = torch.zeros(N, dtype=torch.int32, device=dev)
     cop_wins = torch.zeros((), dtype=torch.int64, device=dev)
     thief_wins = torch.zeros((), dtype=torch.int64, device=dev)
+    if by_map:
+        map_index = getattr(env, "map_index", None)
+        map_index = torch.zeros(N, dtype=torch.int64, device=dev) if map_index is None else map_index.to(dev, torch.int64)
+        names = list(getattr(env, "map_names", None) or [f"map{m}" for m in range(int(map_index.max()) + 1)])
+        cop_by_map = torch.zeros(len(names), dtype=torch.int64, device=dev)
+        thief_by_map = torch.zeros(len(names), dtype=torch.int64, device=dev)
     was_training = {a: (learner.models[a]["policy"].training, learner.models[a]["value"].training) for a in learner.agents}
     for a in learner.agents:
         learner.models[a]["policy"].eval()
@@ -154,6 +164,9 @@ def evaluate_agents(env, learner, n_episodes: int = 5, cop_prefix: str = "cop", 
             counted = done & (finished < n_episodes)
             cop_wins += (counted & (winner == 0)).sum()
             thief_wins += (counted & (winner == 1)).sum()
+            if by_map:
+                cop_by_map += torch.bincount(map_index[counted & (winner == 0)], minlength=len(names))
+                thief_by_map += torch.bincount(map_index[counted & (winner == 1)], minlength=len(names))
             finished += counted.to(torch.int32)
             learner.note_done(done)
             if bool((finished >= n_episodes).all()):
@@ -163,7 +176,15 @@ def evaluate_agents(env, learner, n_episodes: int = 5, cop_prefix: str = "cop", 
     learner.reset_recurrent_state()
     learner._obs = None          # the next rollout starts from a fresh reset, like env.reset() at eval_pfsp_agents.py:53
     total = max(int(finished.sum().item()), 1)
-    return int(cop_wins.item()) / total, int(thief_wins.item()) / total
+    if not by_map:
+        return int(cop_wins.item()) / total, int(thief_wins.item()) / total
+    episodes = torch.zeros(len(names), dtype=torch.int64, device=dev).index_add_(0, map_index, finished.to(torch.int64))
+    per_map = []
+    for m, name in enumerate(names):
+        n_m = int(episodes[m].item())
+        per_map.append({"map": name, "cop": int(cop_by_map[m].item()) / max(n_m, 1),
+                        "thief": int(thief_by_map[m].item()) / max(n_m, 1), "episodes": n_m})
+    return int(cop_wins.item()) / total, int(thief_wins.item()) / total, per_map
 
 
 def evaluate_agent(env, learner, learned_role_prefix: str, opponent_role_prefix: str, opponent_role_archive_path: Path,

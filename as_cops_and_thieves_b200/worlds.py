@@ -40,8 +40,37 @@ class HostRecords(dict):
         raise KeyError(key)
 
 
+def _map_desc(cmap: CompiledMap):
+    """``CatMapDesc`` of a compiled map, and the numpy arrays it points into (keep them alive while it is used)."""
+    keep = dict(
+        hull_off=np.ascontiguousarray(cmap.hull_off, np.int32),
+        vert=np.ascontiguousarray(cmap.vert, np.float64),
+        normal=np.ascontiguousarray(cmap.normal, np.float64),
+        edge_len=np.ascontiguousarray(cmap.edge_len, np.float64),
+        hull_bb=np.ascontiguousarray(cmap.hull_bb, np.float64),
+        init_pos=np.ascontiguousarray(cmap.init_pos, np.float64),
+        region_off=np.ascontiguousarray(cmap.region_off, np.int32),
+        regions=np.ascontiguousarray(cmap.regions if len(cmap.regions) else np.zeros((1, 4)), np.float64),
+        con_cell_off=np.ascontiguousarray(cmap.con_cell_off, np.int32),
+        con_cell_hulls=np.ascontiguousarray(np.append(cmap.con_cell_hulls, 0), np.int32),
+        view_cell_off=np.ascontiguousarray(cmap.view_cell_off, np.int32),
+        view_cell_edges=np.ascontiguousarray(np.append(cmap.view_cell_edges, 0), np.int32),
+    )
+    k = keep
+    md = CatMapDesc(
+        cmap.n_hulls, cmap.n_edges, _lib.np_ptr(k["hull_off"]), _lib.np_ptr(k["vert"]), _lib.np_ptr(k["normal"]),
+        _lib.np_ptr(k["edge_len"]), _lib.np_ptr(k["hull_bb"]), cmap.n_cops, cmap.n_thieves,
+        _lib.np_ptr(k["init_pos"]), _lib.np_ptr(k["region_off"]), _lib.np_ptr(k["regions"]),
+        cmap.grid_x0, cmap.grid_y0, cmap.cell, cmap.nx, cmap.ny,
+        _lib.np_ptr(k["con_cell_off"]), _lib.np_ptr(k["con_cell_hulls"]),
+        _lib.np_ptr(k["view_cell_off"]) if len(k["view_cell_off"]) == cmap.nx * cmap.ny + 1 else None,
+        _lib.np_ptr(k["view_cell_edges"]), float(cmap.view_range))
+    return md, keep
+
+
 class CatWorlds:
-    def __init__(self, cmap: CompiledMap, n_worlds: int, *, device: Union[str, torch.device] = "cuda:0",
+    def __init__(self, cmap: Union[CompiledMap, Sequence[CompiledMap]], n_worlds: Union[int, Sequence[int]], *,
+                 device: Union[str, torch.device] = "cuda:0",
                  gid0: int = 0, params: Optional[EnvParams] = None, want_f32: bool = True,
                  want_shared: bool = True, want_hits: bool = False, pinned_outputs: bool = False,
                  want_critic: bool = False, want_bf16: bool = False, **overrides):
@@ -49,51 +78,57 @@ class CatWorlds:
         results there directly and the host reads them (``tensor.numpy()``) after one stream synchronisation —
         the layout for callers that consume every step on the CPU, like the single-world PettingZoo face.
         ``want_critic``: also emit the critic's 4-channel ray block ``critic_f32 (N, 4, R)``
-        (``lstm_value_net.py:122-137``); ``want_bf16``: bf16 copies of ``obs_f32`` / ``critic_f32``."""
+        (``lstm_value_net.py:122-137``); ``want_bf16``: bf16 copies of ``obs_f32`` / ``critic_f32``.
+
+        Mixed maps: ``cmap`` may be a sequence of compiled maps (at most ``CAT_MAX_MAPS``, all with the same cops and
+        thieves) with ``n_worlds`` the matching sequence of world counts.  Map m then owns the worlds
+        ``world_offsets[m] .. world_offsets[m] + n_worlds[m]`` and all of them are stepped by one launch; world i is
+        the same world as world ``i - world_offsets[m]`` of a single-map ``CatWorlds`` of map m with
+        ``gid0 + world_offsets[m]``.  ``cmaps``, ``world_offsets`` and ``map_index`` (the map of every world, (N,) int64
+        on the device) describe the split; with one map they hold that map alone."""
+        if isinstance(cmap, CompiledMap):
+            multi, cmaps, counts = False, [cmap], [int(n_worlds)]
+        else:
+            multi, cmaps = True, list(cmap)
+            if isinstance(n_worlds, (int, np.integer)):
+                raise ValueError("with a sequence of maps, n_worlds is the sequence of their world counts")
+            counts = [int(n) for n in n_worlds]
+            if len(counts) != len(cmaps) or not cmaps:
+                raise ValueError(f"{len(cmaps)} maps need as many world counts, got {len(counts)}")
         self.device = torch.device(device)
         _require_cuda(self.device)
         self.L = _lib.load()
-        self.cmap = cmap
+        self.cmaps = cmaps
+        self.cmap = cmaps[0]
+        self.worlds_per_map = tuple(counts)
+        self.world_offsets = tuple(int(v) for v in np.cumsum([0] + counts[:-1]))
         p = (params or EnvParams()).as_dict()
         p.update(overrides)
         self.params = p
-        self.n_worlds = int(n_worlds)
+        self.n_worlds = int(sum(counts))
         self.gid0 = int(gid0)
 
-        self._keep = dict(
-            hull_off=np.ascontiguousarray(cmap.hull_off, np.int32),
-            vert=np.ascontiguousarray(cmap.vert, np.float64),
-            normal=np.ascontiguousarray(cmap.normal, np.float64),
-            edge_len=np.ascontiguousarray(cmap.edge_len, np.float64),
-            hull_bb=np.ascontiguousarray(cmap.hull_bb, np.float64),
-            init_pos=np.ascontiguousarray(cmap.init_pos, np.float64),
-            region_off=np.ascontiguousarray(cmap.region_off, np.int32),
-            regions=np.ascontiguousarray(cmap.regions if len(cmap.regions) else np.zeros((1, 4)), np.float64),
-            con_cell_off=np.ascontiguousarray(cmap.con_cell_off, np.int32),
-            con_cell_hulls=np.ascontiguousarray(np.append(cmap.con_cell_hulls, 0), np.int32),
-            view_cell_off=np.ascontiguousarray(cmap.view_cell_off, np.int32),
-            view_cell_edges=np.ascontiguousarray(np.append(cmap.view_cell_edges, 0), np.int32),
-        )
-        k = self._keep
-        md = CatMapDesc(
-            cmap.n_hulls, cmap.n_edges, _lib.np_ptr(k["hull_off"]), _lib.np_ptr(k["vert"]), _lib.np_ptr(k["normal"]),
-            _lib.np_ptr(k["edge_len"]), _lib.np_ptr(k["hull_bb"]), cmap.n_cops, cmap.n_thieves,
-            _lib.np_ptr(k["init_pos"]), _lib.np_ptr(k["region_off"]), _lib.np_ptr(k["regions"]),
-            cmap.grid_x0, cmap.grid_y0, cmap.cell, cmap.nx, cmap.ny,
-            _lib.np_ptr(k["con_cell_off"]), _lib.np_ptr(k["con_cell_hulls"]),
-            _lib.np_ptr(k["view_cell_off"]) if len(k["view_cell_off"]) == cmap.nx * cmap.ny + 1 else None,
-            _lib.np_ptr(k["view_cell_edges"]), float(cmap.view_range))
+        descs = [_map_desc(m) for m in cmaps]
+        self._keep = [kp for _, kp in descs]
         cp = CatParams(**{name: p[name] for name, _ in CatParams._fields_})
         handle = C.c_void_p()
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        _lib.check(self.L.cat_env_create(C.byref(md), C.byref(cp), self.n_worlds, self.gid0, dev_index,
-                                         C.byref(handle)), "cat_env_create")
+        if multi:
+            mds = (CatMapDesc * len(cmaps))(*[md for md, _ in descs])
+            cnt = (C.c_int32 * len(counts))(*counts)
+            _lib.check(self.L.cat_env_create_multi(mds, len(cmaps), cnt, C.byref(cp), self.gid0, dev_index,
+                                                   C.byref(handle)), "cat_env_create_multi")
+        else:
+            _lib.check(self.L.cat_env_create(C.byref(descs[0][0]), C.byref(cp), self.n_worlds, self.gid0, dev_index,
+                                             C.byref(handle)), "cat_env_create")
         self._h = handle
         info = CatEnvInfo()
         _lib.check(self.L.cat_env_info(self._h, C.byref(info)), "cat_env_info")
         self.info = info
         self.A, self.R, self.S, self.P = info.n_agents, info.n_rays, info.state_dim, info.n_pairs
         self.n_cops, self.n_thieves = info.n_cops, info.n_thieves
+        self.map_index = torch.repeat_interleave(torch.arange(len(cmaps), dtype=torch.int64),
+                                                 torch.tensor(counts, dtype=torch.int64)).to(self.device)
 
         N, A, R, dev = self.n_worlds, self.A, self.R, self.device
         nbytes = int(self.L.cat_env_state_bytes(self._h))
@@ -175,6 +210,12 @@ class CatWorlds:
                          dp(self.team_pos), dp(self.obs_f32), dp(self.state_f32), dp(self.hit_point), 0, 0,
                          rec.data_ptr(), self.packed_record_bytes if packed else self.record_bytes,
                          dp(self.critic_f32), dp(self.obs_bf16), dp(self.critic_bf16), 1 if packed else 0)
+
+    def map_info(self, m: int) -> CatEnvInfo:
+        """``cat_env_map_info``: the figures of map ``m`` alone (its worlds, hulls, edges, blob and ray-list bytes)."""
+        info = CatEnvInfo()
+        _lib.check(self.L.cat_env_map_info(self._h, int(m), C.byref(info)), "cat_env_map_info")
+        return info
 
     def overflow_counts(self, reset: bool = False):
         """(wall contacts beyond CAT_WALL_SLOTS, near hulls beyond CAT_NEAR_SLOTS) since creation / the last reset

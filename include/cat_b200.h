@@ -39,9 +39,10 @@
 extern "C" {
 #endif
 
-#define CAT_ABI_VERSION 5
+#define CAT_ABI_VERSION 6
 #define CAT_MAX_AGENTS 8
 #define CAT_MAX_RAYS 128
+#define CAT_MAX_MAPS 8 /* maps of one environment (cat_env_create_multi) */
 #define CAT_WALL_SLOTS 4 /* cached wall arbiters / simultaneous wall contacts kept per agent; a 5th is counted by
                             cat_env_overflow_counts, never dropped silently */
 #define CAT_NEAR_SLOTS 4 /* hulls whose reach can contain a ray origin (alpha = 0 rule) kept per agent; same rule */
@@ -164,7 +165,7 @@ typedef struct {
   int32_t map_blob_bytes;     /* bytes staged into shared memory per CTA */
   int32_t smem_bytes_per_cta;
   int32_t warps_per_cta;
-  int32_t grid;               /* CTAs launched by cat_env_step */
+  int32_t grid;               /* CTAs launched by cat_env_step (cat_env_map_info: those of them that step the map) */
   int32_t n_pairs;
   int32_t ray_list_cells;     /* cells of the (cell, ray) candidate-list grid, 0 = lists disabled */
   int32_t ray_list_nx, ray_list_ny;
@@ -196,8 +197,23 @@ const char* cat_last_error(void);
  * this rank's world 0 (spawn RNG is keyed by global world id). */
 int cat_env_create(const CatMapDesc* map, const CatParams* params, int32_t n_worlds, int64_t gid0,
                    int32_t device, CatEnv** out);
+/* One environment whose worlds run on several maps (mixed-map training), stepped by one launch per call: map m owns
+ * the worlds [off_m, off_m + worlds_per_map[m]), off_m = the sum of the counts before it, and world i of the
+ * environment is the same world as world i - off_m of a cat_env_create environment of map m with gid0 + off_m.
+ * Every map must have the same numbers of cops and thieves (the rays and constants come from `params`, so the
+ * observation, state and record layouts are the same for every map).  Each map's (cell, ray) lists are shared with
+ * every other environment of that map on the device.  Returns CAT_ERR_INVALID for null pointers, n_maps < 1, a
+ * count < 1 or maps with different agent counts, and CAT_ERR_LIMIT for n_maps > CAT_MAX_MAPS; the arguments are
+ * checked before any CUDA call.  cat_env_create(map, params, n, gid0, device, out) is this call with one map.
+ * Every other entry point works on such an environment as on a single-map one. */
+int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map,
+                         const CatParams* params, int64_t gid0, int32_t device, CatEnv** out);
 int cat_env_destroy(CatEnv* env);
+/* n_worlds: every world of the environment; ray_list_bytes: the sum over its maps; map_blob_bytes: the largest blob;
+ * the other map-dependent fields (n_hulls, n_edges, ray_list_cells/nx/ny/cell) describe map 0 */
 int cat_env_info(const CatEnv* env, CatEnvInfo* info);
+/* the same figures for map `map` of the environment alone (n_worlds = that map's worlds, grid = its CTAs of a step) */
+int cat_env_map_info(const CatEnv* env, int32_t map, CatEnvInfo* info);
 int cat_env_record_layout(const CatEnv* env, CatRecordLayout* layout);
 /* the record with CatStepIO.record_packed_types != 0 (what cat_env_step_host moves when packed_types != 0) */
 int cat_env_packed_record_layout(const CatEnv* env, CatRecordLayout* layout);

@@ -4,6 +4,7 @@ reference's ``self_play_driver.py``.  One process per GPU under torchrun; worlds
 all-reduced over NCCL per minibatch.
 
     python tools/train_selfplay.py --map agh-map --worlds 4096 --iterations 2 --timesteps 256
+    python tools/train_selfplay.py --map squarinth,agh-map,labyrinth --worlds 4096   # one policy over three maps
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_selfplay.py ...
 
 Prints one JSON line per self-play iteration (rank 0): environment agent-steps/s inside training, GAE / update /
@@ -28,7 +29,9 @@ from as_cops_and_thieves_b200.sharding import dist_env, shard_range  # noqa: E40
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--map", default="agh-map")
+    ap.add_argument("--map", default="agh-map",
+                    help="built-in map, or a comma-separated list of them: one mixed-map environment whose worlds are "
+                         "split evenly over the maps (every rank hosts the same split)")
     ap.add_argument("--worlds", type=int, default=4096, help="worlds per GPU")
     ap.add_argument("--iterations", type=int, default=2)
     ap.add_argument("--timesteps", type=int, default=256, help="lockstep steps per self-play iteration")
@@ -51,10 +54,16 @@ def main():
         import torch.distributed as dist
         os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
         dist.init_process_group("nccl", device_id=dev)
-    m = load_named_map(a.map)
+    names = [n.strip() for n in a.map.split(",") if n.strip()]
+    maps = [load_named_map(n) for n in names]
     gid0, n_local = shard_range(a.worlds * world_size, rank, world_size)
-    env = BatchedCopsThievesEnv(m, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
-                                spawn_override=free_space_regions(m) if a.free_spawn else None)
+    spawn = [free_space_regions(m) if a.free_spawn else None for m in maps]
+    if len(maps) == 1:
+        env = BatchedCopsThievesEnv(maps[0], n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
+                                    spawn_override=spawn[0])
+    else:
+        env = BatchedCopsThievesEnv(maps, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
+                                    spawn_override=spawn)
     # the reference's schedule (10 000 random / 15 000 before learning / 15 000 frozen policy) counts steps of ONE
     # environment; with thousands of lockstep worlds the same number of TRANSITIONS is reached in a few steps, so the
     # driver scales the durations by the world count unless told otherwise
