@@ -110,11 +110,11 @@ static void ray_lists_release(SharedRayLists* sh) {
 struct EnvMap {
   unsigned char* blob_dev = nullptr;
   int blob_bytes = 0;
+  BlobHeader header{};                   // the header of the uploaded blob: the map's one device description
   int32_t* view_off_dev = nullptr;
   uint16_t* view_edges_dev = nullptr;
   SharedRayLists* ray_lists = nullptr;   // shared with the other environments of this map on this device
   int world_begin = 0, n_worlds = 0;
-  int n_hulls = 0, n_edges = 0;
 };
 
 struct CatEnv {
@@ -412,6 +412,60 @@ static int acquire_ray_lists(const CatMapDesc* map, const CatParams* pr, int dev
   return CAT_OK;
 }
 
+// Upload one map into `em`: its view lists, its share of the (cell, ray) lists and its blob, whose header (kept in
+// em.header) then points at the lists.  On failure whatever was allocated is left in `em` for cat_env_destroy.
+static int upload_map(const CatMapDesc* md, const CatParams* pr, int device, EnvMap& em) {
+#define UPLOAD_TRY(expr, what)                                                                              \
+  do {                                                                                                      \
+    cudaError_t _e = (expr);                                                                                \
+    if (_e != cudaSuccess) return fail(CAT_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(_e));    \
+  } while (0)
+  std::vector<unsigned char> blob = build_blob(md, pr);
+  BlobHeader& hd = em.header;
+  memcpy(&hd, blob.data(), sizeof(hd));
+  const int E = md->n_edges, ncell = md->nx * md->ny;
+  // per-cell candidate lists (optional; valid only if they were built for at least this sensor range)
+  // Worth it only when the full scan is long: the lists live in global memory (two dependent loads per sweep,
+  // cold after an L2 flush), and a map of a few dozen edges is scanned in one or two batches anyway.
+  if (md->view_cell_off && md->view_cell_edges && E >= 96 &&
+      md->view_range >= pr->ray_length + pr->wall_radius + pr->ray_radius) {
+    const int n_list = md->view_cell_off[ncell];
+    std::vector<uint16_t> ve((size_t)(n_list > 0 ? n_list : 1));
+    for (int i = 0; i < n_list; ++i) ve[i] = (uint16_t)md->view_cell_edges[i];
+    UPLOAD_TRY(cudaMalloc(&em.view_off_dev, sizeof(int32_t) * (ncell + 1)), "cudaMalloc(view lists)");
+    UPLOAD_TRY(cudaMalloc(&em.view_edges_dev, sizeof(uint16_t) * ve.size()), "cudaMalloc(view lists)");
+    UPLOAD_TRY(cudaMemcpy(em.view_off_dev, md->view_cell_off, sizeof(int32_t) * (ncell + 1), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
+    UPLOAD_TRY(cudaMemcpy(em.view_edges_dev, ve.data(), sizeof(uint16_t) * ve.size(), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
+    hd.view_off = em.view_off_dev; hd.view_edges = em.view_edges_dev;
+  }
+  // per-(cell, ray) candidate lists of the sensor sweep (ray_lists.h), built from the map description
+  if (!(pr->ray_list_cell < 0.0)) {
+    const int rc = acquire_ray_lists(md, pr, device, &em.ray_lists);
+    if (rc != CAT_OK) return rc;
+    const SharedRayLists* sh = em.ray_lists;
+    hd.ray_slots = sh->slots_dev; hd.ray_ovf = sh->ovf_dev;
+    hd.ray_slot_count = (unsigned)(sh->slot_words / 4); hd.ray_ovf_words = (unsigned)sh->ovf_words;
+    hd.rg_x0 = sh->g.x0; hd.rg_y0 = sh->g.y0; hd.rg_inv_cell = sh->g.inv_cell; hd.rg_nx = sh->g.nx; hd.rg_ny = sh->g.ny;
+  }
+  memcpy(blob.data(), &hd, sizeof(hd));
+  em.blob_bytes = (int)blob.size();
+  UPLOAD_TRY(cudaMalloc(&em.blob_dev, em.blob_bytes), "cudaMalloc(map blob)");
+  UPLOAD_TRY(cudaMemcpy(em.blob_dev, blob.data(), em.blob_bytes, cudaMemcpyHostToDevice), "cudaMemcpy(map blob)");
+#undef UPLOAD_TRY
+  return CAT_OK;
+}
+
+// Map m's own figures in `inf`: its worlds, hulls, edges, blob, CTAs of a full launch and (cell, ray) lists.
+static void map_info(const CatEnv* env, int m, CatEnvInfo& inf) {
+  const EnvMap& em = env->maps[m];
+  const SharedRayLists* sh = em.ray_lists;
+  inf.n_worlds = em.n_worlds; inf.n_hulls = em.header.n_hulls; inf.n_edges = em.header.n_edges; inf.map_blob_bytes = em.blob_bytes;
+  inf.grid = (m + 1 < env->kp.n_maps ? env->kp.maps[m + 1].cta_begin : env->grid) - env->kp.maps[m].cta_begin;
+  inf.ray_list_nx = em.header.rg_nx; inf.ray_list_ny = em.header.rg_ny; inf.ray_list_cells = inf.ray_list_nx * inf.ray_list_ny;
+  inf.ray_list_cell = sh ? sh->g.cell : 0.f;
+  inf.ray_list_bytes = sh ? (int64_t)(sh->slot_words + sh->ovf_words) * 4 : 0;
+}
+
 int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds, int64_t gid0, int32_t device,
                    CatEnv** out) {
   if (!map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
@@ -438,9 +492,6 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
   const int n_worlds = (int)total;
   const int A = map->n_cops + map->n_thieves, R = pr->n_rays;
   const int P = A * (A - 1) / 2;
-  std::vector<std::vector<unsigned char>> blobs;
-  for (int m = 0; m < n_maps; ++m) blobs.push_back(build_blob(&maps[m], pr));
-
   CatEnv* env = new CatEnv();
   env->device = device;
   env->n_worlds = n_worlds;
@@ -455,65 +506,27 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
   CREATE_TRY(cudaMalloc(&env->overflow_dev, 2 * sizeof(unsigned long long)), "cudaMalloc(overflow counters)");
   CREATE_TRY(cudaMemset(env->overflow_dev, 0, 2 * sizeof(unsigned long long)), "cudaMemset(overflow counters)");
   env->maps.resize(n_maps);
-  CatEnvInfo& inf = env->info;
-  int64_t ray_list_bytes = 0;
   for (int m = 0, w0 = 0; m < n_maps; w0 += worlds_per_map[m], ++m) {
-    const CatMapDesc* md = &maps[m];
     EnvMap& em = env->maps[m];
     em.world_begin = w0; em.n_worlds = worlds_per_map[m];
-    em.n_hulls = md->n_hulls; em.n_edges = md->n_edges;
-    std::vector<unsigned char>& blob = blobs[m];
-    BlobHeader hd;
-    memcpy(&hd, blob.data(), sizeof(hd));
-    const int E = md->n_edges, ncell = md->nx * md->ny;
-    // per-cell candidate lists (optional; valid only if they were built for at least this sensor range)
-    // Worth it only when the full scan is long: the lists live in global memory (two dependent loads per sweep,
-    // cold after an L2 flush), and a map of a few dozen edges is scanned in one or two batches anyway.
-    if (md->view_cell_off && md->view_cell_edges && E >= 96 &&
-        md->view_range >= pr->ray_length + pr->wall_radius + pr->ray_radius) {
-      const int n_list = md->view_cell_off[ncell];
-      std::vector<uint16_t> ve((size_t)(n_list > 0 ? n_list : 1));
-      for (int i = 0; i < n_list; ++i) ve[i] = (uint16_t)md->view_cell_edges[i];
-      CREATE_TRY(cudaMalloc(&em.view_off_dev, sizeof(int32_t) * (ncell + 1)), "cudaMalloc(view lists)");
-      CREATE_TRY(cudaMalloc(&em.view_edges_dev, sizeof(uint16_t) * ve.size()), "cudaMalloc(view lists)");
-      CREATE_TRY(cudaMemcpy(em.view_off_dev, md->view_cell_off, sizeof(int32_t) * (ncell + 1), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
-      CREATE_TRY(cudaMemcpy(em.view_edges_dev, ve.data(), sizeof(uint16_t) * ve.size(), cudaMemcpyHostToDevice), "cudaMemcpy(view lists)");
-      hd.view_off = em.view_off_dev; hd.view_edges = em.view_edges_dev;
-    }
-    // per-(cell, ray) candidate lists of the sensor sweep (ray_lists.h), built from the map description
-    if (!(pr->ray_list_cell < 0.0)) {
-      const int rc = acquire_ray_lists(md, pr, device, &em.ray_lists);
-      if (rc != CAT_OK) { cat_env_destroy(env); return rc; }
-      const SharedRayLists* sh = em.ray_lists;
-      hd.ray_slots = sh->slots_dev; hd.ray_ovf = sh->ovf_dev;
-      hd.ray_slot_count = (unsigned)(sh->slot_words / 4); hd.ray_ovf_words = (unsigned)sh->ovf_words;
-      hd.rg_x0 = sh->g.x0; hd.rg_y0 = sh->g.y0; hd.rg_inv_cell = sh->g.inv_cell; hd.rg_nx = sh->g.nx; hd.rg_ny = sh->g.ny;
-      ray_list_bytes += (int64_t)(sh->slot_words + sh->ovf_words) * 4;
-    }
-    memcpy(blob.data(), &hd, sizeof(hd));
-    em.blob_bytes = (int)blob.size();
-    CREATE_TRY(cudaMalloc(&em.blob_dev, em.blob_bytes), "cudaMalloc(map blob)");
-    CREATE_TRY(cudaMemcpy(em.blob_dev, blob.data(), em.blob_bytes, cudaMemcpyHostToDevice), "cudaMemcpy(map blob)");
+    const int rc = upload_map(&maps[m], pr, device, em);
+    if (rc != CAT_OK) { cat_env_destroy(env); return rc; }
     env->blob_bytes = std::max(env->blob_bytes, em.blob_bytes);
   }
 
   KParams& k = env->kp;
   {   // map 0's values: what a single-map launch reads (a mixed-map launch reads each map's from its blob header)
     const EnvMap& em = env->maps[0];
+    const BlobHeader& h = em.header;
     k.blob = em.blob_dev; k.blob_bytes = em.blob_bytes;
-    k.view_off = em.view_off_dev; k.view_edges = em.view_edges_dev;
-    if (const SharedRayLists* sh = em.ray_lists) {
-      k.ray_slots = sh->slots_dev; k.ray_ovf = sh->ovf_dev;
-      k.ray_slot_count = (unsigned)(sh->slot_words / 4); k.ray_ovf_words = (unsigned)sh->ovf_words;
-      k.rg_x0 = sh->g.x0; k.rg_y0 = sh->g.y0; k.rg_inv_cell = sh->g.inv_cell; k.rg_nx = sh->g.nx; k.rg_ny = sh->g.ny;
-      inf.ray_list_cells = sh->g.nx * sh->g.ny; inf.ray_list_nx = sh->g.nx; inf.ray_list_ny = sh->g.ny; inf.ray_list_cell = sh->g.cell;
-    }
-    inf.ray_list_bytes = ray_list_bytes;
+    k.view_off = h.view_off; k.view_edges = h.view_edges;
+    k.ray_slots = h.ray_slots; k.ray_ovf = h.ray_ovf; k.ray_slot_count = h.ray_slot_count; k.ray_ovf_words = h.ray_ovf_words;
+    k.rg_x0 = h.rg_x0; k.rg_y0 = h.rg_y0; k.rg_inv_cell = h.rg_inv_cell; k.rg_nx = h.rg_nx; k.rg_ny = h.rg_ny;
+    k.n_edges = h.n_edges;
   }
   k.overflow = env->overflow_dev;
   k.n_worlds = n_worlds; k.gid0 = gid0;
   k.A = A; k.nc = map->n_cops; k.R = R;
-  k.n_edges = map->n_edges;
   k.lay = make_layout(A, R);          // record / scratch / output-record offsets (world_kernel.cuh)
   CatRecordLayout& rc = env->rec;
   rc.off_dist = 0; rc.off_type = k.lay.r_off_type; rc.off_reward = k.lay.r_off_reward;
@@ -561,8 +574,12 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
   env->threads = shp.threads; env->smem_bytes = shp.smem;
   env->grid = fill_map_table(env, k, 0, n_worlds, shp.grid, shp.threads / 32);   // the table every full launch uses
 
+  // the environment's figures: map 0's, then the totals over the maps (worlds, list bytes, the largest blob, the grid)
+  CatEnvInfo& inf = env->info;
+  map_info(env, 0, inf);
+  for (int m = 1; m < n_maps; ++m) { CatEnvInfo other{}; map_info(env, m, other); inf.ray_list_bytes += other.ray_list_bytes; }
   inf.n_worlds = n_worlds; inf.n_agents = A; inf.n_cops = map->n_cops; inf.n_thieves = map->n_thieves;
-  inf.n_rays = R; inf.n_hulls = map->n_hulls; inf.n_edges = map->n_edges; inf.state_dim = k.state_dim; inf.record_words = k.lay.rec_words;
+  inf.n_rays = R; inf.state_dim = k.state_dim; inf.record_words = k.lay.rec_words;
   inf.map_blob_bytes = env->blob_bytes; inf.smem_bytes_per_cta = env->smem_bytes; inf.warps_per_cta = env->threads / 32;
   inf.grid = env->grid; inf.n_pairs = P;
 #undef CREATE_TRY
@@ -596,15 +613,8 @@ int cat_env_info(const CatEnv* env, CatEnvInfo* info) {
 int cat_env_map_info(const CatEnv* env, int32_t map, CatEnvInfo* info) {
   if (!env || !info) return fail(CAT_ERR_INVALID, "null argument");
   if (map < 0 || map >= (int)env->maps.size()) return fail(CAT_ERR_INVALID, "map index out of range");
-  const EnvMap& m = env->maps[map];
   CatEnvInfo inf = env->info;
-  inf.n_worlds = m.n_worlds; inf.n_hulls = m.n_hulls; inf.n_edges = m.n_edges; inf.map_blob_bytes = m.blob_bytes;
-  inf.grid = (map + 1 < env->kp.n_maps ? env->kp.maps[map + 1].cta_begin : env->grid) - env->kp.maps[map].cta_begin;
-  inf.ray_list_cells = 0; inf.ray_list_nx = 0; inf.ray_list_ny = 0; inf.ray_list_cell = 0.f; inf.ray_list_bytes = 0;
-  if (const SharedRayLists* sh = m.ray_lists) {
-    inf.ray_list_cells = sh->g.nx * sh->g.ny; inf.ray_list_nx = sh->g.nx; inf.ray_list_ny = sh->g.ny; inf.ray_list_cell = sh->g.cell;
-    inf.ray_list_bytes = (int64_t)(sh->slot_words + sh->ovf_words) * 4;
-  }
+  map_info(env, map, inf);
   *info = inf;
   return CAT_OK;
 }
