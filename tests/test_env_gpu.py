@@ -258,7 +258,8 @@ def test_gae_statistics_buffer_protocol(cuda_device):
     g = torch.Generator().manual_seed(3)
     stats = torch.zeros(6, dtype=torch.float64, device=cuda_device)
     stream = torch.cuda.current_stream(cuda_device).cuda_stream
-    for call, (T, M) in enumerate(((40, 4096), (7, 33), (300, 64), (64, 1600)), start=1):
+    # (256, 49152): the bench size, 768 TMA CTAs in about 1.3 waves drawing tickets and adding their sums
+    for call, (T, M) in enumerate(((40, 4096), (7, 33), (300, 64), (64, 1600), (256, 49152)), start=1):
         r = torch.randn((T, M), generator=g).to(cuda_device)
         v = torch.randn((T, M), generator=g).to(cuda_device)
         d = (torch.rand((T, M), generator=g) < 0.05).to(torch.uint8).to(cuda_device)
