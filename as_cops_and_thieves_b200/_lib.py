@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-CAT_ABI_VERSION = 6
+CAT_ABI_VERSION = 7
 CAT_MAX_AGENTS = 8
 CAT_MAX_RAYS = 128
 CAT_MAX_MAPS = 8
@@ -83,6 +83,15 @@ class CatStateView(C.Structure):
         "pair_age", "pair_jn")]
 
 
+class CatRenderIO(C.Structure):
+    _fields_ = [
+        ("n_frames", C.c_int32), ("world", C.c_void_p), ("n_elements", C.c_int64), ("map_of", C.c_void_p),
+        ("pos", C.c_void_p), ("pos_stride", C.c_int64), ("ray_dist", C.c_void_p), ("ray_dist_stride", C.c_int64),
+        ("ray_type", C.c_void_p), ("ray_type_stride", C.c_int64), ("downsample", C.c_int32),
+        ("agent_radius", C.c_double), ("frames", C.c_void_p),
+    ]
+
+
 #: every symbol ``include/cat_b200.h`` declares
 EXPORTS = (
     "cat_abi_version", "cat_last_error", "cat_env_create", "cat_env_create_multi", "cat_env_destroy", "cat_env_info",
@@ -90,6 +99,7 @@ EXPORTS = (
     "cat_env_record_layout", "cat_env_packed_record_layout", "cat_env_overflow_counts", "cat_ray_lists_host",
     "cat_env_set_seed", "cat_env_state_bytes", "cat_env_init_state", "cat_env_reset", "cat_env_step", "cat_env_step_host", "cat_env_observe",
     "cat_env_get_state", "cat_env_set_state", "cat_gae", "cat_adv_normalize",
+    "cat_renderer_create", "cat_renderer_destroy", "cat_renderer_frame_size", "cat_render", "cat_ray_directions",
 )
 
 _LIB = None
@@ -138,6 +148,12 @@ def load():
         fn.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(CatStateView), C.c_void_p]
     L.cat_gae.argtypes = [C.c_void_p] * 7 + [C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_void_p]
     L.cat_adv_normalize.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+    L.cat_renderer_create.argtypes = [C.POINTER(CatMapDesc), C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int32,
+                                      C.POINTER(C.c_void_p)]
+    L.cat_renderer_destroy.argtypes = [C.c_void_p]
+    L.cat_renderer_frame_size.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+    L.cat_render.argtypes = [C.c_void_p, C.POINTER(CatRenderIO), C.c_void_p]
+    L.cat_ray_directions.argtypes = [C.c_int32, C.c_void_p]
     _LIB = L
     return L
 

@@ -57,6 +57,7 @@ int fail(int code, const std::string& msg) {
 #include "world_kernel.cuh"
 #include "state_view.cuh"
 #include "gae_kernels.cuh"
+#include "render_kernel.cuh"
 
 inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 
@@ -272,6 +273,13 @@ static int check_map(const CatMapDesc* map, const CatParams* pr) {
   return CAT_OK;
 }
 
+// The fp32 ray directions of every consumer (the step's blob, the renderer, cat_ray_directions): out[2 i], out[2 i + 1]
+// = cos, sin of i 2 pi / R (entity.py:182 linspace(0, 2pi, R, endpoint=False)).
+static void ray_directions(int R, float* out) {
+  const double step = (2.0 * M_PI) / (double)R;
+  for (int i = 0; i < R; ++i) { out[2 * i] = (float)cos(i * step); out[2 * i + 1] = (float)sin(i * step); }
+}
+
 // The shared-memory blob of one map (BlobHeader + arrays).  The header's global-memory table pointers are left zero:
 // the caller fills them in once the tables are on the device.
 static std::vector<unsigned char> build_blob(const CatMapDesc* map, const CatParams* pr) {
@@ -334,9 +342,10 @@ static std::vector<unsigned char> build_blob(const CatMapDesc* map, const CatPar
     uint16_t* cl = reinterpret_cast<uint16_t*>(blob.data() + hd.off_conlist);
     for (int i = 0; i < map->con_cell_off[ncell]; ++i) cl[i] = (uint16_t)map->con_cell_hulls[i];
     float* dir = reinterpret_cast<float*>(blob.data() + hd.off_dir);
-    const double step = (2.0 * M_PI) / (double)R;  // entity.py:182 linspace(0, 2pi, R, endpoint=False)
+    std::vector<float> u(2 * R);
+    ray_directions(R, u.data());
     for (int i = 0; i < R; ++i) {
-      const float ux = (float)cos(i * step), uy = (float)sin(i * step);
+      const float ux = u[2 * i], uy = u[2 * i + 1];
       dir[4 * i] = ux; dir[4 * i + 1] = uy;
       dir[4 * i + 2] = ux != 0.f ? 1.f / ux : 0.f; dir[4 * i + 3] = uy != 0.f ? 1.f / uy : 0.f;
     }
@@ -879,6 +888,156 @@ int cat_adv_normalize(float* advantages, int64_t n, const double* stats_dev, int
   if (blocks < 1) blocks = 1;
   if (blocks > 148 * 16) blocks = 148 * 16;
   CUDA_TRY(launch_pdl(cat_adv_normalize_kernel, (int)blocks, threads, 0, reinterpret_cast<cudaStream_t>(stream), advantages, (long long)n, stats_dev, (long long)count));
+  CUDA_TRY(cudaGetLastError());
+  return CAT_OK;
+}
+
+
+// ---- renderer (render_kernel.cuh)
+struct CatRenderer {
+  int device = 0, n_maps = 0, A = 0, nc = 0, R = 0, Wmax = 0, Hmax = 0;
+  RenderMap maps[CAT_MAX_MAPS] = {};
+  float2* dirs_dev = nullptr;
+};
+
+int cat_renderer_destroy(CatRenderer* r) {
+  if (!r) return CAT_OK;
+  DeviceGuard guard(r->device);
+  for (int m = 0; m < r->n_maps; ++m)
+    if (r->maps[m].wall) cudaFree(const_cast<uint32_t*>(r->maps[m].wall));
+  if (r->dirs_dev) cudaFree(r->dirs_dev);
+  delete r;
+  return CAT_OK;
+}
+
+// Map m's wall layer: the hulls go to the device in fp64 (with render_rgb's clip boxes), one kernel sets the bits.
+static int build_wall_layer(const CatMapDesc* md, int W, int H, RenderMap& rm) {
+  const int nh = md->n_hulls, ne = md->n_edges;
+  rm.W = W; rm.H = H; rm.hwords = (H + 31) / 32;
+  std::vector<WallHull> hulls(nh > 0 ? nh : 1);
+  for (int h = 0; h < nh; ++h) {
+    const double* bb = md->hull_bb + 4 * h;   // l, b, r, t; render_rgb: [max(0, floor(l - 1)), min(W, ceil(r + 1) + 1))
+    auto lo = [](double v) { return (int)std::max(0.0, std::min(1e9, floor(v - 1.0))); };
+    auto hi = [](double v, int n) { return (int)std::min((double)n, std::max(-1.0, ceil(v + 1.0) + 1.0)); };
+    hulls[h] = WallHull{md->hull_off[h], md->hull_off[h + 1], lo(bb[0]), hi(bb[2], W), lo(bb[1]), hi(bb[3], H)};
+  }
+  const size_t words = (size_t)W * rm.hwords;
+  WallHull* hulls_dev = nullptr;
+  double2 *vert_dev = nullptr, *normal_dev = nullptr;
+  uint32_t* bits = nullptr;
+  cudaError_t e = cudaMalloc(&bits, words * 4);
+  if (e == cudaSuccess) rm.wall = bits;
+  if (e == cudaSuccess) e = cudaMalloc(&hulls_dev, sizeof(WallHull) * hulls.size());
+  if (e == cudaSuccess) e = cudaMalloc(&vert_dev, sizeof(double2) * (ne > 0 ? ne : 1));
+  if (e == cudaSuccess) e = cudaMalloc(&normal_dev, sizeof(double2) * (ne > 0 ? ne : 1));
+  if (e == cudaSuccess) e = cudaMemcpy(hulls_dev, hulls.data(), sizeof(WallHull) * hulls.size(), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && ne > 0) e = cudaMemcpy(vert_dev, md->vert, sizeof(double2) * ne, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && ne > 0) e = cudaMemcpy(normal_dev, md->normal, sizeof(double2) * ne, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    const long long n = (long long)words * 32;
+    cat_wall_bits_kernel<<<(unsigned)((n + 255) / 256), 256>>>(hulls_dev, nh, vert_dev, normal_dev, H, rm.hwords, n, bits);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (hulls_dev) cudaFree(hulls_dev);
+  if (vert_dev) cudaFree(vert_dev);
+  if (normal_dev) cudaFree(normal_dev);
+  return e == cudaSuccess ? CAT_OK : fail(CAT_ERR_CUDA, std::string("renderer wall layer: ") + cudaGetErrorString(e));
+}
+
+int cat_renderer_create(const CatMapDesc* maps, const int32_t* windows, int32_t n_maps, int32_t n_rays, int32_t device,
+                        CatRenderer** out) {
+  if (!maps || !windows || !out) return fail(CAT_ERR_INVALID, "null argument");
+  *out = nullptr;
+  if (n_maps < 1) return fail(CAT_ERR_INVALID, "n_maps must be >= 1");
+  if (n_maps > CAT_MAX_MAPS) return fail(CAT_ERR_LIMIT, "too many maps (CAT_MAX_MAPS)");
+  if (n_rays < 2 || n_rays > CAT_MAX_RAYS) return fail(CAT_ERR_LIMIT, "n_rays out of range (2..CAT_MAX_RAYS)");
+  for (int m = 0; m < n_maps; ++m) {
+    const CatMapDesc& md = maps[m];
+    if (windows[2 * m] < 1 || windows[2 * m] > 8192 || windows[2 * m + 1] < 1 || windows[2 * m + 1] > 8192)
+      return fail(CAT_ERR_INVALID, "window sides must be in 1..8192");
+    if (md.n_cops < 1 || md.n_thieves < 1) return fail(CAT_ERR_INVALID, "need at least one cop and one thief");
+    if (md.n_cops + md.n_thieves > CAT_MAX_AGENTS) return fail(CAT_ERR_LIMIT, "too many agents (CAT_MAX_AGENTS)");
+    if (md.n_cops != maps[0].n_cops || md.n_thieves != maps[0].n_thieves)
+      return fail(CAT_ERR_INVALID, "every map of a renderer needs the same numbers of cops and thieves");
+    if (md.n_hulls < 0 || md.n_edges < 0) return fail(CAT_ERR_INVALID, "negative hull / edge count");
+    if (md.n_hulls > 0 && (!md.hull_off || !md.vert || !md.normal || !md.hull_bb)) return fail(CAT_ERR_INVALID, "null hull array");
+  }
+  CatRenderer* r = new CatRenderer();
+  r->device = device; r->n_maps = n_maps; r->nc = maps[0].n_cops; r->A = maps[0].n_cops + maps[0].n_thieves; r->R = n_rays;
+  DeviceGuard guard(device);
+  if (!guard.ok) { delete r; return fail(CAT_ERR_CUDA, "cudaSetDevice(" + std::to_string(device) + ") failed (no CUDA device?)"); }
+  for (int m = 0; m < n_maps; ++m) {
+    r->Wmax = std::max(r->Wmax, (int)windows[2 * m]); r->Hmax = std::max(r->Hmax, (int)windows[2 * m + 1]);
+    const int rc = build_wall_layer(&maps[m], windows[2 * m], windows[2 * m + 1], r->maps[m]);
+    if (rc != CAT_OK) { cat_renderer_destroy(r); return rc; }
+  }
+  std::vector<float> u(2 * n_rays);
+  ray_directions(n_rays, u.data());
+  cudaError_t e = cudaMalloc(&r->dirs_dev, sizeof(float2) * n_rays);
+  if (e == cudaSuccess) e = cudaMemcpy(r->dirs_dev, u.data(), sizeof(float2) * n_rays, cudaMemcpyHostToDevice);
+  // the largest frame table any renderer needs (CAT_MAX_AGENTS x CAT_MAX_RAYS segments); a per-function attribute
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(cat_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, render_smem_bytes(CAT_MAX_AGENTS * CAT_MAX_RAYS));
+  if (e != cudaSuccess) { cat_renderer_destroy(r); return fail(CAT_ERR_CUDA, std::string("cat_renderer_create: ") + cudaGetErrorString(e)); }
+  *out = r;
+  return CAT_OK;
+}
+
+static int frame_size(const CatRenderer* r, int d, int* w, int* h) {
+  if (d < 1) return fail(CAT_ERR_INVALID, "downsample must be >= 1");
+  *w = (r->Wmax - d / 2 + d - 1) / d; *h = (r->Hmax - d / 2 + d - 1) / d;
+  if (*w < 1 || *h < 1) return fail(CAT_ERR_INVALID, "downsample leaves an empty frame");
+  return CAT_OK;
+}
+
+int cat_renderer_frame_size(const CatRenderer* r, int32_t downsample, int32_t* w, int32_t* h) {
+  if (!r || !w || !h) return fail(CAT_ERR_INVALID, "null argument");
+  return frame_size(r, downsample, w, h);
+}
+
+int cat_ray_directions(int32_t n_rays, float* out) {
+  if (!out) return fail(CAT_ERR_INVALID, "null argument");
+  if (n_rays < 2 || n_rays > CAT_MAX_RAYS) return fail(CAT_ERR_LIMIT, "n_rays out of range (2..CAT_MAX_RAYS)");
+  ray_directions(n_rays, out);
+  return CAT_OK;
+}
+
+int cat_render(const CatRenderer* r, const CatRenderIO* io, void* stream) {
+  if (!r || !io) return fail(CAT_ERR_INVALID, "null argument");
+  if (io->n_frames < 0) return fail(CAT_ERR_INVALID, "n_frames must be >= 0");
+  if (io->n_elements < 0) return fail(CAT_ERR_INVALID, "n_elements must be >= 0");
+  if (io->downsample < 1) return fail(CAT_ERR_INVALID, "downsample must be >= 1");
+  if (!io->pos || !io->frames) return fail(CAT_ERR_INVALID, "null pos / frames");
+  if ((reinterpret_cast<uintptr_t>(io->pos) & 3) || (io->pos_stride & 3))
+    return fail(CAT_ERR_INVALID, "pos must be 4-byte aligned with a stride that is a multiple of 4");
+  if (!io->ray_dist != !io->ray_type) return fail(CAT_ERR_INVALID, "ray_dist and ray_type go together");
+  if (io->ray_dist && ((reinterpret_cast<uintptr_t>(io->ray_dist) & 1) || (io->ray_dist_stride & 1)))
+    return fail(CAT_ERR_INVALID, "ray_dist must be 2-byte aligned with an even stride");
+  if (!(io->agent_radius >= 0.0) || !isfinite(io->agent_radius)) return fail(CAT_ERR_INVALID, "agent_radius must be finite and >= 0");
+  // the checks that need the renderer's figures
+  const int A = r->A, R = r->R;
+  if (io->pos_stride < 8 * A) return fail(CAT_ERR_INVALID, "pos stride smaller than 8 * n_agents");
+  if (io->ray_dist && (io->ray_dist_stride < 2LL * A * R || io->ray_type_stride < (long long)A * R))
+    return fail(CAT_ERR_INVALID, "ray strides smaller than one element's block");
+  RenderParams p{};
+  const int rc = frame_size(r, io->downsample, &p.Wd, &p.Hd);
+  if (rc != CAT_OK) return rc;
+  p.tiles_y = (p.Hd + kRenderTY - 1) / kRenderTY;
+  p.tiles = (p.Wd + kRenderTX - 1) / kRenderTX * p.tiles_y;
+  if ((long long)io->n_frames * p.tiles > 0x7FFFFFFFLL) return fail(CAT_ERR_LIMIT, "too many frames for one launch");
+  if (io->n_frames == 0) return CAT_OK;
+  for (int m = 0; m < r->n_maps; ++m) p.maps[m] = r->maps[m];
+  p.n_maps = r->n_maps; p.A = A; p.nc = r->nc; p.R = R; p.dirs = r->dirs_dev;
+  p.n_elements = io->n_elements; p.world = io->world; p.map_of = io->map_of;
+  p.pos = static_cast<const unsigned char*>(io->pos); p.pos_stride = io->pos_stride;
+  p.ray_dist = static_cast<const unsigned char*>(io->ray_dist); p.dist_stride = io->ray_dist_stride;
+  p.ray_type = static_cast<const unsigned char*>(io->ray_type); p.type_stride = io->ray_type_stride;
+  p.d = io->downsample; p.radius = io->agent_radius; p.radius2 = pow(io->agent_radius, 2.0);
+  p.frames = io->frames;
+  DEVICE_SCOPE(r);
+  const int smem = render_smem_bytes(io->ray_dist ? A * R : 0);
+  cat_render_kernel<<<(unsigned)((long long)io->n_frames * p.tiles), kRenderThreads, smem, reinterpret_cast<cudaStream_t>(stream)>>>(p);
   CUDA_TRY(cudaGetLastError());
   return CAT_OK;
 }

@@ -221,10 +221,9 @@ class BaseEnv(_EnvCommon, _ParallelEnvBase):
         return self._state
 
     def render(self):
+        """``rgb_array``: the world drawn on the GPU, ``render.render_rgb`` bit for bit (numpy (W, H, 3) uint8)."""
         if self.render_mode == "rgb_array":
-            from .render import render_rgb
-            pos = self._w.get_state()["pos"][0].cpu().numpy()
-            return render_rgb(self._cmap, pos)
+            return self._w.render_frames()[0].cpu().numpy()
         return None
 
     def close(self):
@@ -361,10 +360,15 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         return self._w.critic_f32
 
     def render(self, world: int = 0):
-        """``rgb_array`` of one world, drawn on that world's own map."""
-        from .render import render_rgb
-        pos = self._w.get_state()["pos"][world].cpu().numpy()
-        return render_rgb(self._cmaps[int(self._w.map_index[world])], pos)
+        """``rgb_array`` of one world, drawn on that world's own map (numpy (W, H, 3) uint8 of that map's window):
+        ``render.render_rgb`` bit for bit, drawn on the GPU."""
+        cmap = self._cmaps[int(self._w.map_index[world])]
+        frame = self._w.render_frames([int(world)])[0]
+        return frame[:int(cmap.window[0]), :int(cmap.window[1])].cpu().numpy()
+
+    def render_frames(self, worlds=None, rays: bool = False, downsample: int = 1, out: Optional[torch.Tensor] = None):
+        """Frames of many worlds in one launch, on the device: ``CatWorlds.render_frames``."""
+        return self._w.render_frames(worlds, rays=rays, downsample=downsample, out=out)
 
     def close(self) -> None:
         self._w.close()

@@ -225,6 +225,9 @@ class CatWorlds:
         return int(out[0]), int(out[1])
 
     def close(self) -> None:
+        if getattr(self, "_renderer", None) is not None:
+            self._renderer.close()
+            self._renderer = None
         if getattr(self, "_h", None):
             self.L.cat_env_destroy(self._h)
             self._h = None
@@ -409,6 +412,53 @@ class CatWorlds:
     def observe(self) -> None:
         _lib.check(self.L.cat_env_observe(self._h, self.state.data_ptr(), C.byref(self._io), self._stream()),
                    "cat_env_observe")
+
+    # ------------------------------------------------------------------ frames (render.py)
+    def positions(self) -> torch.Tensor:
+        """(N, A, 2) float32 view of the agents' positions inside the packed state buffer (words 0 .. 2A-1 of each
+        world's record): read-only use, no copy."""
+        return self.state.view(torch.float32).as_strided((self.n_worlds, self.A, 2), (self.info.record_words, 2, 1))
+
+    def renderer(self):
+        """The ``render.Renderer`` of this environment's maps, created on first use (outside graph capture)."""
+        if getattr(self, "_renderer", None) is None:
+            from .render import Renderer
+            self._renderer = Renderer(self.cmaps, self.R, self.device)
+        return self._renderer
+
+    def render_frames(self, worlds=None, rays: bool = False, downsample: int = 1, out: Optional[torch.Tensor] = None,
+                      agent_radius: float = 5.0) -> torch.Tensor:
+        """``rgb_array`` frames (K, W', H', 3) uint8 on the device of the worlds ``worlds`` (None: every world; a
+        sequence or an int64 tensor, on the device under graph capture), one launch on the current stream; each frame is
+        ``render.render_rgb`` of the world's own map, zero-padded to the largest window, downsampled as
+        ``frame[d//2::d, d//2::d]``.
+
+        ``rays=True`` draws each agent's sensor rays as its sensor reports them from the drawn positions: it first runs
+        ``cat_env_observe`` into a private record buffer (observing writes no state back), so the environment's own
+        outputs are untouched, and for a world that does not end in the next step the overlay is that step's
+        observation bit for bit.  The renderer and the private buffer are created by the first call, which must
+        therefore happen outside CUDA-graph capture (as ``step_host``'s buffers do); later calls allocate nothing when
+        ``out`` is given and ``worlds`` is None or a device tensor."""
+        if worlds is not None and not (isinstance(worlds, torch.Tensor) and worlds.device == self.device
+                                       and worlds.dtype == torch.int64):
+            worlds = torch.as_tensor(worlds, dtype=torch.int64).reshape(-1).to(self.device)
+        return self.renderer().render(self.positions(), world=worlds, map_of=self.map_index,
+                                      rays=self.sensor_rays() if rays else None, downsample=downsample,
+                                      agent_radius=agent_radius, out=out)
+
+    def sensor_rays(self):
+        """(obs_dist (N, A, R) float16, obs_type (N, A, R) uint8): what every agent's sensor reports from the current
+        positions, written by ``cat_env_observe`` into a private record buffer (created by the first call) on the
+        current stream.  Neither the state nor the environment's outputs change.  The step computes its observation
+        before it moves the agents, so for a world that does not end in the next step this is that step's observation."""
+        if getattr(self, "_sensor_rec", None) is None:
+            self._sensor_rec = torch.zeros(self.n_worlds * self.record_bytes, dtype=torch.uint8, device=self.device)
+            self._sensor_io = CatStepIO(record=self._sensor_rec.data_ptr(), record_world_stride=self.record_bytes)
+            v = self._record_views(self._sensor_rec)
+            self._sensor_views = (v["obs_dist"], v["obs_type"])
+        _lib.check(self.L.cat_env_observe(self._h, self.state.data_ptr(), C.byref(self._sensor_io), self._stream()),
+                   "cat_env_observe")
+        return self._sensor_views
 
     # ------------------------------------------------------------------ state access (parity tests, checkpoints)
     def _view_tensors(self) -> Dict[str, torch.Tensor]:

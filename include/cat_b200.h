@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define CAT_ABI_VERSION 6
+#define CAT_ABI_VERSION 7
 #define CAT_MAX_AGENTS 8
 #define CAT_MAX_RAYS 128
 #define CAT_MAX_MAPS 8 /* maps of one environment (cat_env_create_multi) */
@@ -276,6 +276,49 @@ int cat_gae(const float* rewards, const uint8_t* dones, const float* values, con
  * has cat_gae's layout (pass the buffer cat_gae filled).  For a global normalisation across ranks, all-reduce the sums and
  * the count and pass a zeroed CAT_GAE_STATS_DOUBLES buffer with the reduced sums in [0..1] (calls = 0 selects slot 0). */
 int cat_adv_normalize(float* advantages, int64_t n, const double* stats_dev, int64_t count, void* stream);
+
+/* ---- Renderer: rgb_array frames of many worlds in one launch (python: render.Renderer, CatWorlds.render_frames).
+ * A renderer needs no CatEnv, so recorded trajectories can be drawn after their environment is gone.  A frame is the
+ * image render.render_rgb(cmap, pos, agent_radius, rays) returns, bit for bit: u8 [W][H][3] (the layout of
+ * pygame.surfarray.array3d), layers from first to last: black; the sensor rays when asked for (by ray type: wall
+ * (96, 96, 96), cop (0, 160, 255), thief (255, 160, 0), empty (40, 40, 40); a pixel is on ray i of agent a when its
+ * centre is within 0.5 of the segment from the agent's position P to P + dist[a][i] * direction[i], and a later
+ * (a, i) wins); walls (white); the agents in index order, cops (0, 0, 255), thieves (255, 0, 0).  A frame is
+ * (largest window width, largest window height) of the renderer's maps; pixels outside the frame's own map's window
+ * are zero.  With downsample d the frame is frame_1[d/2::d, d/2::d]: (W - d/2 + d - 1) / d by (H - d/2 + d - 1) / d. */
+typedef struct CatRenderer CatRenderer;
+
+typedef struct {
+  int32_t n_frames;          /* K */
+  const int64_t* world;      /* device [K]: the element frame k shows; NULL = k.  An id outside [0, n_elements) gives
+                                an all-zero frame, as does an element whose map_of is not a map of the renderer */
+  int64_t n_elements;
+  const int64_t* map_of;     /* device, the map of every element (CatWorlds.map_index); NULL = map 0 */
+  const void* pos;           /* device: agent a of element e is the fp32 (x, y) at pos + e * pos_stride + 8 a (4-byte
+                                aligned) — the packed state buffer holds them in words 0 .. 2A-1 of each record */
+  int64_t pos_stride;        /* bytes, a multiple of 4, >= 8 A */
+  const void* ray_dist;      /* optional (NULL = no rays): f16 [A][R] at ray_dist + e * ray_dist_stride (2-byte aligned) */
+  int64_t ray_dist_stride;   /* bytes, even, >= 2 A R */
+  const void* ray_type;      /* u8 [A][R] ObjectType at ray_type + e * ray_type_stride; given with ray_dist */
+  int64_t ray_type_stride;   /* bytes, >= A R */
+  int32_t downsample;        /* >= 1 */
+  double agent_radius;       /* finite, >= 0 */
+  uint8_t* frames;           /* device u8 [K][W'][H'][3], cat_renderer_frame_size; indexed with 64-bit offsets */
+} CatRenderIO;
+
+/* windows: [n_maps][2] window (width, height) of each map, sides in 1..8192.  Every map needs the same numbers of cops
+ * and thieves; n_rays in 2..CAT_MAX_RAYS.  The arguments are checked before any CUDA call.  Builds each map's wall
+ * layer (a bit per pixel) on the device and synchronises: call it outside graph capture. */
+int cat_renderer_create(const CatMapDesc* maps, const int32_t* windows, int32_t n_maps, int32_t n_rays, int32_t device,
+                        CatRenderer** out);
+int cat_renderer_destroy(CatRenderer* renderer);
+/* host only: the frame size (W', H') at this downsample */
+int cat_renderer_frame_size(const CatRenderer* renderer, int32_t downsample, int32_t* w, int32_t* h);
+/* K frames, one launch on `stream`: no allocation, no synchronisation, CUDA-graph capturable */
+int cat_render(const CatRenderer* renderer, const CatRenderIO* io, void* stream);
+/* host only: the fp32 ray directions the step and the renderer use, out[2 i] = (float)cos(i 2 pi / R),
+ * out[2 i + 1] = (float)sin(i 2 pi / R) */
+int cat_ray_directions(int32_t n_rays, float* out);
 
 /* Environment variables the library reads (tuning / test knobs; none is needed for normal use, results never depend on them):
  *   CAT_GENERIC_KERNEL=1       cat_env_create: run the any-shape instantiation <0, 0> even for 3 agents x 90 rays (tests)
