@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-CAT_ABI_VERSION = 7
+CAT_ABI_VERSION = 8
 CAT_MAX_AGENTS = 8
 CAT_MAX_RAYS = 128
 CAT_MAX_MAPS = 8
@@ -62,6 +62,8 @@ class CatStepIO(C.Structure):
         ("obs_dist_world_stride", C.c_int32), ("obs_type_world_stride", C.c_int32),
         ("record", C.c_void_p), ("record_world_stride", C.c_int32),
         ("critic_f32", C.c_void_p), ("obs_bf16", C.c_void_p), ("critic_bf16", C.c_void_p), ("record_packed_types", C.c_int32),
+        ("final_record", C.c_void_p), ("final_record_world_stride", C.c_int32),
+        ("final_obs_f32", C.c_void_p), ("final_state_f32", C.c_void_p), ("final_critic_f32", C.c_void_p),
     ]
 
 

@@ -712,6 +712,15 @@ static int prepare(CatEnv* env, void* state_dev, const CatStepIO* io, int mode, 
         return fail(CAT_ERR_INVALID, "record output must be 16-byte aligned with a world stride that is a multiple of 16 and >= CatRecordLayout.bytes");
       k.obs_dist = nullptr; k.obs_type = nullptr; k.reward = nullptr; k.terminated = nullptr; k.truncated = nullptr; k.winner = nullptr;
     }
+    if (mode == MODE_STEP) {   // final outputs: step launches only (reset / observe share the caller's CatStepIO)
+      if (io->final_record) {
+        k.final_record = reinterpret_cast<unsigned char*>(io->final_record);
+        k.final_record_stride = io->final_record_world_stride ? io->final_record_world_stride : k.lay.r_bytes;
+        if ((reinterpret_cast<uintptr_t>(io->final_record) & 15) || (k.final_record_stride & 15) || k.final_record_stride < k.lay.r_bytes)
+          return fail(CAT_ERR_INVALID, "final_record must be 16-byte aligned with a world stride that is a multiple of 16 and >= CatRecordLayout.bytes");
+      }
+      k.final_obs_f32 = io->final_obs_f32; k.final_state_f32 = io->final_state_f32; k.final_critic_f32 = io->final_critic_f32;
+    }
   } else if (mode == MODE_STEP) {
     return fail(CAT_ERR_INVALID, "step needs a CatStepIO");
   }
@@ -719,10 +728,11 @@ static int prepare(CatEnv* env, void* state_dev, const CatStepIO* io, int mode, 
   return CAT_OK;
 }
 
-// the instantiation for this launch: the record-only one for a step whose record is all it writes
+// the instantiation for this launch: the record-only one for a step whose record is all it writes (no final outputs)
 static WorldKernel kernel_for(const CatEnv* env, const KParams& k) {
   const bool record_only = k.mode == MODE_STEP && k.record && !k.shared_dist && !k.shared_type && !k.team_pos && !k.obs_f32 && !k.state_f32 &&
-                           !k.hit_point && !k.critic_f32 && !k.obs_bf16 && !k.critic_bf16;
+                           !k.hit_point && !k.critic_f32 && !k.obs_bf16 && !k.critic_bf16 &&
+                           !k.final_record && !k.final_obs_f32 && !k.final_state_f32 && !k.final_critic_f32;
   return record_only ? env->kernel_record : env->kernel;
 }
 

@@ -189,6 +189,13 @@ struct KParams {
   // one entry that mirrors the fields above.
   int n_maps;
   MapSlice maps[CAT_MAX_MAPS];
+  // Final outputs (CatStepIO.final_*): what a world that ends in this step would have emitted with auto_reset = 0.  Set by
+  // step launches only and read by the TX = true instantiations only (kernel_for never picks the record-only one for them).
+  unsigned char* final_record;    // unpacked record, final_record_stride apart
+  int final_record_stride;
+  float* final_obs_f32;
+  float* final_state_f32;
+  float* final_critic_f32;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -965,25 +972,33 @@ __device__ __forceinline__ uint16_t f32_to_bf16_bits(float v) {   // round to ne
 // Optional learner-facing layouts (what skrl's wrapper would build on the host): per-agent flattened observation,
 // the flattened centralised-critic state, the critic's 4-channel ray block (lstm_value_net.py:122-137), and bf16
 // copies.  Only called when the caller asked for them; kept out of line so the native-dtype fast path stays small.
-__device__ __noinline__ void write_flat_layouts(const KParams& k, const uint16_t* rdist, const uint8_t* rtype,
+// `o`: the destination — the step's own arrays, or the final-output arrays of a world that ends (write_final_outputs).
+struct FlatOut {
+  float* obs_f32;
+  uint16_t* obs_bf16;
+  float* critic_f32;
+  uint16_t* critic_bf16;
+  float* state_f32;
+};
+__device__ __noinline__ void write_flat_layouts(const KParams& k, const FlatOut o, const uint16_t* rdist, const uint8_t* rtype,
                                                 const float* pos, long long world) {
   const int A = k.A, R = k.R, lane = threadIdx.x & 31;
-  if (k.obs_f32 || k.obs_bf16) {  // [A][N][2R]: [distance | object_type] as skrl flattens the Dict (keys sorted)
+  if (o.obs_f32 || o.obs_bf16) {  // [A][N][2R]: [distance | object_type] as skrl flattens the Dict (keys sorted)
 #pragma unroll 1
     for (int a = 0; a < A; ++a) {
-      const size_t o = ((size_t)a * k.n_worlds + world) * (2 * R);
+      const size_t off = ((size_t)a * k.n_worlds + world) * (2 * R);
 #pragma unroll 1
       for (int i = lane; i < 2 * R; i += 32) {
         const float v = i < R ? __half2float(__ushort_as_half(rdist[a * R + i])) : (float)rtype[a * R + i - R];
-        if (k.obs_f32) k.obs_f32[o + i] = v;
-        if (k.obs_bf16) k.obs_bf16[o + i] = f32_to_bf16_bits(v);
+        if (o.obs_f32) o.obs_f32[off + i] = v;
+        if (o.obs_bf16) o.obs_bf16[off + i] = f32_to_bf16_bits(v);
       }
     }
   }
-  if (k.critic_f32 || k.critic_bf16) {
+  if (o.critic_f32 || o.critic_bf16) {
     // LSTMValue's channel stack, cut from the FIRST agent's block of env.state() (SURVEY.md C-8):
     // [own_obj_types | own_distances | object_type_shared | distance_shared] of cop_0; shared = first non-EMPTY of the cops
-    const size_t o = (size_t)world * 4 * R;
+    const size_t off = (size_t)world * 4 * R;
 #pragma unroll 1
     for (int i = lane; i < 4 * R; i += 32) {
       const int ch = i / R, ri = i - ch * R;
@@ -998,13 +1013,13 @@ __device__ __noinline__ void write_flat_layouts(const KParams& k, const uint16_t
           if (t == TYPE_EMPTY) { t = rtype[b * R + ri]; d = rdist[b * R + ri]; }
         v = ch == 2 ? (float)t : __half2float(__ushort_as_half(d));
       }
-      if (k.critic_f32) k.critic_f32[o + i] = v;
-      if (k.critic_bf16) k.critic_bf16[o + i] = f32_to_bf16_bits(v);
+      if (o.critic_f32) o.critic_f32[off + i] = v;
+      if (o.critic_bf16) o.critic_bf16[off + i] = f32_to_bf16_bits(v);
     }
   }
-  if (k.state_f32) {
+  if (o.state_f32) {
     // env.state(): per agent [distance_shared | object_type_shared | own_distances | own_obj_types | team_positions]
-    float* dst = k.state_f32 + (size_t)world * k.state_dim;
+    float* dst = o.state_f32 + (size_t)world * k.state_dim;
     int base = 0;
 #pragma unroll 1
     for (int a = 0; a < A; ++a) {
@@ -1112,17 +1127,19 @@ __device__ __forceinline__ void write_optional_outputs(const KParams& k, const W
       }
     }
   }
-  if (k.obs_f32 || k.state_f32 || k.critic_f32 || k.obs_bf16 || k.critic_bf16) write_flat_layouts(k, w.rdist, w.rtype, pos, world);
+  if (k.obs_f32 || k.state_f32 || k.critic_f32 || k.obs_bf16 || k.critic_bf16)
+    write_flat_layouts(k, FlatOut{k.obs_f32, k.obs_bf16, k.critic_f32, k.critic_bf16, k.state_f32}, w.rdist, w.rtype, pos, world);
 }
 
-template <int TA, int TR>
+// The staged record of one world to the step's record output, or (FINAL) to the final record, which is never packed.
+template <int TA, int TR, bool FINAL>
 __device__ __forceinline__ void write_record(const KParams& k, const Warp& w, long long world) {
   const int A = TA ? TA : k.A, R = TR ? TR : k.R, lane = w.lane, nrays = A * R;
   {
     // one record per world, staged contiguously: [f16 distance | u8 type | f32 reward | flags], 16-byte stores
     unsigned char* stage = reinterpret_cast<unsigned char*>(w.rdist);
     int n16 = LAY(r_bytes) >> 4;
-    if (k.record_packed) {
+    if (!FINAL && k.record_packed) {
       // host-facing form (CatRecordLayout.type_bits == 2): 16 staged u8 types -> one 32-bit word, written back over the
       // start of the type area (each round reads its 512 source bytes before any lane writes: the 128 bytes a round
       // writes lie inside source bytes an earlier or the same round has read); rewards and flags move up behind them.
@@ -1159,11 +1176,12 @@ __device__ __forceinline__ void write_record(const KParams& k, const Warp& w, lo
       __syncwarp();
       n16 = LAY(rp_bytes) >> 4;
     }
-    uint4* dst = reinterpret_cast<uint4*>(k.record + (size_t)world * k.record_stride);
+    uint4* dst = reinterpret_cast<uint4*>(FINAL ? k.final_record + (size_t)world * k.final_record_stride
+                                                    : k.record + (size_t)world * k.record_stride);
     const uint4* src = reinterpret_cast<const uint4*>(stage);
 #pragma unroll 1
     for (int i = lane; i < n16; i += 32) dst[i] = src[i];
-    if (k.record_packed) {
+    if (!FINAL && k.record_packed) {
       // the staged record's own tail (rewards / flags / padding behind the u8 types) held packed-form bytes: restore
       // what the next world expects there — zero padding (its rewards, flags and types are rewritten every step)
       __syncwarp();
@@ -1179,7 +1197,17 @@ __device__ __forceinline__ void write_record(const KParams& k, const Warp& w, lo
 template <int TA, int TR, bool TX>
 __device__ __forceinline__ void write_observation(const KParams& k, const Warp& w, long long world, bool flags_too) {
   if (TX) write_optional_outputs<TA, TR>(k, w, world, flags_too);
-  if (TX ? k.record != nullptr : true) write_record<TA, TR>(k, w, world);
+  if (TX ? k.record != nullptr : true) write_record<TA, TR, false>(k, w, world);
+}
+
+// A world that ends in this step: its terminal observation, rewards and flags (staged, pre-physics) to the final outputs —
+// the record and flat layouts the step would write with auto_reset = 0.
+template <int TA, int TR>
+__device__ __forceinline__ void write_final_outputs(const KParams& k, const Warp& w, long long world) {
+  if (k.final_record) write_record<TA, TR, true>(k, w, world);
+  if (k.final_obs_f32 || k.final_state_f32 || k.final_critic_f32)
+    write_flat_layouts(k, FlatOut{k.final_obs_f32, nullptr, k.final_critic_f32, nullptr, k.final_state_f32}, w.rdist, w.rtype,
+                       w.rec, world);
 }
 
 // cop.py:49-75 / thief.py:48-69 in fp32 from the f16 distance (SURVEY.md C-3).
@@ -1767,9 +1795,15 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
       if (do_reset) { reset_world(k, m, w, world); do_reset = false; staged = false; }
       // entity.py:143 — observation of the pre-physics state (SURVEY.md C-1).  A world that ends on this step and
       // is re-spawned in it emits the NEW episode's observation (C-10) and a terminal reward that does not depend
-      // on what is seen, so its terminal sensor sweep would be thrown away: skip it.  With one world per warp the
-      // launch lasts as long as its slowest warp, and a second sweep made every finishing world that warp.
-      if (!(do_step && (captured || timeout) && k.auto_reset)) observe_world<TA, TR, TL, TX, TM>(k, m, w, world, staged, slot_stage);
+      // on what is seen, so its terminal sensor sweep would be thrown away unless the launch asks for final outputs:
+      // skip it then.  With one world per warp the launch lasts as long as its slowest warp, and a second sweep made
+      // every finishing world that warp.
+      const bool ends = do_step && (captured || timeout);
+      const bool final_out = TX && ends && (k.final_record || k.final_obs_f32 || k.final_state_f32 || k.final_critic_f32);
+      // (TX = false keeps the test spelled out: written through `ends`, ptxas schedules the record-only kernel, which
+      // never writes final outputs, differently — DESIGN.md §2.2)
+      if (TX ? !(ends && k.auto_reset) || final_out : !(do_step && (captured || timeout) && k.auto_reset))
+        observe_world<TA, TR, TL, TX, TM>(k, m, w, world, staged, slot_stage);
       bool again = false;
       if (do_step) {
         if (lane < A) w.rew[lane] = agent_reward(k, lane, w.minbits[lane], captured, timeout);
@@ -1785,6 +1819,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
         if (lane == 0) { w.flg[0] = 0; w.flg[1] = 0; w.flg[2] = 0xFF; }
       }
       __syncwarp();
+      if (final_out) write_final_outputs<TA, TR>(k, w, world);
       if (!again) write_observation<TA, TR, TX>(k, w, world, mode == MODE_STEP);
       __syncwarp();
       if (do_step) {

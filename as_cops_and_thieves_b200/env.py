@@ -257,6 +257,12 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
     ``agents`` never empties: finished worlds are re-spawned inside the step kernel and report the
     observation of the new episode (SURVEY.md C-10), with the terminal reward / flags of the old one.
 
+    ``final_observations=True``: the step kernel also keeps the last observation of every episode that ends, the
+    gymnasium ``final_observation``: ``infos[agent]["final_observation"]`` is an (N, 2R) view of that agent's final
+    observation, and ``final_state()`` / ``final_critic()`` the final ``state()`` / ``critic()``.  They are written
+    only for the worlds that end in the step and are valid where ``terminated``; a truncated (timed-out) episode can be
+    bootstrapped from them (``MAPPOConfig.time_limit_bootstrap``).
+
     Mixed maps: ``map`` may be a sequence of maps (at most 8, all with the same cops and thieves).  ``num_envs`` is
     then split over them as evenly as possible (the remainder to the first maps, ``split_worlds``) or given per map;
     ``spawn_override`` is None or one entry per map, ``cell`` applies to every map.  Map m owns a contiguous block of
@@ -268,7 +274,7 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
                  time_step: float = 1 / 60.0, device: Union[str, torch.device] = "cuda:0", seed: int = 0, gid0: int = 0,
                  physical_params: Optional[dict] = None, stale_shape_cache: bool = True,
                  spawn_override: Optional[Union[dict, Sequence[Optional[dict]]]] = None, cell: Optional[float] = None,
-                 render_mode=None):
+                 render_mode=None, final_observations: bool = False):
         params = _make_params(max_step_count, time_step, physical_params, auto_reset=1, seed=int(seed),
                               stale_shape_cache=int(stale_shape_cache))
         self._params = params
@@ -277,7 +283,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._cmap = compile_map(map, spawn_override=spawn_override, cell=cell)
             self._cmaps = [self._cmap]
             self._setup_common(map, self._cmap, params)
-            self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True)
+            self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True,
+                                want_final=final_observations)
         else:
             self.maps = list(map)
             n = len(self.maps)
@@ -294,7 +301,7 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             window = (max(m.window_dimensions[0] for m in self.maps), max(m.window_dimensions[1] for m in self.maps))
             self._setup_common(self.maps[0], self._cmap, params, window=window)
             self._w = CatWorlds(self._cmaps, counts, device=device, gid0=gid0, params=params, want_f32=True,
-                                want_critic=True)
+                                want_critic=True, want_final=final_observations)
             num_envs = sum(counts)
         self.map_names = [c.name for c in self._cmaps]
         self.map_index = self._w.map_index
@@ -329,8 +336,11 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             rew = {a: w.reward[:, i:i + 1] for i, a in enumerate(self.possible_agents)}
             term = w.terminated.view(torch.bool).unsqueeze(1)
             trunc = w.truncated.view(torch.bool).unsqueeze(1)
-            v = (obs, rew, {a: term for a in self.possible_agents}, {a: trunc for a in self.possible_agents},
-                 {a: {"winner": w.winner} for a in self.possible_agents})
+            infos = {a: {"winner": w.winner} for a in self.possible_agents}
+            if w.final_obs_f32 is not None:
+                for i, a in enumerate(self.possible_agents):
+                    infos[a]["final_observation"] = w.final_obs_f32[i]
+            v = (obs, rew, {a: term for a in self.possible_agents}, {a: trunc for a in self.possible_agents}, infos)
             self._cached_views = v
         return v
 
@@ -358,6 +368,16 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         """The critic's front end, written by the step kernel itself: the 4 ray channels ``LSTMValue`` cuts out of
         ``state()`` (``lstm_value_net.py:122-137``) as ``(N, 4, R)`` float32 — no slice / stack copies on the way."""
         return self._w.critic_f32
+
+    def final_state(self) -> Optional[torch.Tensor]:
+        """``state()`` of the last step of every episode that ended, (N, S) float32, valid where ``terminated``
+        (None without ``final_observations``)."""
+        return self._w.final_state_f32
+
+    def final_critic(self) -> Optional[torch.Tensor]:
+        """``critic()`` of the last step of every episode that ended, (N, 4, R) float32, valid where ``terminated``
+        (None without ``final_observations``)."""
+        return self._w.final_critic_f32
 
     def render(self, world: int = 0):
         """``rgb_array`` of one world, drawn on that world's own map (numpy (W, H, 3) uint8 of that map's window):

@@ -218,6 +218,9 @@ class MAPPOConfig:
     model: str = "lstm"                # "lstm" (self_play_driver.py via initialize_lstm_models_for_mappo) | "mlp"
     sequence_length: int = 16          # lstm_policy_net.py:16
     cuda_graph: bool = True            # replay the whole rollout (nets + env kernels) as one CUDA graph
+    # skrl's time_limit_bootstrap: a truncated (timed-out) transition stores rew + discount_factor * V(s_final), V from
+    # each agent's critic on the episode's final observation (needs BatchedCopsThievesEnv(final_observations=True))
+    time_limit_bootstrap: bool = False
     update_autocast: str = "none"      # "bf16": run the PPO update's forward / backward under torch.autocast (the
                                        # reference trains in fp32, so this is off by default; ~2x faster updates)
     distributed: bool = False          # all-reduce gradients (and advantage statistics) across ranks
@@ -315,6 +318,12 @@ class MAPPOLearner:
         # step kernel (env.critic()) instead of storing / slicing / stacking the 1090-float state
         self.critic_block = self.cfg.model == "lstm" and getattr(env, "critic", None) is not None and env.critic() is not None
         self.n_value_in = 4 * env.worlds.R if self.critic_block else self.n_state
+        if self.cfg.time_limit_bootstrap:
+            final = getattr(env, "final_critic" if self.critic_block else "final_state", None)
+            if final is None or final() is None:
+                raise ValueError("time_limit_bootstrap needs an environment that keeps final observations "
+                                 "(BatchedCopsThievesEnv(..., final_observations=True))")
+        self._no_reset = torch.zeros((N, 1), dtype=torch.bool, device=dev)
         self.mem_state = torch.zeros((T, N, self.n_value_in), device=dev)
         self.mem_done = torch.zeros((T, N), dtype=torch.bool, device=dev)
         self.mem_reset = torch.zeros((T, N), dtype=torch.bool, device=dev)   # episode of world n ended just before step t
@@ -421,7 +430,9 @@ class MAPPOLearner:
     def _rollout_body(self, uniform_random: bool) -> None:
         """``rollouts`` lockstep transitions on static buffers only (no host syncs, no allocations that outlive
         the call): SequentialTrainer.train's inner loop — act -> env.step -> env.state -> record_transition.
-        Done worlds are re-spawned inside the step kernel (SURVEY.md C-10)."""
+        Done worlds are re-spawned inside the step kernel (SURVEY.md C-10).  With ``time_limit_bootstrap`` each critic
+        also evaluates the final value input of the step from the hidden state it carries, without advancing that state,
+        and a truncated world's stored reward becomes ``rew + discount_factor * V_final``."""
         env, cfg = self.env, self.cfg
         L = cfg.sequence_length
         obs_bufs = env._obs_dict()                 # views of the environment's persistent output buffers
@@ -452,8 +463,16 @@ class MAPPOLearner:
                     self._hc[a]["value"][0].copy_(hc[0]); self._hc[a]["value"][1].copy_(hc[1])
                 m["val"][t].copy_(v.view(-1))
             _, rew, term, trunc, _ = env.step(self._act)
+            if cfg.time_limit_bootstrap:
+                final = self._final_value_input().unsqueeze(1)
+                truncated = trunc[self.agents[0]].view(-1).float()
             for a in self.agents:
-                self.mem[a]["rew"][t].copy_(rew[a].view(-1))
+                if cfg.time_limit_bootstrap:
+                    v_final, _ = self.models[a]["value"](final, self._hc[a]["value"], self._no_reset)
+                    torch.addcmul(rew[a].view(-1), v_final.view(-1), truncated, value=cfg.discount_factor,
+                                  out=self.mem[a]["rew"][t])
+                else:
+                    self.mem[a]["rew"][t].copy_(rew[a].view(-1))
             done = (term[self.agents[0]] | trunc[self.agents[0]]).view(-1)
             self.mem_done[t].copy_(done)
             self._prev_done.copy_(done)
@@ -461,6 +480,10 @@ class MAPPOLearner:
     def _value_input(self) -> torch.Tensor:
         """What the critics read: the kernel's (N, 4, R) block viewed as (N, 4 R), or the flattened state (N, S)."""
         return self.env.critic().view(self.env.num_envs, -1) if self.critic_block else self.env.state()
+
+    def _final_value_input(self) -> torch.Tensor:
+        """``_value_input`` of the last step of the episodes that ended in the step just taken (valid where done)."""
+        return self.env.final_critic().view(self.env.num_envs, -1) if self.critic_block else self.env.final_state()
 
     def collect(self) -> None:
         """One rollout.  The first call per mode runs eagerly (warm-up: cuDNN plans, allocator); later calls

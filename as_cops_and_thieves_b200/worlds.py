@@ -73,12 +73,21 @@ class CatWorlds:
                  device: Union[str, torch.device] = "cuda:0",
                  gid0: int = 0, params: Optional[EnvParams] = None, want_f32: bool = True,
                  want_shared: bool = True, want_hits: bool = False, pinned_outputs: bool = False,
-                 want_critic: bool = False, want_bf16: bool = False, **overrides):
+                 want_critic: bool = False, want_bf16: bool = False, want_final: bool = False, **overrides):
         """``pinned_outputs=True`` places every output tensor in mapped pinned HOST memory: the kernel stores its
         results there directly and the host reads them (``tensor.numpy()``) after one stream synchronisation —
         the layout for callers that consume every step on the CPU, like the single-world PettingZoo face.
         ``want_critic``: also emit the critic's 4-channel ray block ``critic_f32 (N, 4, R)``
         (``lstm_value_net.py:122-137``); ``want_bf16``: bf16 copies of ``obs_f32`` / ``critic_f32``.
+
+        ``want_final``: every step also writes, for each world that ENDS in it (``terminated``), what the step would
+        have emitted with ``auto_reset = 0`` — the observation of the positions it ended in with the terminal rewards
+        and flags — into a second set of outputs: the record views ``final_obs_dist``, ``final_obs_type``,
+        ``final_reward``, ``final_terminated``, ``final_truncated``, ``final_winner``, and ``final_obs_f32`` /
+        ``final_state_f32`` / ``final_critic_f32`` where ``want_f32`` / ``want_critic`` ask for the plain ones.  With
+        auto-reset the plain outputs of such a world already hold the new episode, so this is the only copy of its last
+        observation (gymnasium's ``final_observation``).  Entries of worlds that do not end are left untouched: read them
+        where ``terminated``.
 
         Mixed maps: ``cmap`` may be a sequence of compiled maps (at most ``CAT_MAX_MAPS``, all with the same cops and
         thieves) with ``n_worlds`` the matching sequence of world counts.  Map m then owns the worlds
@@ -166,6 +175,17 @@ class CatWorlds:
         self.critic_f32 = alloc((N, 4, R), torch.float32) if want_critic else None
         self.obs_bf16 = alloc((A, N, 2 * R), torch.bfloat16) if want_bf16 and want_f32 else None
         self.critic_bf16 = alloc((N, 4, R), torch.bfloat16) if want_bf16 and want_critic else None
+        self.want_final = bool(want_final)
+        self._final_out = alloc(N * self.record_bytes, torch.uint8) if want_final else None
+        fviews = self._record_views(self._final_out) if want_final else dict.fromkeys(views)
+        self.final_obs_dist, self.final_obs_type, self.final_reward = fviews["obs_dist"], fviews["obs_type"], fviews["reward"]
+        self.final_terminated, self.final_truncated = fviews["terminated"], fviews["truncated"]
+        self.final_winner = fviews["winner"]
+        if want_final:
+            self.final_winner.fill_(-1)
+        self.final_obs_f32 = alloc((A, N, 2 * R), torch.float32) if want_final and want_f32 else None
+        self.final_state_f32 = alloc((N, self.S), torch.float32) if want_final and want_f32 else None
+        self.final_critic_f32 = alloc((N, 4, R), torch.float32) if want_final and want_critic else None
         self._host = None
         self._io = self._make_io()
         self._ptr_table = (C.c_void_p * 8)()
@@ -209,7 +229,9 @@ class CatWorlds:
         return CatStepIO(None, 0, None, None, None, None, None, None, None, dp(self.shared_dist), dp(self.shared_type),
                          dp(self.team_pos), dp(self.obs_f32), dp(self.state_f32), dp(self.hit_point), 0, 0,
                          rec.data_ptr(), self.packed_record_bytes if packed else self.record_bytes,
-                         dp(self.critic_f32), dp(self.obs_bf16), dp(self.critic_bf16), 1 if packed else 0)
+                         dp(self.critic_f32), dp(self.obs_bf16), dp(self.critic_bf16), 1 if packed else 0,
+                         dp(self._final_out), self.record_bytes, dp(self.final_obs_f32), dp(self.final_state_f32),
+                         dp(self.final_critic_f32))
 
     def map_info(self, m: int) -> CatEnvInfo:
         """``cat_env_map_info``: the figures of map ``m`` alone (its worlds, hulls, edges, blob and ray-list bytes)."""

@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define CAT_ABI_VERSION 7
+#define CAT_ABI_VERSION 8
 #define CAT_MAX_AGENTS 8
 #define CAT_MAX_RAYS 128
 #define CAT_MAX_MAPS 8 /* maps of one environment (cat_env_create_multi) */
@@ -144,6 +144,20 @@ typedef struct {
   /* != 0: `record` takes the PACKED form of the record (cat_env_packed_record_layout; types at 2 bits each, 640 B
    * instead of 832 B per world for 3 agents x 90 rays) — the form meant to cross PCIe on the host-facing path. */
   int32_t record_packed_types;
+  /* FINAL OUTPUTS (step launches only; cat_env_reset / cat_env_observe ignore them).  For every world that ENDS in the
+   * step (terminated: captured or timed out) they receive what that step would have emitted with auto_reset = 0: the
+   * observation of the pre-physics positions with the terminal rewards, terminated, truncated and winner — bit for bit
+   * the record / obs_f32 / state_f32 / critic_f32 of an auto_reset = 0 twin.  With auto_reset = 1 the normal outputs
+   * of such a world hold the re-spawned episode's observation, so this is the only place its last observation appears
+   * (gymnasium's final_observation: truncated episodes can be bootstrapped from V(s_final)).  The entries of worlds
+   * that do not end are left untouched.  Any may be NULL; a step with none set costs nothing extra.
+   *   final_record: the unpacked record (cat_env_record_layout), the alignment and stride rules of `record`
+   *   final_obs_f32 / final_state_f32 / final_critic_f32: the layouts of obs_f32 / state_f32 / critic_f32 */
+  void* final_record;
+  int32_t final_record_world_stride;
+  float* final_obs_f32;
+  float* final_state_f32;
+  float* final_critic_f32;
 } CatStepIO;
 
 /* byte offsets inside one world's output record (cat_env_record_layout / cat_env_packed_record_layout) */

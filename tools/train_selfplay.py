@@ -44,6 +44,8 @@ def main():
     ap.add_argument("--schedule", default="scaled", choices=["scaled", "reference", "off"],
                     help="random_timesteps / learning_starts / freeze durations: the reference's values divided by the "
                          "number of worlds (same number of transitions), the reference's values as they are, or none")
+    ap.add_argument("--time-limit-bootstrap", action="store_true",
+                    help="bootstrap timed-out episodes from the critic's value of their final observation")
     a = ap.parse_args()
 
     rank, local_rank, world_size = dist_env()
@@ -60,16 +62,16 @@ def main():
     spawn = [free_space_regions(m) if a.free_spawn else None for m in maps]
     if len(maps) == 1:
         env = BatchedCopsThievesEnv(maps[0], n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
-                                    spawn_override=spawn[0])
+                                    spawn_override=spawn[0], final_observations=a.time_limit_bootstrap)
     else:
         env = BatchedCopsThievesEnv(maps, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
-                                    spawn_override=spawn)
+                                    spawn_override=spawn, final_observations=a.time_limit_bootstrap)
     # the reference's schedule (10 000 random / 15 000 before learning / 15 000 frozen policy) counts steps of ONE
     # environment; with thousands of lockstep worlds the same number of TRANSITIONS is reached in a few steps, so the
     # driver scales the durations by the world count unless told otherwise
     scale = max(1, a.worlds * world_size) if a.schedule == "scaled" else 1
     cfg = MAPPOConfig(rollouts=a.rollouts, model=a.model, distributed=world_size > 1, world_size=world_size,
-                      update_autocast=a.autocast, random_timesteps=-(-10000 // scale) if a.schedule != "off" else 0,
+                      update_autocast=a.autocast, time_limit_bootstrap=a.time_limit_bootstrap, random_timesteps=-(-10000 // scale) if a.schedule != "off" else 0,
                       learning_starts=-(-15000 // scale) if a.schedule != "off" else 0,
                       policy_freeze_duration=-(-15000 // scale) if a.schedule != "off" else 0,
                       opponent_freeze_duration=-(-15000 // scale) if a.schedule != "off" else 0)
