@@ -97,7 +97,7 @@ class CatRenderIO(C.Structure):
 #: every symbol ``include/cat_b200.h`` declares
 EXPORTS = (
     "cat_abi_version", "cat_last_error", "cat_env_create", "cat_env_create_multi", "cat_env_destroy", "cat_env_info",
-    "cat_env_map_info",
+    "cat_env_map_info", "cat_env_create_swappable", "cat_env_set_map", "cat_map_blob_bytes", "cat_ray_lists_device",
     "cat_env_record_layout", "cat_env_packed_record_layout", "cat_env_overflow_counts", "cat_ray_lists_host",
     "cat_env_set_seed", "cat_env_state_bytes", "cat_env_init_state", "cat_env_reset", "cat_env_step", "cat_env_step_host", "cat_env_observe",
     "cat_env_get_state", "cat_env_set_state", "cat_gae", "cat_adv_normalize",
@@ -131,6 +131,10 @@ def load():
                                  C.POINTER(C.c_void_p)]
     L.cat_env_create_multi.argtypes = [C.POINTER(CatMapDesc), C.c_int32, C.POINTER(C.c_int32), C.POINTER(CatParams), C.c_int64,
                                        C.c_int32, C.POINTER(C.c_void_p)]
+    L.cat_env_create_swappable.argtypes = [C.POINTER(CatMapDesc), C.c_int32, C.POINTER(C.c_int32), C.POINTER(CatParams), C.c_int32,
+                                           C.c_int64, C.c_int32, C.POINTER(C.c_void_p)]
+    L.cat_env_set_map.argtypes = [C.c_void_p, C.c_int32, C.POINTER(CatMapDesc), C.c_void_p]
+    L.cat_map_blob_bytes.argtypes = [C.POINTER(CatMapDesc), C.POINTER(CatParams), C.POINTER(C.c_int32)]
     L.cat_env_destroy.argtypes = [C.c_void_p]
     L.cat_env_info.argtypes = [C.c_void_p, C.POINTER(CatEnvInfo)]
     L.cat_env_map_info.argtypes = [C.c_void_p, C.c_int32, C.POINTER(CatEnvInfo)]
@@ -143,6 +147,7 @@ def load():
     L.cat_env_step_host.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
     L.cat_ray_lists_host.argtypes = [C.POINTER(CatMapDesc), C.c_int32, C.c_double, C.c_double, C.c_double, C.POINTER(C.c_double * 5),
                                      C.c_void_p, C.POINTER(C.c_int64), C.c_void_p, C.POINTER(C.c_int64)]
+    L.cat_ray_lists_device.argtypes = L.cat_ray_lists_host.argtypes + [C.c_int32]
     L.cat_env_record_layout.argtypes = [C.c_void_p, C.POINTER(CatRecordLayout)]
     L.cat_env_packed_record_layout.argtypes = [C.c_void_p, C.POINTER(CatRecordLayout)]
     L.cat_env_overflow_counts.argtypes = [C.c_void_p, C.POINTER(C.c_uint64 * 2), C.c_int32]

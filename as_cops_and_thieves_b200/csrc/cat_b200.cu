@@ -54,6 +54,7 @@ int fail(int code, const std::string& msg) {
   } while (0)
 
 #include "ray_lists.h"
+#include "ray_lists_kernel.cuh"
 #include "world_kernel.cuh"
 #include "state_view.cuh"
 #include "gae_kernels.cuh"
@@ -132,7 +133,11 @@ struct CatEnv {
   int smem_bytes = 0;
   int grid = 0;
   int threads = kThreads;
-  int blob_bytes = 0, max_optin = 0, n_sm = 0;   // blob_bytes: the largest of the maps' blobs
+  int blob_bytes = 0, max_optin = 0, n_sm = 0;   // blob_bytes: the largest of the maps' blobs (swappable: the capacity)
+  // cat_env_create_swappable: every map's blob is allocated at blob_bytes and the mixed-map kernels run, so that
+  // cat_env_set_map changes neither the launch shape nor the KParams of a captured launch
+  bool swappable = false;
+  CatParams params{};
   // chunked host path: a second stream for the device-to-host copies and one event per chunk
   cudaStream_t copy_stream = nullptr;
   std::vector<cudaEvent_t> chunk_events;
@@ -240,6 +245,86 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, siz
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
+
+// One run of the device list builder (ray_lists_kernel.cuh) on the current device: size() uploads the map and runs the
+// counting passes, fill() writes the lists into the caller's arrays of slot_words / ovf_words words.  Synchronous; the
+// temporary arrays are freed with the object.
+struct RayListDeviceBuild {
+  RayListSetup su;
+  RayListDev p{};
+  size_t slot_words = 0, ovf_words = 0;
+  std::vector<void*> allocs;
+  int grid = 1;
+  ~RayListDeviceBuild() { for (void* a : allocs) cudaFree(a); }
+
+  template <typename T> cudaError_t alloc(T** ptr, size_t n) {
+    void* v = nullptr;
+    const cudaError_t e = cudaMalloc(&v, std::max<size_t>(n, 1) * sizeof(T));
+    if (e == cudaSuccess) { allocs.push_back(v); *ptr = static_cast<T*>(v); }
+    return e;
+  }
+  template <typename T> cudaError_t upload(const T** ptr, const T* src, size_t n) {
+    T* d = nullptr;
+    cudaError_t e = alloc(&d, n);
+    if (e == cudaSuccess && n) e = cudaMemcpy(d, src, n * sizeof(T), cudaMemcpyHostToDevice);
+    *ptr = d;
+    return e;
+  }
+  unsigned long long total(const unsigned long long* scanned, int n, cudaError_t* e) {
+    unsigned long long v = 0;
+    if (*e == cudaSuccess) *e = cudaMemcpy(&v, scanned + n, sizeof(v), cudaMemcpyDeviceToHost);
+    return v;
+  }
+
+  int size(const CatMapDesc* map, int R, double L, double rsum, double cell) {
+    ray_list_setup(map, R, L, rsum, cell, &su);
+    const int H = map->n_hulls, E = map->n_edges, cells = su.g.nx * su.g.ny;
+    if ((long long)su.g.nx * su.g.ny * R * 4 > 0x7FFFFFFFll) return fail(CAT_ERR_LIMIT, "ray-list grid too large");
+    p.H = H; p.E = E; p.R = R; p.nx = su.g.nx; p.ny = su.g.ny;
+    p.gx0 = su.gx0; p.gy0 = su.gy0; p.cell = su.cell; p.L = su.L; p.rs = su.rs;
+    std::vector<double> a(2 * (size_t)E), nn(2 * (size_t)E), u(2 * (size_t)R);
+    std::vector<int32_t> ehull(E);
+    for (int e = 0; e < E; ++e) { a[2 * e] = su.ax[e]; a[2 * e + 1] = su.ay[e]; nn[2 * e] = su.nnx[e]; nn[2 * e + 1] = su.nny[e]; }
+    for (int h = 0; h < H; ++h) for (int e = map->hull_off[h]; e < map->hull_off[h + 1]; ++e) ehull[e] = h;
+    for (int i = 0; i < R; ++i) { u[2 * i] = su.ux[i]; u[2 * i + 1] = su.uy[i]; }
+    grid = std::min(cells, 4096);
+    cudaError_t e = upload(&p.vert, map->vert, 2 * (size_t)E);
+    if (e == cudaSuccess) e = upload(&p.normal, map->normal, 2 * (size_t)E);
+    if (e == cudaSuccess) e = upload(&p.a, a.data(), a.size());
+    if (e == cudaSuccess) e = upload(&p.nn, nn.data(), nn.size());
+    if (e == cudaSuccess) e = upload(&p.hull_bb, map->hull_bb, 4 * (size_t)H);
+    if (e == cudaSuccess) e = upload(&p.ehull, ehull.data(), ehull.size());
+    if (e == cudaSuccess) e = upload(&p.u, u.data(), u.size());
+    if (e == cudaSuccess) e = alloc(&p.cand_off, cells + 1);
+    if (e == cudaSuccess) { cat_ray_list_cand_kernel<false><<<grid, kRlThreads>>>(p); e = cudaGetLastError(); }
+    if (e == cudaSuccess) { cat_ray_list_scan_kernel<<<1, 1024>>>(p.cand_off, cells); e = cudaGetLastError(); }
+    const unsigned long long n_cand = total(p.cand_off, cells, &e);
+    if (e == cudaSuccess) e = alloc(&p.cand_e, n_cand);
+    if (e == cudaSuccess) e = alloc(&p.cand_lb, n_cand);
+    if (e == cudaSuccess) { cat_ray_list_cand_kernel<true><<<grid, kRlThreads>>>(p); e = cudaGetLastError(); }
+    if (e == cudaSuccess) e = alloc(&p.n_list, (size_t)cells * R);
+    if (e == cudaSuccess) e = alloc(&p.words, cells + 1);
+    if (e == cudaSuccess) e = alloc(&p.longs, cells + 1);
+    if (e == cudaSuccess) { cat_ray_list_kernel<false><<<grid, kRlThreads>>>(p); e = cudaGetLastError(); }
+    if (e == cudaSuccess) { cat_ray_list_scan_kernel<<<1, 1024>>>(p.words, cells); e = cudaGetLastError(); }
+    if (e == cudaSuccess) { cat_ray_list_scan_kernel<<<1, 1024>>>(p.longs, cells); e = cudaGetLastError(); }
+    const unsigned long long n_words = total(p.words, cells, &e), n_long = total(p.longs, cells, &e);
+    if (e == cudaSuccess) e = alloc(&p.long_buf, n_long);
+    if (e != cudaSuccess) return fail(CAT_ERR_CUDA, std::string("ray lists (device build): ") + cudaGetErrorString(e));
+    if (4 + n_words > 0x7FFFFFFFull) return fail(CAT_ERR_LIMIT, "ray-list overflow array too large for 31-bit links");
+    slot_words = (size_t)cells * R * 4;
+    ovf_words = 4 + (size_t)n_words;
+    return CAT_OK;
+  }
+
+  int fill(uint32_t* slots_dev, uint32_t* ovf_dev) {
+    p.slots = slots_dev; p.ovf = ovf_dev;
+    cat_ray_list_kernel<true><<<grid, kRlThreads>>>(p);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    return e == cudaSuccess ? CAT_OK : fail(CAT_ERR_CUDA, std::string("ray lists (device build): ") + cudaGetErrorString(e));
+  }
+};
 
 extern "C" {
 
@@ -377,7 +462,7 @@ static std::vector<unsigned char> build_blob(const CatMapDesc* map, const CatPar
   return blob;
 }
 
-// The per-(cell, ray) candidate lists of one map on one device: found in the cache or built, uploaded and cached.
+// The per-(cell, ray) candidate lists of one map on one device: found in the cache or built (on the device), and cached.
 static int acquire_ray_lists(const CatMapDesc* map, const CatParams* pr, int device, SharedRayLists** out) {
   const int R = pr->n_rays, H = map->n_hulls, E = map->n_edges;
   const double rsum = pr->wall_radius + pr->ray_radius;
@@ -399,21 +484,22 @@ static int acquire_ray_lists(const CatMapDesc* map, const CatParams* pr, int dev
   for (SharedRayLists* c : g_ray_lists)
     if (c->key == key) { sh = c; break; }
   if (!sh) {
-    RayLists rl;
-    build_ray_lists(map, R, pr->ray_length, rsum, pr->ray_list_cell, &rl);
+    RayListDeviceBuild b;
+    int rc = b.size(map, R, pr->ray_length, rsum, pr->ray_list_cell);
+    if (rc != CAT_OK) return rc;
     sh = new SharedRayLists();
-    sh->key.swap(key);
-    sh->g = rl.g; sh->slot_words = rl.slots.size(); sh->ovf_words = rl.ovf.size();
-    cudaError_t e1 = cudaMalloc(&sh->slots_dev, rl.slots.size() * 4);
-    cudaError_t e2 = e1 == cudaSuccess ? cudaMalloc(&sh->ovf_dev, rl.ovf.size() * 4) : e1;
-    if (e2 == cudaSuccess) e2 = cudaMemcpy(sh->slots_dev, rl.slots.data(), rl.slots.size() * 4, cudaMemcpyHostToDevice);
-    if (e2 == cudaSuccess) e2 = cudaMemcpy(sh->ovf_dev, rl.ovf.data(), rl.ovf.size() * 4, cudaMemcpyHostToDevice);
-    if (e2 != cudaSuccess) {
+    sh->g = b.su.g; sh->slot_words = b.slot_words; sh->ovf_words = b.ovf_words;
+    const cudaError_t e1 = cudaMalloc(&sh->slots_dev, b.slot_words * 4);
+    const cudaError_t e2 = e1 == cudaSuccess ? cudaMalloc(&sh->ovf_dev, b.ovf_words * 4) : e1;
+    rc = e2 == cudaSuccess ? b.fill(reinterpret_cast<uint32_t*>(sh->slots_dev), sh->ovf_dev)
+                           : fail(CAT_ERR_CUDA, std::string("ray lists: ") + cudaGetErrorString(e2));
+    if (rc != CAT_OK) {
       if (sh->slots_dev) cudaFree(sh->slots_dev);
       if (sh->ovf_dev) cudaFree(sh->ovf_dev);
       delete sh;
-      return fail(CAT_ERR_CUDA, std::string("ray lists: ") + cudaGetErrorString(e2));
+      return rc;
     }
+    sh->key.swap(key);
     g_ray_lists.push_back(sh);
   }
   ++sh->refs;
@@ -421,15 +507,17 @@ static int acquire_ray_lists(const CatMapDesc* map, const CatParams* pr, int dev
   return CAT_OK;
 }
 
-// Upload one map into `em`: its view lists, its share of the (cell, ray) lists and its blob, whose header (kept in
-// em.header) then points at the lists.  On failure whatever was allocated is left in `em` for cat_env_destroy.
-static int upload_map(const CatMapDesc* md, const CatParams* pr, int device, EnvMap& em) {
 #define UPLOAD_TRY(expr, what)                                                                              \
   do {                                                                                                      \
     cudaError_t _e = (expr);                                                                                \
     if (_e != cudaSuccess) return fail(CAT_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(_e));    \
   } while (0)
-  std::vector<unsigned char> blob = build_blob(md, pr);
+
+// Everything of one map but its blob allocation: its view lists and its share of the (cell, ray) lists go into `em`, and
+// `blob` receives the blob whose header (also kept in em.header) points at them.  On failure whatever was allocated is
+// left in `em` for release_map_tables.
+static int prepare_map(const CatMapDesc* md, const CatParams* pr, int device, EnvMap& em, std::vector<unsigned char>& blob) {
+  blob = build_blob(md, pr);
   BlobHeader& hd = em.header;
   memcpy(&hd, blob.data(), sizeof(hd));
   const int E = md->n_edges, ncell = md->nx * md->ny;
@@ -457,12 +545,31 @@ static int upload_map(const CatMapDesc* md, const CatParams* pr, int device, Env
     hd.rg_x0 = sh->g.x0; hd.rg_y0 = sh->g.y0; hd.rg_inv_cell = sh->g.inv_cell; hd.rg_nx = sh->g.nx; hd.rg_ny = sh->g.ny;
   }
   memcpy(blob.data(), &hd, sizeof(hd));
-  em.blob_bytes = (int)blob.size();
-  UPLOAD_TRY(cudaMalloc(&em.blob_dev, em.blob_bytes), "cudaMalloc(map blob)");
-  UPLOAD_TRY(cudaMemcpy(em.blob_dev, blob.data(), em.blob_bytes, cudaMemcpyHostToDevice), "cudaMemcpy(map blob)");
-#undef UPLOAD_TRY
   return CAT_OK;
 }
+
+// The view lists and the (cell, ray) lists of `em` (not its blob).
+static void release_map_tables(EnvMap& em) {
+  if (em.view_off_dev) cudaFree(em.view_off_dev);
+  if (em.view_edges_dev) cudaFree(em.view_edges_dev);
+  ray_lists_release(em.ray_lists);
+  em.view_off_dev = nullptr; em.view_edges_dev = nullptr; em.ray_lists = nullptr;
+}
+
+// Upload one map into `em`: prepare_map, then its blob in an allocation of `capacity` bytes (0: the blob's size) with a
+// zeroed tail.  On failure whatever was allocated is left in `em` for cat_env_destroy.
+static int upload_map(const CatMapDesc* md, const CatParams* pr, int device, int capacity, EnvMap& em) {
+  std::vector<unsigned char> blob;
+  const int rc = prepare_map(md, pr, device, em, blob);
+  if (rc != CAT_OK) return rc;
+  em.blob_bytes = capacity > 0 ? capacity : (int)blob.size();
+  UPLOAD_TRY(cudaMalloc(&em.blob_dev, em.blob_bytes), "cudaMalloc(map blob)");
+  UPLOAD_TRY(cudaMemcpy(em.blob_dev, blob.data(), blob.size(), cudaMemcpyHostToDevice), "cudaMemcpy(map blob)");
+  if (em.blob_bytes > (int)blob.size())
+    UPLOAD_TRY(cudaMemset(em.blob_dev + blob.size(), 0, em.blob_bytes - blob.size()), "cudaMemset(map blob)");
+  return CAT_OK;
+}
+#undef UPLOAD_TRY
 
 // Map m's own figures in `inf`: its worlds, hulls, edges, blob, CTAs of a full launch and (cell, ray) lists.
 static void map_info(const CatEnv* env, int m, CatEnvInfo& inf) {
@@ -475,6 +582,34 @@ static void map_info(const CatEnv* env, int m, CatEnvInfo& inf) {
   inf.ray_list_bytes = sh ? (int64_t)(sh->slot_words + sh->ovf_words) * 4 : 0;
 }
 
+// The environment's figures: map 0's, then the totals over the maps (worlds, list bytes, the largest blob, the grid).
+static void env_info(CatEnv* env) {
+  const KParams& k = env->kp;
+  CatEnvInfo& inf = env->info;
+  map_info(env, 0, inf);
+  for (int m = 1; m < (int)env->maps.size(); ++m) { CatEnvInfo other{}; map_info(env, m, other); inf.ray_list_bytes += other.ray_list_bytes; }
+  inf.n_worlds = env->n_worlds; inf.n_agents = k.A; inf.n_cops = k.nc; inf.n_thieves = k.A - k.nc;
+  inf.n_rays = k.R; inf.state_dim = k.state_dim; inf.record_words = k.lay.rec_words;
+  inf.map_blob_bytes = env->blob_bytes; inf.smem_bytes_per_cta = env->smem_bytes; inf.warps_per_cta = env->threads / 32;
+  inf.grid = env->grid; inf.n_pairs = k.lay.P;
+}
+
+static int create_env(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map, const CatParams* pr,
+                      int64_t gid0, int32_t device, int blob_capacity, CatEnv** out);
+
+// Map 0's values in the launch parameters: what a single-map launch reads (a mixed-map launch reads each map's from its
+// blob header).  Refreshed when map 0 is replaced, so they never point at released lists.
+static void set_map0_params(CatEnv* env) {
+  KParams& k = env->kp;
+  const EnvMap& em = env->maps[0];
+  const BlobHeader& h = em.header;
+  k.blob = em.blob_dev; k.blob_bytes = em.blob_bytes;
+  k.view_off = h.view_off; k.view_edges = h.view_edges;
+  k.ray_slots = h.ray_slots; k.ray_ovf = h.ray_ovf; k.ray_slot_count = h.ray_slot_count; k.ray_ovf_words = h.ray_ovf_words;
+  k.rg_x0 = h.rg_x0; k.rg_y0 = h.rg_y0; k.rg_inv_cell = h.rg_inv_cell; k.rg_nx = h.rg_nx; k.rg_ny = h.rg_ny;
+  k.n_edges = h.n_edges;
+}
+
 int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds, int64_t gid0, int32_t device,
                    CatEnv** out) {
   if (!map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
@@ -483,6 +618,35 @@ int cat_env_create(const CatMapDesc* map, const CatParams* pr, int32_t n_worlds,
 
 int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map, const CatParams* pr,
                          int64_t gid0, int32_t device, CatEnv** out) {
+  return create_env(maps, n_maps, worlds_per_map, pr, gid0, device, 0, out);
+}
+
+int cat_map_blob_bytes(const CatMapDesc* map, const CatParams* pr, int32_t* bytes) {
+  if (!map || !pr || !bytes) return fail(CAT_ERR_INVALID, "null argument");
+  const int rc = check_map(map, pr);
+  if (rc != CAT_OK) return rc;
+  *bytes = (int32_t)build_blob(map, pr).size();
+  return CAT_OK;
+}
+
+// 227 KB: the largest dynamic shared memory a block of an sm_100 device can opt in to
+static constexpr int kMaxBlobCapacity = 227 * 1024;
+
+int cat_env_create_swappable(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map, const CatParams* pr,
+                             int32_t blob_capacity, int64_t gid0, int32_t device, CatEnv** out) {
+  if (!maps || !worlds_per_map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
+  *out = nullptr;
+  if (pr->ray_list_cell < 0.0) return fail(CAT_ERR_INVALID, "a swappable environment needs ray lists (ray_list_cell >= 0)");
+  // the step kernel stages the blob with one cp.async.bulk of blob_bytes, which must be a multiple of 16; and no blob
+  // can exceed a block's shared memory (create_env checks the device's own limit before it allocates anything)
+  if (blob_capacity < 16 || blob_capacity % 16) return fail(CAT_ERR_INVALID, "blob_capacity must be a positive multiple of 16");
+  if (blob_capacity > kMaxBlobCapacity) return fail(CAT_ERR_LIMIT, "blob_capacity exceeds a block's shared memory");
+  return create_env(maps, n_maps, worlds_per_map, pr, gid0, device, blob_capacity, out);
+}
+
+// cat_env_create_multi, and with blob_capacity > 0 cat_env_create_swappable
+static int create_env(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map, const CatParams* pr,
+                      int64_t gid0, int32_t device, int blob_capacity, CatEnv** out) {
   if (!maps || !worlds_per_map || !pr || !out) return fail(CAT_ERR_INVALID, "null argument");
   *out = nullptr;
   if (n_maps < 1) return fail(CAT_ERR_INVALID, "n_maps must be >= 1");
@@ -494,18 +658,32 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
     if (rc != CAT_OK) return rc;
     if (maps[m].n_cops != maps[0].n_cops || maps[m].n_thieves != maps[0].n_thieves)
       return fail(CAT_ERR_INVALID, "every map of an environment needs the same numbers of cops and thieves");
+    if (blob_capacity > 0 && (int)build_blob(&maps[m], pr).size() > blob_capacity)
+      return fail(CAT_ERR_LIMIT, "map blob larger than blob_capacity");
     total += worlds_per_map[m];
   }
   if (total > 0x7FFFFFFFll) return fail(CAT_ERR_LIMIT, "too many worlds");
   const CatMapDesc* map = &maps[0];   // agents, rays and constants are the same for every map
   const int n_worlds = (int)total;
   const int A = map->n_cops + map->n_thieves, R = pr->n_rays;
-  const int P = A * (A - 1) / 2;
   CatEnv* env = new CatEnv();
   env->device = device;
   env->n_worlds = n_worlds;
+  env->swappable = blob_capacity > 0;
+  env->params = *pr;
   DeviceGuard guard(device);
   if (!guard.ok) { delete env; return fail(CAT_ERR_CUDA, "cudaSetDevice(" + std::to_string(device) + ") failed (no CUDA device?)"); }
+  if (blob_capacity > 0) {   // the capacity must leave room for two warps' scratch on this device, checked before any allocation
+    int optin = 0;
+    if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess) {
+      delete env;
+      return fail(CAT_ERR_CUDA, "cudaDeviceGetAttribute(cudaDevAttrMaxSharedMemoryPerBlockOptin) failed");
+    }
+    if ((long long)align_up(blob_capacity, 128) + 2LL * make_layout(A, R).scratch_bytes > optin) {
+      delete env;
+      return fail(CAT_ERR_LIMIT, "blob_capacity leaves no launch shape (shared memory per block: " + std::to_string(optin) + " B)");
+    }
+  }
   // every failure below goes through cat_env_destroy: nothing allocated so far is leaked
 #define CREATE_TRY(expr, what)                                                                              \
   do {                                                                                                      \
@@ -518,21 +696,13 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
   for (int m = 0, w0 = 0; m < n_maps; w0 += worlds_per_map[m], ++m) {
     EnvMap& em = env->maps[m];
     em.world_begin = w0; em.n_worlds = worlds_per_map[m];
-    const int rc = upload_map(&maps[m], pr, device, em);
+    const int rc = upload_map(&maps[m], pr, device, blob_capacity, em);
     if (rc != CAT_OK) { cat_env_destroy(env); return rc; }
     env->blob_bytes = std::max(env->blob_bytes, em.blob_bytes);
   }
 
   KParams& k = env->kp;
-  {   // map 0's values: what a single-map launch reads (a mixed-map launch reads each map's from its blob header)
-    const EnvMap& em = env->maps[0];
-    const BlobHeader& h = em.header;
-    k.blob = em.blob_dev; k.blob_bytes = em.blob_bytes;
-    k.view_off = h.view_off; k.view_edges = h.view_edges;
-    k.ray_slots = h.ray_slots; k.ray_ovf = h.ray_ovf; k.ray_slot_count = h.ray_slot_count; k.ray_ovf_words = h.ray_ovf_words;
-    k.rg_x0 = h.rg_x0; k.rg_y0 = h.rg_y0; k.rg_inv_cell = h.rg_inv_cell; k.rg_nx = h.rg_nx; k.rg_ny = h.rg_ny;
-    k.n_edges = h.n_edges;
-  }
+  set_map0_params(env);
   k.overflow = env->overflow_dev;
   k.n_worlds = n_worlds; k.gid0 = gid0;
   k.A = A; k.nc = map->n_cops; k.R = R;
@@ -570,8 +740,8 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
   // The attribute belongs to the FUNCTION (per device), not to this environment: always raise it to the device
   // maximum, so creating an environment for a smaller map never lowers the cap of one that is still alive.
   cudaFuncAttributes fattr{};
-  env->kernel = pick_world_kernel(A, R, k.ray_slots != nullptr, true, n_maps > 1);
-  env->kernel_record = pick_world_kernel(A, R, k.ray_slots != nullptr, false, n_maps > 1);
+  env->kernel = pick_world_kernel(A, R, k.ray_slots != nullptr, true, n_maps > 1 || env->swappable);
+  env->kernel_record = pick_world_kernel(A, R, k.ray_slots != nullptr, false, n_maps > 1 || env->swappable);
   CREATE_TRY(cudaFuncGetAttributes(&fattr, env->kernel), "cudaFuncGetAttributes");
   max_optin -= (int)fattr.sharedSizeBytes;      // the opt-in limit covers static + dynamic shared memory
   CREATE_TRY(cudaFuncSetAttribute(env->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin), "cudaFuncSetAttribute");
@@ -583,14 +753,7 @@ int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* 
   env->threads = shp.threads; env->smem_bytes = shp.smem;
   env->grid = fill_map_table(env, k, 0, n_worlds, shp.grid, shp.threads / 32);   // the table every full launch uses
 
-  // the environment's figures: map 0's, then the totals over the maps (worlds, list bytes, the largest blob, the grid)
-  CatEnvInfo& inf = env->info;
-  map_info(env, 0, inf);
-  for (int m = 1; m < n_maps; ++m) { CatEnvInfo other{}; map_info(env, m, other); inf.ray_list_bytes += other.ray_list_bytes; }
-  inf.n_worlds = n_worlds; inf.n_agents = A; inf.n_cops = map->n_cops; inf.n_thieves = map->n_thieves;
-  inf.n_rays = R; inf.state_dim = k.state_dim; inf.record_words = k.lay.rec_words;
-  inf.map_blob_bytes = env->blob_bytes; inf.smem_bytes_per_cta = env->smem_bytes; inf.warps_per_cta = env->threads / 32;
-  inf.grid = env->grid; inf.n_pairs = P;
+  env_info(env);
 #undef CREATE_TRY
   *out = env;
   return CAT_OK;
@@ -601,9 +764,7 @@ int cat_env_destroy(CatEnv* env) {
   DeviceGuard guard(env->device);
   for (EnvMap& m : env->maps) {
     if (m.blob_dev) cudaFree(m.blob_dev);
-    if (m.view_off_dev) cudaFree(m.view_off_dev);
-    if (m.view_edges_dev) cudaFree(m.view_edges_dev);
-    ray_lists_release(m.ray_lists);
+    release_map_tables(m);
   }
   if (env->overflow_dev) cudaFree(env->overflow_dev);
   for (cudaEvent_t e : env->chunk_events) cudaEventDestroy(e);
@@ -625,6 +786,58 @@ int cat_env_map_info(const CatEnv* env, int32_t map, CatEnvInfo* info) {
   CatEnvInfo inf = env->info;
   map_info(env, map, inf);
   *info = inf;
+  return CAT_OK;
+}
+
+int cat_env_set_map(CatEnv* env, int32_t m, const CatMapDesc* desc, void* stream) {
+  if (!env || !desc) return fail(CAT_ERR_INVALID, "null argument");
+  if (!env->swappable) return fail(CAT_ERR_INVALID, "the environment was not created by cat_env_create_swappable");
+  if (m < 0 || m >= (int)env->maps.size()) return fail(CAT_ERR_INVALID, "map index out of range");
+  const CatParams* pr = &env->params;
+  int rc = check_map(desc, pr);
+  if (rc != CAT_OK) return rc;
+  if (desc->n_cops != env->kp.nc || desc->n_cops + desc->n_thieves != env->kp.A)
+    return fail(CAT_ERR_INVALID, "the new map needs the environment's numbers of cops and thieves");
+  if ((int)build_blob(desc, pr).size() > env->blob_bytes) return fail(CAT_ERR_LIMIT, "map blob larger than the environment's blob_capacity");
+  DEVICE_SCOPE(env);
+  // build everything new first: on failure the environment keeps its old map
+  EnvMap fresh;
+  std::vector<unsigned char> blob;
+  rc = prepare_map(desc, pr, env->device, fresh, blob);
+  if (rc != CAT_OK) { release_map_tables(fresh); return rc; }
+  // a step in flight may still be staging the old blob (before griddepcontrol.wait): nothing is overwritten before it ends
+  cudaError_t e = cudaDeviceSynchronize();
+  EnvMap& em = env->maps[m];
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(em.blob_dev, blob.data(), blob.size(), cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess && em.blob_bytes > (int)blob.size()) e = cudaMemsetAsync(em.blob_dev + blob.size(), 0, em.blob_bytes - blob.size(), s);
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) { release_map_tables(fresh); return fail(CAT_ERR_CUDA, std::string("cat_env_set_map: ") + cudaGetErrorString(e)); }
+  release_map_tables(em);
+  em.view_off_dev = fresh.view_off_dev; em.view_edges_dev = fresh.view_edges_dev; em.ray_lists = fresh.ray_lists;
+  em.header = fresh.header;
+  if (m == 0) set_map0_params(env);
+  env_info(env);
+  return CAT_OK;
+}
+
+int cat_ray_lists_device(const CatMapDesc* map, int32_t n_rays, double ray_length, double rsum, double cell, double grid_out[5],
+                         uint32_t* slots_dev, int64_t* n_slot_words, uint32_t* ovf_dev, int64_t* n_ovf_words, int32_t device) {
+  if (!map || !grid_out || !n_slot_words || !n_ovf_words) return fail(CAT_ERR_INVALID, "null argument");
+  if (n_rays < 2 || n_rays > CAT_MAX_RAYS || map->n_hulls < 1 || map->n_edges > 65535) return fail(CAT_ERR_LIMIT, "ray / hull / edge count out of range");
+  DeviceGuard guard(device);
+  if (!guard.ok) return fail(CAT_ERR_CUDA, "cudaSetDevice(" + std::to_string(device) + ") failed (no CUDA device?)");
+  RayListDeviceBuild b;
+  int rc = b.size(map, n_rays, ray_length, rsum, cell);
+  if (rc != CAT_OK) return rc;
+  const RayListGrid& g = b.su.g;
+  grid_out[0] = g.x0; grid_out[1] = g.y0; grid_out[2] = g.cell; grid_out[3] = g.nx; grid_out[4] = g.ny;
+  if (slots_dev && ovf_dev) {
+    if (*n_slot_words < (int64_t)b.slot_words || *n_ovf_words < (int64_t)b.ovf_words) return fail(CAT_ERR_INVALID, "buffers too small");
+    rc = b.fill(slots_dev, ovf_dev);
+    if (rc != CAT_OK) return rc;
+  }
+  *n_slot_words = (int64_t)b.slot_words; *n_ovf_words = (int64_t)b.ovf_words;
   return CAT_OK;
 }
 

@@ -1,6 +1,7 @@
-// ray_lists.h — host-side (init time) builder of the per-(cell, ray) candidate lists of the sensor sweep.
-// Included by cat_b200.cu inside its anonymous namespace.  maps.ray_lists() is the numpy statement of the same
-// construction (tests/test_maps.py compares the two).
+// ray_lists.h — the per-(cell, ray) candidate lists of the sensor sweep: their layout, the host set-up both builders
+// share, and the host reference builder (cat_ray_lists_host).  Environments build their lists on the device
+// (ray_lists_kernel.cuh), which writes the same words.  Included by cat_b200.cu inside its anonymous namespace.
+// maps.ray_lists() is the numpy statement of the same construction (tests/test_maps.py compares the two).
 //
 // The sensor's ray directions are fixed (entity.py:182), so for ray index i the fat rays of every origin inside
 // a grid cell sweep the cell translated along direction i: in the ray's own frame (t along, w across) a region
@@ -66,10 +67,18 @@ inline uint32_t bound_bits(double lb) {
 
 }  // namespace raylist_detail
 
+// What both builders (this one and the device one, ray_lists_kernel.cuh) take from the host: the list grid, the sensor
+// reach, the rays' directions (cos / sin of the host's libm) and per edge its start vertex A and the next edge's normal.
+struct RayListSetup {
+  RayListGrid g;
+  double gx0 = 0.0, gy0 = 0.0, cell = 0.0, L = 0.0, rs = 0.0;
+  std::vector<double> ux, uy;          // [R]
+  std::vector<double> ax, ay, nnx, nny; // [E]
+};
+
 // `cell` <= 0: automatic.  Grid = bounding box of the hulls grown by the sensor reach: an origin outside it cannot
 // see any wall, so the kernel treats "outside the grid" as "empty lists".
-static void build_ray_lists(const CatMapDesc* map, int R, double L, double rsum, double cell, RayLists* out) {
-  using namespace raylist_detail;
+static void ray_list_setup(const CatMapDesc* map, int R, double L, double rsum, double cell, RayListSetup* s) {
   const int H = map->n_hulls, E = map->n_edges;
   const double eps = 1e-2, rs = rsum + eps, reach = L + rs + 1.0;
   double bl = 1e300, bb = 1e300, br = -1e300, bt = -1e300;
@@ -81,7 +90,7 @@ static void build_ray_lists(const CatMapDesc* map, int R, double L, double rsum,
   // automatic: about 64k cells, not below 6 units (narrower strips = shorter lists = fewer edge tests and fewer overflow
   // links per ray).  Measured on agh-map x 16384, us per step: 308 / 248 / 208 / 198 / 187 at 48 / 32 / 19 / 16 / 12 units
   // with the first list kernel; 137 / 129 / 124 / 121 / 120 at 13.6 / 10 / 8 / 6.8 / 6.3 units with the final one
-  // (33 / 58 / 88 / 120 / 136 MB of lists: HBM is not the scarce resource here, and the builder takes about a second).
+  // (33 / 58 / 88 / 120 / 136 MB of lists: HBM is not the scarce resource here).
   if (!(cell > 0.0)) {
     double target = 65536.0, min_cell = 6.0;
     if (const char* e = getenv("CAT_RAY_LIST_CELLS")) { const double v = atof(e); if (v >= 64.0) target = v; }          // tuning knobs
@@ -89,31 +98,46 @@ static void build_ray_lists(const CatMapDesc* map, int R, double L, double rsum,
     cell = std::max(min_cell, sqrt(gw * gh / target));
   }
   const int nx = std::max(1, (int)ceil(gw / cell)), ny = std::max(1, (int)ceil(gh / cell));
-  out->g.x0 = (float)gx0; out->g.y0 = (float)gy0; out->g.cell = (float)cell; out->g.inv_cell = (float)(1.0 / cell);
-  out->g.nx = nx; out->g.ny = ny;
+  s->g.x0 = (float)gx0; s->g.y0 = (float)gy0; s->g.cell = (float)cell; s->g.inv_cell = (float)(1.0 / cell);
+  s->g.nx = nx; s->g.ny = ny;
+  s->gx0 = gx0; s->gy0 = gy0; s->cell = cell; s->L = L; s->rs = rs;
 
   // per edge: A (start), B (end = vert[e]), n, next normal
-  std::vector<double> ax(E), ay(E), nnx(E), nny(E);
-  std::vector<int> ehull(E);
+  s->ax.assign(E, 0.0); s->ay.assign(E, 0.0); s->nnx.assign(E, 0.0); s->nny.assign(E, 0.0);
   for (int h = 0; h < H; ++h) {
     const int o = map->hull_off[h], e1 = map->hull_off[h + 1];
     for (int e = o; e < e1; ++e) {
       const int p = e > o ? e - 1 : e1 - 1, q = e + 1 < e1 ? e + 1 : o;
-      ax[e] = map->vert[2 * p]; ay[e] = map->vert[2 * p + 1];
-      nnx[e] = map->normal[2 * q]; nny[e] = map->normal[2 * q + 1];
-      ehull[e] = h;
+      s->ax[e] = map->vert[2 * p]; s->ay[e] = map->vert[2 * p + 1];
+      s->nnx[e] = map->normal[2 * q]; s->nny[e] = map->normal[2 * q + 1];
     }
   }
-  // (2) per (ray, edge), direction only
-  std::vector<double> ux(R), uy(R);
-  std::vector<uint8_t> against((size_t)R * E);
+  s->ux.resize(R); s->uy.resize(R);
   for (int i = 0; i < R; ++i) {
     const double th = i * (2.0 * M_PI / R);
-    ux[i] = cos(th); uy[i] = sin(th);
+    s->ux[i] = cos(th); s->uy[i] = sin(th);
+  }
+}
+
+// The reference builder (host threads): cat_ray_lists_host.  Environments build their lists with the device builder,
+// which gives the same words.
+static void build_ray_lists(const CatMapDesc* map, int R, double L, double rsum, double cell, RayLists* out) {
+  using namespace raylist_detail;
+  const int H = map->n_hulls, E = map->n_edges;
+  const double eps = 1e-2;
+  RayListSetup su;
+  ray_list_setup(map, R, L, rsum, cell, &su);
+  out->g = su.g;
+  const double rs = su.rs, gx0 = su.gx0, gy0 = su.gy0;
+  cell = su.cell;
+  const int nx = su.g.nx, ny = su.g.ny;
+  const std::vector<double>& ax = su.ax, &ay = su.ay, &nnx = su.nnx, &nny = su.nny, &ux = su.ux, &uy = su.uy;
+  // (2) per (ray, edge), direction only
+  std::vector<uint8_t> against((size_t)R * E);
+  for (int i = 0; i < R; ++i)
     for (int e = 0; e < E; ++e)
       against[(size_t)i * E + e] = (ux[i] * map->normal[2 * e] + uy[i] * map->normal[2 * e + 1] < 1e-4) ||
                                    (ux[i] * nnx[e] + uy[i] * nny[e] < 1e-4);
-  }
 
   out->slots.assign((size_t)nx * ny * R * 4, kRayEnd);
   std::vector<std::vector<uint32_t>> row_ovf(ny);

@@ -268,13 +268,17 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
     ``spawn_override`` is None or one entry per map, ``cell`` applies to every map.  Map m owns a contiguous block of
     the worlds (``map_index`` gives the map of each, ``map_names`` their names), one launch steps all of them, and the
     observation, state and critic layouts are the single-map ones.  ``team_positions`` is bounded by the largest window.
+
+    ``swappable_maps=True``: ``set_map(m, map)`` replaces map m of the live environment (a procedural layout, say:
+    ``maps.generate_maze``) and resets its worlds, without re-creating the environment, its buffers or a captured
+    rollout graph (``CatWorlds.set_map``).
     """
 
     def __init__(self, map: Union[Map, Sequence[Map]], num_envs: Union[int, Sequence[int]], *, max_step_count: int = 400,
                  time_step: float = 1 / 60.0, device: Union[str, torch.device] = "cuda:0", seed: int = 0, gid0: int = 0,
                  physical_params: Optional[dict] = None, stale_shape_cache: bool = True,
                  spawn_override: Optional[Union[dict, Sequence[Optional[dict]]]] = None, cell: Optional[float] = None,
-                 render_mode=None, final_observations: bool = False):
+                 render_mode=None, final_observations: bool = False, swappable_maps: bool = False):
         params = _make_params(max_step_count, time_step, physical_params, auto_reset=1, seed=int(seed),
                               stale_shape_cache=int(stale_shape_cache))
         self._params = params
@@ -284,7 +288,7 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._cmaps = [self._cmap]
             self._setup_common(map, self._cmap, params)
             self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True,
-                                want_final=final_observations)
+                                want_final=final_observations, swappable_maps=swappable_maps)
         else:
             self.maps = list(map)
             n = len(self.maps)
@@ -301,8 +305,9 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             window = (max(m.window_dimensions[0] for m in self.maps), max(m.window_dimensions[1] for m in self.maps))
             self._setup_common(self.maps[0], self._cmap, params, window=window)
             self._w = CatWorlds(self._cmaps, counts, device=device, gid0=gid0, params=params, want_f32=True,
-                                want_critic=True, want_final=final_observations)
+                                want_critic=True, want_final=final_observations, swappable_maps=swappable_maps)
             num_envs = sum(counts)
+        self._cell = cell
         self.map_names = [c.name for c in self._cmaps]
         self.map_index = self._w.map_index
         self.num_envs = int(num_envs)
@@ -317,6 +322,26 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
     @property
     def worlds(self) -> CatWorlds:
         return self._w
+
+    def set_map(self, m: int, map: Map, spawn_override: Optional[dict] = None) -> torch.Tensor:
+        """Replace map ``m`` of a ``swappable_maps`` environment by ``map`` (same agents; compiled with this
+        environment's ``cell``) and reset its worlds; returns the (N,) bool mask of those worlds, whose observations in
+        the step's output views are now their first ones on the new map.  Pass the mask to ``MAPPOLearner.note_reset``
+        so that their recurrent states start afresh.  ``maps``, ``map_names`` and the shared observation spaces
+        (``team_positions`` is bounded by the largest window) follow the new map."""
+        cmap = compile_map(map, spawn_override=spawn_override, cell=self._cell)
+        if cmap.agent_ids != self._cmap.agent_ids:
+            raise ValueError("the new map needs the environment's agents")
+        mask = self._w.set_map(m, cmap)
+        self.maps[m] = map
+        self._cmaps[m] = cmap
+        self._cmap = self._cmaps[0]
+        self.map_names[m] = cmap.name
+        window = (max(mp.window_dimensions[0] for mp in self.maps), max(mp.window_dimensions[1] for mp in self.maps))
+        self._setup_common(self.maps[0], self._cmap, self._params, window=window)
+        _EnvCommon.get_nested_agent_observation_spaces.cache_clear()   # built from the old spaces
+        self.state_spaces = {a: self.shared_observation_spaces for a in self.possible_agents}
+        return mask
 
     def state_space_of(self, agent: str):
         return self.state_spaces[agent]

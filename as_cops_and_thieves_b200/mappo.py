@@ -405,6 +405,12 @@ class MAPPOLearner:
     def note_done(self, done: torch.Tensor) -> None:
         self._prev_done.copy_(done.view(-1).bool())
 
+    def note_reset(self, mask: torch.Tensor) -> None:
+        """Worlds reset outside the rollout (``BatchedCopsThievesEnv.set_map`` returns their (N,) mask): their
+        recurrent states are zeroed at the next step, as after an episode end.  In place, so a captured rollout graph
+        stays valid and is not recaptured."""
+        self._prev_done.logical_or_(mask.to(device=self._prev_done.device).view(-1).bool())
+
     def reset_recurrent_state(self) -> None:
         """Zero every carried (h, c) and the done flags IN PLACE (the rollout graph holds these buffers)."""
         for a in self.agents:

@@ -80,12 +80,35 @@ class Map:
         self.unit_size = 5.0
         self.blocks: List[List[Tuple[float, float]]] = []
         self.agent_spawn_regions: Dict[str, List[dict]] = {}
-        self._parse_json_map(self.map_path, scale, agents)
+        with open(self.map_path, "r") as f:
+            self._parse_map_data(json.load(f), scale, agents)
+
+    @classmethod
+    def from_dict(cls, data: dict, name: str) -> "Map":
+        """A map from an already parsed JSON document of either schema ``Map(path)`` reads (``catmap-1`` or the
+        reference's); ``name`` stands in for the file name (``compile_map`` names the compiled map after it)."""
+        m = cls.__new__(cls)
+        m.map_path = str(name)
+        m.unit_size = 5.0
+        m.blocks, m.agent_spawn_regions = [], {}
+        m._parse_map_data(data, None, None)
+        return m
+
+    def to_dict(self) -> dict:
+        """The ``catmap-1`` document of this map (what ``Map.from_dict`` and ``Map(path)`` read back)."""
+        counts: Dict[str, int] = {}
+        agents = []
+        for a in self._agents:
+            idx = counts.get(a["type"], 0)
+            counts[a["type"]] = idx + 1
+            regs = self.agent_spawn_regions.get(f"{a['type']}_{idx}")
+            agents.append({"type": a["type"], "pos": [a["x"], a["y"]],
+                           **({"regions": [[r["x"], r["y"], r["w"], r["h"]] for r in regs]} if regs else {})})
+        return {"format": "catmap-1", "window": list(self.window_dimensions), "canvas": list(self.canvas_dimensions),
+                "blocks": [[c for v in ring for c in v] for ring in self.blocks], "agents": agents}
 
     # ------------------------------------------------------------------ parsing
-    def _parse_json_map(self, map_path: str, scale, agents_override) -> None:
-        with open(map_path, "r") as f:
-            data = json.load(f)
+    def _parse_map_data(self, data: dict, scale, agents_override) -> None:
         if data.get("format") == "catmap-1":
             self.window_dimensions = tuple(data["window"])
             self.canvas_dimensions = tuple(data["canvas"])
@@ -573,8 +596,125 @@ LABYRINTH_AGENTS = [
 ]
 
 
+#: the maps shipped under maps_data/
+SHIPPED_MAPS = ("squarinth", "labyrinth", "lbirinth", "grandbyrinth", "agh-map")
+
+
 def load_named_map(name: str) -> Map:
     """Built-in maps by the names BASELINE.json uses; labyrinth gets its scale + injected agents."""
     if name == "labyrinth":
         return Map(builtin_map_path(name), scale=LABYRINTH_SCALE, agents=LABYRINTH_AGENTS)
     return Map(builtin_map_path(name))
+
+
+# ---------------------------------------------------------------------------------- procedural maps
+#: clearance of a maze's spawn regions from every wall hull beyond agent radius + wall radius
+MAZE_SPAWN_MARGIN = 2.0
+
+
+def generate_maze(seed: int, *, cols: int = 16, rows: int = 9, window: Tuple[float, float] = (1280.0, 720.0),
+                  corridor: float = 60.0, wall: float = 16.0, n_cops: int = 2, n_thieves: int = 1,
+                  agent_radius: float = 5.0, margin: float = MAZE_SPAWN_MARGIN) -> Map:
+    """A perfect maze (exactly one path between any two cells) on a ``cols`` x ``rows`` grid, as a ``Map`` named
+    ``maze-<seed>``.  The same seed gives the same maze on every host and rank (numpy's PCG64 stream).
+
+    Cells are ``corridor`` units wide and separated by walls ``wall`` units thick; the maze is centred in ``window``.  Each
+    straight run of wall segments along a grid line is one axis-aligned rect block (the outer boundary is four of them),
+    so the map has few hulls and edges.  The cops spawn in one cell and the thieves in another, the two ends of a longest
+    path of the maze; each spawn region keeps ``agent_radius + WALL_RADIUS + margin`` from every hull."""
+    pitch = corridor + wall
+    width, height = cols * pitch + wall, rows * pitch + wall
+    if cols < 2 or rows < 2 or corridor <= 0 or wall <= 0:
+        raise ValueError("a maze needs cols, rows >= 2 and positive corridor and wall widths")
+    if width > window[0] or height > window[1]:
+        raise ValueError(f"a {cols} x {rows} maze of pitch {pitch} ({width} x {height}) does not fit the window {window}")
+    clear = agent_radius + WALL_RADIUS + margin
+    if corridor <= 2 * clear:
+        raise ValueError(f"corridor {corridor} leaves no spawn region at clearance {clear}")
+    x0, y0 = (window[0] - width) / 2.0, (window[1] - height) / 2.0
+    rng = np.random.default_rng(int(seed))
+    # recursive backtracker over the cells; open_e[c, r]: passage (c, r) <-> (c + 1, r), open_n: (c, r) <-> (c, r + 1)
+    open_e = np.zeros((cols, rows), bool)
+    open_n = np.zeros((cols, rows), bool)
+    seen = np.zeros((cols, rows), bool)
+    stack = [(int(rng.integers(cols)), int(rng.integers(rows)))]
+    seen[stack[0]] = True
+    while stack:
+        c, r = stack[-1]
+        nbrs = [(dc, dr) for dc, dr in ((1, 0), (-1, 0), (0, 1), (0, -1))
+                if 0 <= c + dc < cols and 0 <= r + dr < rows and not seen[c + dc, r + dr]]
+        if not nbrs:
+            stack.pop()
+            continue
+        dc, dr = nbrs[int(rng.integers(len(nbrs)))]
+        if dc:
+            open_e[min(c, c + dc), r] = True
+        else:
+            open_n[c, min(r, r + dr)] = True
+        seen[c + dc, r + dr] = True
+        stack.append((c + dc, r + dr))
+
+    blocks: List[List[Tuple[float, float]]] = []
+
+    def rect(x, y, w, h):
+        blocks.append([(x, y), (x + w, y), (x + w, y + h), (x, y + h), (x, y)])
+
+    # horizontal grid line j: segment i (under cell (i, j)) is a wall unless the cells (i, j - 1) and (i, j) connect
+    for j in range(rows + 1):
+        seg = [j in (0, rows) or not open_n[i, j - 1] for i in range(cols)]
+        i = 0
+        while i < cols:
+            if not seg[i]:
+                i += 1
+                continue
+            k = i
+            while k + 1 < cols and seg[k + 1]:
+                k += 1
+            rect(x0 + i * pitch, y0 + j * pitch, (k - i + 1) * pitch + wall, wall)
+            i = k + 1
+    # vertical grid line i: segment j is a wall unless the cells (i - 1, j) and (i, j) connect
+    for i in range(cols + 1):
+        seg = [i in (0, cols) or not open_e[i - 1, j] for j in range(rows)]
+        j = 0
+        while j < rows:
+            if not seg[j]:
+                j += 1
+                continue
+            k = j
+            while k + 1 < rows and seg[k + 1]:
+                k += 1
+            rect(x0 + i * pitch, y0 + j * pitch, wall, (k - j + 1) * pitch + wall)
+            j = k + 1
+
+    def farthest(start):
+        dist = {start: 0}
+        queue = [start]
+        for c, r in queue:
+            for nc, nr, ok in ((c + 1, r, c + 1 < cols and open_e[c, r]), (c - 1, r, c > 0 and open_e[c - 1, r]),
+                               (c, r + 1, r + 1 < rows and open_n[c, r]), (c, r - 1, r > 0 and open_n[c, r - 1])):
+                if ok and (nc, nr) not in dist:
+                    dist[(nc, nr)] = dist[(c, r)] + 1
+                    queue.append((nc, nr))
+        return queue[-1]          # BFS order: the last cell reached is a farthest one
+    cop_cell = farthest((0, 0))
+    thief_cell = farthest(cop_cell)
+
+    def region(cell):
+        c, r = cell
+        return dict(x=x0 + c * pitch + wall + clear, y=y0 + r * pitch + wall + clear,
+                    w=corridor - 2 * clear, h=corridor - 2 * clear)
+
+    def centre(cell):
+        c, r = cell
+        return x0 + c * pitch + wall + corridor / 2.0, y0 + r * pitch + wall + corridor / 2.0
+    agents = []
+    for kind, n, cell in (("cop", n_cops, cop_cell), ("thief", n_thieves, thief_cell)):
+        cy = centre(cell)[1]
+        reg = region(cell)
+        for a in range(n):   # distinct start positions inside the cell's spawn region, spread along x
+            px = reg["x"] + reg["w"] * (a + 1) / (n + 1)
+            agents.append({"type": kind, "pos": [px, cy], "regions": [[reg["x"], reg["y"], reg["w"], reg["h"]]]})
+    data = {"format": "catmap-1", "window": [float(window[0]), float(window[1])],
+            "canvas": [float(window[0]), float(window[1])],
+            "blocks": [[float(c) for v in ring for c in v] for ring in blocks], "agents": agents}
+    return Map.from_dict(data, f"maze-{int(seed)}")

@@ -203,7 +203,8 @@ class TrajectoryRecorder:
     worlds' positions and maps, with ``rays`` what their sensors report from those positions (``CatWorlds.sensor_rays``,
     one extra observe launch: the observation a step returns was taken before it moved the agents), and the step's
     rewards, terminated, truncated and winner.  ``frames()`` renders recorded steps in one launch; ``save()`` writes an ``.npz`` that ``render_rgb``
-    can redraw without a GPU (``redraw``)."""
+    can redraw without a GPU (``redraw``).  Both raise if the environment replaced a map (``set_map``) after recording
+    began: the recorded map indices would then name the new map."""
 
     def __init__(self, env, worlds: Union[Sequence[int], "object"], capacity: int, rays: bool = True):
         import torch
@@ -226,6 +227,8 @@ class TrajectoryRecorder:
         if self.t >= self.capacity:
             raise IndexError(f"the recorder is full ({self.capacity} steps)")
         w, t, idx = self.w, self.t, self.worlds
+        if t == 0:
+            self._maps_replaced = w.maps_replaced
         torch.index_select(w.positions(), 0, idx, out=self.pos[t])
         torch.index_select(w.map_index, 0, idx, out=self.map_of[t])
         if self.rays:
@@ -238,8 +241,14 @@ class TrajectoryRecorder:
         torch.index_select(w.winner, 0, idx, out=self.winner[t])
         self.t += 1
 
+    def _check_maps(self) -> None:
+        if self.t and self.w.maps_replaced != self._maps_replaced:
+            raise RuntimeError("the environment replaced a map (set_map) after this recording began: its map indices "
+                               "no longer name the maps the steps ran on")
+
     def frames(self, start: int = 0, stop: Optional[int] = None, downsample: int = 1):
         """(stop - start, K, W', H', 3) uint8 frames of the recorded steps [start, stop), one launch."""
+        self._check_maps()
         stop = self.t if stop is None else min(int(stop), self.t)
         n, K, A, R = max(0, stop - start), self.worlds.numel(), self.w.A, self.w.R
         rays = None
@@ -251,6 +260,7 @@ class TrajectoryRecorder:
 
     def save(self, path) -> None:
         """``.npz`` of the recorded steps, with the map names and ray directions ``redraw`` needs."""
+        self._check_maps()
         t = self.t
         arrays = dict(worlds=self.worlds.cpu().numpy(), map_names=np.array([c.name for c in self.w.cmaps]),
                       windows=np.array([c.window for c in self.w.cmaps], np.int32),

@@ -8,6 +8,7 @@ path: constructing it without a CUDA device raises.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 from typing import Dict, Mapping, Optional, Sequence, Union
 
 import numpy as np
@@ -68,12 +69,46 @@ def _map_desc(cmap: CompiledMap):
     return md, keep
 
 
+def _cat_params(p: Mapping) -> CatParams:
+    return CatParams(**{name: p[name] for name, _ in CatParams._fields_})
+
+
+def map_blob_bytes(cmap: CompiledMap, params: Mapping) -> int:
+    """``cat_map_blob_bytes``: the shared-memory blob of ``cmap`` under the parameters ``params`` (an ``EnvParams``
+    dict), what a swappable environment's ``map_blob_capacity`` must cover.  Host only."""
+    L = _lib.load()
+    md, _keep = _map_desc(cmap)
+    cp = _cat_params(params)
+    out = C.c_int32(0)
+    _lib.check(L.cat_map_blob_bytes(C.byref(md), C.byref(cp), C.byref(out)), "cat_map_blob_bytes")
+    return int(out.value)
+
+
+@functools.lru_cache(maxsize=8)
+def _shipped_blob_capacity(key: tuple) -> int:
+    from .maps import SHIPPED_MAPS, compile_map, free_space_regions, load_named_map
+    params = dict(key)
+    best = 0
+    for name in SHIPPED_MAPS:
+        m = load_named_map(name)
+        for so in (None, free_space_regions(m)):
+            best = max(best, map_blob_bytes(compile_map(m, name=name, spawn_override=so), params))
+    return best
+
+
+def default_blob_capacity(params: Mapping) -> int:
+    """The largest blob of the shipped maps (with their own spawn regions and with ``free_space_regions``) under
+    ``params``: the default ``map_blob_capacity`` of a swappable environment (agh-map's blob)."""
+    return _shipped_blob_capacity(tuple(sorted((k, params[k]) for k, _ in CatParams._fields_)))
+
+
 class CatWorlds:
     def __init__(self, cmap: Union[CompiledMap, Sequence[CompiledMap]], n_worlds: Union[int, Sequence[int]], *,
                  device: Union[str, torch.device] = "cuda:0",
                  gid0: int = 0, params: Optional[EnvParams] = None, want_f32: bool = True,
                  want_shared: bool = True, want_hits: bool = False, pinned_outputs: bool = False,
-                 want_critic: bool = False, want_bf16: bool = False, want_final: bool = False, **overrides):
+                 want_critic: bool = False, want_bf16: bool = False, want_final: bool = False,
+                 swappable_maps: bool = False, map_blob_capacity: Optional[int] = None, **overrides):
         """``pinned_outputs=True`` places every output tensor in mapped pinned HOST memory: the kernel stores its
         results there directly and the host reads them (``tensor.numpy()``) after one stream synchronisation —
         the layout for callers that consume every step on the CPU, like the single-world PettingZoo face.
@@ -94,7 +129,16 @@ class CatWorlds:
         ``world_offsets[m] .. world_offsets[m] + n_worlds[m]`` and all of them are stepped by one launch; world i is
         the same world as world ``i - world_offsets[m]`` of a single-map ``CatWorlds`` of map m with
         ``gid0 + world_offsets[m]``.  ``cmaps``, ``world_offsets`` and ``map_index`` (the map of every world, (N,) int64
-        on the device) describe the split; with one map they hold that map alone."""
+        on the device) describe the split; with one map they hold that map alone.
+
+        ``swappable_maps``: the environment is created by ``cat_env_create_swappable``, so ``set_map`` can replace any
+        of its maps later without invalidating its buffers or a captured CUDA graph.  Each map's blob is then allocated
+        at ``map_blob_capacity`` bytes (a positive multiple of 16; default: the largest blob of the creation maps and the
+        shipped maps, ``default_blob_capacity``), and the mixed-map kernels run even for one map.  Needs ray lists
+        (``ray_list_cell >= 0``)."""
+        if map_blob_capacity is not None and (int(map_blob_capacity) < 16 or int(map_blob_capacity) % 16):
+            # the step kernel stages a blob with one bulk copy whose size must be a multiple of 16 bytes
+            raise ValueError(f"map_blob_capacity must be a positive multiple of 16, got {map_blob_capacity}")
         if isinstance(cmap, CompiledMap):
             multi, cmaps, counts = False, [cmap], [int(n_worlds)]
         else:
@@ -119,10 +163,20 @@ class CatWorlds:
 
         descs = [_map_desc(m) for m in cmaps]
         self._keep = [kp for _, kp in descs]
-        cp = CatParams(**{name: p[name] for name, _ in CatParams._fields_})
+        cp = _cat_params(p)
         handle = C.c_void_p()
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        if multi:
+        self.swappable = bool(swappable_maps)
+        self.maps_replaced = 0       # set_map calls so far (render.TrajectoryRecorder checks it)
+        if self.swappable:
+            if map_blob_capacity is None:
+                map_blob_capacity = max([default_blob_capacity(p)] + [map_blob_bytes(m, p) for m in cmaps])
+            self.map_blob_capacity = int(map_blob_capacity)
+            mds = (CatMapDesc * len(cmaps))(*[md for md, _ in descs])
+            cnt = (C.c_int32 * len(counts))(*counts)
+            _lib.check(self.L.cat_env_create_swappable(mds, len(cmaps), cnt, C.byref(cp), self.map_blob_capacity, self.gid0,
+                                                       dev_index, C.byref(handle)), "cat_env_create_swappable")
+        elif multi:
             mds = (CatMapDesc * len(cmaps))(*[md for md, _ in descs])
             cnt = (C.c_int32 * len(counts))(*counts)
             _lib.check(self.L.cat_env_create_multi(mds, len(cmaps), cnt, C.byref(cp), self.gid0, dev_index,
@@ -238,6 +292,32 @@ class CatWorlds:
         info = CatEnvInfo()
         _lib.check(self.L.cat_env_map_info(self._h, int(m), C.byref(info)), "cat_env_map_info")
         return info
+
+    def set_map(self, m: int, cmap: CompiledMap) -> torch.Tensor:
+        """Replace map ``m`` of a swappable environment by ``cmap`` (same cops and thieves; its blob must fit
+        ``map_blob_capacity``) and reset that map's worlds: ``cat_env_set_map``, then ``reset(mask)``, so the outputs of
+        those worlds hold their first observation on the new map, as after ``reset(mask)``.  The other worlds are not
+        touched.  Synchronises the device and may allocate: call it between steps, outside graph capture.  A CUDA graph
+        captured before stays valid and steps the new map on its next replay.  Returns the (N,) bool mask of the reset
+        worlds (a recurrent learner zeroes their states: ``MAPPOLearner.note_reset``).  On failure nothing changes."""
+        m = int(m)
+        if not 0 <= m < len(self.cmaps):
+            raise IndexError(f"map index {m} out of range (0..{len(self.cmaps) - 1})")
+        md, keep = _map_desc(cmap)
+        _lib.check(self.L.cat_env_set_map(self._h, m, C.byref(md), self._stream()), "cat_env_set_map")
+        del keep
+        self.cmaps[m] = cmap
+        self.cmap = self.cmaps[0]
+        self.maps_replaced += 1
+        info = CatEnvInfo()
+        _lib.check(self.L.cat_env_info(self._h, C.byref(info)), "cat_env_info")
+        self.info = info
+        if getattr(self, "_renderer", None) is not None:   # it holds the old map's wall layer: rebuilt on next use
+            self._renderer.close()
+            self._renderer = None
+        mask = self.map_index == m
+        self.reset(mask)
+        return mask
 
     def overflow_counts(self, reset: bool = False):
         """(wall contacts beyond CAT_WALL_SLOTS, near hulls beyond CAT_NEAR_SLOTS) since creation / the last reset

@@ -222,6 +222,35 @@ int cat_env_create(const CatMapDesc* map, const CatParams* params, int32_t n_wor
  * Every other entry point works on such an environment as on a single-map one. */
 int cat_env_create_multi(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map,
                          const CatParams* params, int64_t gid0, int32_t device, CatEnv** out);
+/* A cat_env_create_multi environment whose maps can be replaced later (cat_env_set_map), e.g. to cycle a training run
+ * through procedurally generated layouts without re-creating the environment, its buffers or a captured CUDA graph.
+ * It differs from cat_env_create_multi in three ways:
+ *   - it always runs the mixed-map kernels, even with one map: they read every map-dependent value (list pointers and
+ *     grid, counts) from the blob each CTA stages, never from the launch parameters a captured graph keeps;
+ *   - every map's blob is allocated once at blob_capacity bytes, and CatEnvInfo.map_blob_bytes and the launch shape
+ *     are those of the capacity, so replacing a map changes neither.  blob_capacity must be a positive multiple of 16
+ *     (the kernel stages the blob with one bulk copy of that size; CAT_ERR_INVALID otherwise) and >= every creation
+ *     map's cat_map_blob_bytes; CAT_ERR_LIMIT if it is smaller, larger than 227 KB, or leaves no launch shape in the
+ *     device's shared memory (checked before anything is allocated);
+ *   - it needs (cell, ray) lists: params->ray_list_cell < 0 returns CAT_ERR_INVALID.
+ * Every other argument and result is cat_env_create_multi's. */
+int cat_env_create_swappable(const CatMapDesc* maps, int32_t n_maps, const int32_t* worlds_per_map,
+                             const CatParams* params, int32_t blob_capacity, int64_t gid0, int32_t device, CatEnv** out);
+/* Replace map m of a swappable environment by `desc` (same numbers of cops and thieves).  Checked before any CUDA call:
+ * CAT_ERR_INVALID if the environment is not swappable, m is out of range, desc is NULL or its agent counts differ;
+ * CAT_ERR_LIMIT if its blob (cat_map_blob_bytes) exceeds the environment's blob_capacity.  The new view lists and
+ * (cell, ray) lists are built first (the lists on the device, shared through the same cache as at creation); only then is
+ * the blob copied into the existing allocation, its tail zeroed, and the old map's lists released.  On any failure the
+ * environment stays on its old map.
+ * Ordering: a step kernel stages its map's blob before it waits on the previous kernel (programmatic dependent launch),
+ * so this call synchronises the DEVICE before it overwrites anything and again before it returns.  It may allocate and is
+ * not graph-capturable; a graph captured before it stays valid and steps the new map on its next replay.
+ * World state is not touched: the worlds of map m still hold positions on the old map and MUST be reset
+ * (cat_env_reset with a mask of those worlds) before the next step. */
+int cat_env_set_map(CatEnv* env, int32_t m, const CatMapDesc* desc, void* stream);
+/* host only: the bytes of the shared-memory blob of this map with these parameters (what blob_capacity must cover);
+ * the map is checked as cat_env_create checks it */
+int cat_map_blob_bytes(const CatMapDesc* map, const CatParams* params, int32_t* bytes);
 int cat_env_destroy(CatEnv* env);
 /* n_worlds: every world of the environment; ray_list_bytes: the sum over its maps; map_blob_bytes: the largest blob;
  * the other map-dependent fields (n_hulls, n_edges, ray_list_cells/nx/ny/cell) describe map 0 */
@@ -265,12 +294,18 @@ int cat_env_get_state(CatEnv* env, const void* state_dev, const CatStateView* vi
 int cat_env_set_state(CatEnv* env, void* state_dev, const CatStateView* view, void* stream);
 
 /* Inspection / test entry point (host only, needs no GPU): the per-(cell, ray) candidate lists cat_env_create builds for
- * this map and these sensor parameters (csrc/ray_lists.h).  grid_out = {x0, y0, cell, nx, ny}.  Call with slots = ovf =
+ * this map and these sensor parameters, from the host reference builder (csrc/ray_lists.h).  grid_out = {x0, y0, cell, nx, ny}.  Call with slots = ovf =
  * NULL to get the sizes (in 32-bit words) in n_slot_words / n_ovf_words, then again with buffers of those sizes.
  * slot[(cell * n_rays + ray) * 4 .. +4]: entries (bf16 bits of the lower bound of the hit distance << 16 | edge id),
  * 0x7F80FFFF = end, bit 31 = link to a 4-word chunk of ovf (word offset in the low 31 bits). */
 int cat_ray_lists_host(const CatMapDesc* map, int32_t n_rays, double ray_length, double rsum, double cell,
                        double grid_out[5], uint32_t* slots, int64_t* n_slot_words, uint32_t* ovf, int64_t* n_ovf_words);
+/* The same lists built on device `device` by the builder every environment uses (csrc/ray_lists_kernel.cuh): the same
+ * words as cat_ray_lists_host, into DEVICE buffers slots / ovf, with the same two-call sizing protocol.  Synchronises the
+ * device; CAT_ERR_CUDA without one. */
+int cat_ray_lists_device(const CatMapDesc* map, int32_t n_rays, double ray_length, double rsum, double cell,
+                         double grid_out[5], uint32_t* slots, int64_t* n_slot_words, uint32_t* ovf, int64_t* n_ovf_words,
+                         int32_t device);
 
 /* skrl MAPPO._update GAE (SURVEY.md a-10; call site agent_learning_utils.py:198-199).
  * rewards/values [T][M] f32, dones [T][M] u8, last_values [M]; returns/advantages [T][M].

@@ -5,6 +5,7 @@ all-reduced over NCCL per minibatch.
 
     python tools/train_selfplay.py --map agh-map --worlds 4096 --iterations 2 --timesteps 256
     python tools/train_selfplay.py --map squarinth,agh-map,labyrinth --worlds 4096   # one policy over three maps
+    python tools/train_selfplay.py --map squarinth --procedural 2 --swap-every 4     # + 2 slots of fresh mazes
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_selfplay.py ...
 
 Prints one JSON line per self-play iteration (rank 0): environment agent-steps/s inside training, GAE / update /
@@ -23,7 +24,7 @@ sys.path.insert(0, str(ROOT))
 from as_cops_and_thieves_b200 import selfplay  # noqa: E402
 from as_cops_and_thieves_b200.env import BatchedCopsThievesEnv  # noqa: E402
 from as_cops_and_thieves_b200.mappo import MAPPOConfig, MAPPOLearner  # noqa: E402
-from as_cops_and_thieves_b200.maps import free_space_regions, load_named_map  # noqa: E402
+from as_cops_and_thieves_b200.maps import free_space_regions, generate_maze, load_named_map  # noqa: E402
 from as_cops_and_thieves_b200.sharding import dist_env, shard_range  # noqa: E402
 
 
@@ -46,6 +47,11 @@ def main():
                          "number of worlds (same number of transitions), the reference's values as they are, or none")
     ap.add_argument("--time-limit-bootstrap", action="store_true",
                     help="bootstrap timed-out episodes from the critic's value of their final observation")
+    ap.add_argument("--procedural", type=int, default=0,
+                    help="add this many map slots holding generated mazes (maps.generate_maze) to --map")
+    ap.add_argument("--swap-every", type=int, default=0,
+                    help="with --procedural: every this many updates, replace one maze slot (round robin) by a fresh maze")
+    ap.add_argument("--maze-seed", type=int, default=0, help="seed of the first maze; later mazes take the next seeds")
     a = ap.parse_args()
 
     rank, local_rank, world_size = dist_env()
@@ -60,12 +66,21 @@ def main():
     maps = [load_named_map(n) for n in names]
     gid0, n_local = shard_range(a.worlds * world_size, rank, world_size)
     spawn = [free_space_regions(m) if a.free_spawn else None for m in maps]
+    # every rank generates the same mazes from the same seeds, so the sharded worlds see the same layouts
+    next_maze = a.maze_seed
+    for _ in range(a.procedural):
+        maps.append(generate_maze(next_maze))
+        spawn.append(None)            # a maze brings its own spawn regions
+        next_maze += 1
+    swappable = a.procedural > 0
+    swaps = {"updates": 0, "next": next_maze}
     if len(maps) == 1:
         env = BatchedCopsThievesEnv(maps[0], n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
                                     spawn_override=spawn[0], final_observations=a.time_limit_bootstrap)
     else:
         env = BatchedCopsThievesEnv(maps, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
-                                    spawn_override=spawn, final_observations=a.time_limit_bootstrap)
+                                    spawn_override=spawn, final_observations=a.time_limit_bootstrap,
+                                    swappable_maps=swappable)
     # the reference's schedule (10 000 random / 15 000 before learning / 15 000 frozen policy) counts steps of ONE
     # environment; with thousands of lockstep worlds the same number of TRANSITIONS is reached in a few steps, so the
     # driver scales the durations by the world count unless told otherwise
@@ -84,6 +99,12 @@ def main():
             for st in stats.values():
                 agg["gae_ms"] += st.gae_ms; agg["update_ms"] += st.update_ms; agg["allreduce_ms"] += st.allreduce_ms
             agg["updates"] += 1
+            swaps["updates"] += 1
+            if swappable and a.swap_every > 0 and swaps["updates"] % a.swap_every == 0:
+                seed = swaps["next"]
+                slot = len(names) + (seed - a.maze_seed) % a.procedural
+                learner.note_reset(env.set_map(slot, generate_maze(seed)))
+                swaps["next"] = seed + 1
         env_s0, t0 = learner.env_seconds, time.perf_counter()
         step0 = learner.timestep
         learner.train(learner.timestep + a.timesteps, callback=cb)
