@@ -196,6 +196,13 @@ struct KParams {
   float* final_obs_f32;
   float* final_state_f32;
   float* final_critic_f32;
+  // Episode statistics (cat_env_attach_episode_stats), carried by every launch of the environment while attached and read
+  // by the TX = true instantiations only (kernel_for never picks the record-only one while ep_acc is set).
+  float* ep_acc;                  // [N][A] running returns
+  float* ep_return;               // [N][A] return of the episode a world ended in this step
+  int32_t* ep_length;             // [N]
+  CatEpisodeTotals* ep_totals;    // [n_maps]
+  int ep_map0;                    // the environment's map slot of maps[0] (a host-path chunk's table starts at its first map)
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -1582,6 +1589,50 @@ __device__ __forceinline__ void reset_world(const KParams& k, const MapView& m, 
   __syncwarp();
 }
 
+// Order-preserving u32 key of an fp32 value (CatEpisodeTotals): sign bit clear -> bits | 0x80000000, set -> ~bits.
+// Non-zero for every non-NaN value, and so is its complement, so 0 stays "empty" for both the maximum and the minimum.
+__device__ __forceinline__ uint32_t ep_key(float v) {
+  const uint32_t b = __float_as_uint(v);
+  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+
+// Episode statistics of one stepped world (cat_env_attach_episode_stats), once its rewards are staged: lanes < A add
+// their agent's emitted reward to the running return (acc, loaded by the caller); a world that ends publishes the episode's
+// return and length and adds it to the totals of its map slot, and its running return restarts at zero.
+template <int TA, int TR>
+__device__ __forceinline__ void episode_stats(const KParams& k, const Warp& w, long long world, int mi, float acc, bool done,
+                                              bool captured) {
+  const int A = TA ? TA : k.A, lane = w.lane;
+  CatEpisodeTotals* t = k.ep_totals ? k.ep_totals + k.ep_map0 + mi : nullptr;
+  if (lane < A) {
+    const size_t i = (size_t)world * A + lane;
+    const float ret = acc + w.rew[lane];   // one fp32 add: cumulative_rewards += rewards
+    k.ep_acc[i] = done ? 0.f : ret;
+    if (done) {
+      if (k.ep_return) k.ep_return[i] = ret;
+      if (t) {
+        const double r = (double)ret;
+        atomicAdd(&t->return_sum[lane], r);
+        atomicAdd(&t->return_sq_sum[lane], r * r);   // exact: a float's square fits a double
+        const uint32_t key = ep_key(ret);
+        atomicMax(&t->return_max_key[lane], key);
+        atomicMax(&t->return_min_key[lane], ~key);
+      }
+    }
+  }
+  if (done && lane == 0) {
+    const int32_t len = reinterpret_cast<const int32_t*>(w.rec)[LAY(o_sc)];   // the step_count this step reached
+    if (k.ep_length) k.ep_length[world] = len;
+    if (t) {
+      atomicAdd(reinterpret_cast<unsigned long long*>(&t->episodes), 1ull);
+      atomicAdd(reinterpret_cast<unsigned long long*>(captured ? &t->captures : &t->timeouts), 1ull);
+      atomicAdd(reinterpret_cast<unsigned long long*>(&t->length_sum), (unsigned long long)(uint32_t)len);
+      atomicMax(&t->length_max_key, (uint32_t)len);
+      atomicMax(&t->length_min_key, ~(uint32_t)len);
+    }
+  }
+}
+
 // TA / TR: agents per world and rays per agent as compile-time constants (the 2 cops + 1 thief x 90 rays of every
 // shipped map: <3, 90>), or 0 = read them from the parameters (any other configuration: <0, 0>).  TL: the environment
 // has ray lists (the default) — the instantiation carries no rasteriser code at all.  TX = false: a STEP launch that wants the
@@ -1730,9 +1781,18 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
         else if (i == LAY(o_flags)) v = __uint_as_float(0xFFu);
         grec[i] = v;
       }
+      if (TX && k.ep_acc && lane < A) k.ep_acc[(size_t)world * A + lane] = 0.f;   // no episode is running yet
       continue;
     }
     if (mode == MODE_RESET && k.reset_mask && !k.reset_mask[world]) continue;
+    // Episode statistics: a reset drops the running returns (it never counts an episode); a step loads them here, next
+    // to the record, so that the load's latency hides behind the sensor sweep.
+    const bool ep_on = TX && k.ep_acc != nullptr;
+    float ep_acc = 0.f;
+    if (ep_on && lane < A) {
+      if (mode == MODE_STEP) ep_acc = k.ep_acc[(size_t)world * A + lane];
+      else if (mode == MODE_RESET) k.ep_acc[(size_t)world * A + lane] = 0.f;
+    }
 
     if (prefetched && world == first_world) {
       if (lane < LAY(rec_words)) w.rec[lane] = pf0;
@@ -1814,6 +1874,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
           w.flg[2] = (uint8_t)(done ? (captured ? 0 : 1) : -1);         // winner
         }
         again = done && k.auto_reset;  // SURVEY.md C-10: emit the observation of the re-spawned state instead
+        if (ep_on) episode_stats<TA, TR>(k, w, world, mi, ep_acc, done, captured);
       } else if (mode != MODE_STEP) {
         if (lane < A) w.rew[lane] = 0.f;
         if (lane == 0) { w.flg[0] = 0; w.flg[1] = 0; w.flg[2] = 0xFF; }

@@ -272,13 +272,19 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
     ``swappable_maps=True``: ``set_map(m, map)`` replaces map m of the live environment (a procedural layout, say:
     ``maps.generate_maze``) and resets its worlds, without re-creating the environment, its buffers or a captured
     rollout graph (``CatWorlds.set_map``).
+
+    ``episode_statistics=True``: the step kernel tracks every world's return, as skrl's trainer does, within the same
+    launch.  ``infos[agent]["episode"]`` is ``{"r": (N,) returns of that agent, "l": (N,) lengths}`` of the episodes that
+    ended in the step (gymnasium's ``RecordEpisodeStatistics`` shape, valid where ``terminated``), and
+    ``episode_statistics()`` sums up every episode since the last read, overall or per map.
     """
 
     def __init__(self, map: Union[Map, Sequence[Map]], num_envs: Union[int, Sequence[int]], *, max_step_count: int = 400,
                  time_step: float = 1 / 60.0, device: Union[str, torch.device] = "cuda:0", seed: int = 0, gid0: int = 0,
                  physical_params: Optional[dict] = None, stale_shape_cache: bool = True,
                  spawn_override: Optional[Union[dict, Sequence[Optional[dict]]]] = None, cell: Optional[float] = None,
-                 render_mode=None, final_observations: bool = False, swappable_maps: bool = False):
+                 render_mode=None, final_observations: bool = False, swappable_maps: bool = False,
+                 episode_statistics: bool = False):
         params = _make_params(max_step_count, time_step, physical_params, auto_reset=1, seed=int(seed),
                               stale_shape_cache=int(stale_shape_cache))
         self._params = params
@@ -288,7 +294,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._cmaps = [self._cmap]
             self._setup_common(map, self._cmap, params)
             self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True,
-                                want_final=final_observations, swappable_maps=swappable_maps)
+                                want_final=final_observations, swappable_maps=swappable_maps,
+                                want_episode_stats=episode_statistics)
         else:
             self.maps = list(map)
             n = len(self.maps)
@@ -305,7 +312,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             window = (max(m.window_dimensions[0] for m in self.maps), max(m.window_dimensions[1] for m in self.maps))
             self._setup_common(self.maps[0], self._cmap, params, window=window)
             self._w = CatWorlds(self._cmaps, counts, device=device, gid0=gid0, params=params, want_f32=True,
-                                want_critic=True, want_final=final_observations, swappable_maps=swappable_maps)
+                                want_critic=True, want_final=final_observations, swappable_maps=swappable_maps,
+                                want_episode_stats=episode_statistics)
             num_envs = sum(counts)
         self._cell = cell
         self.map_names = [c.name for c in self._cmaps]
@@ -365,6 +373,9 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             if w.final_obs_f32 is not None:
                 for i, a in enumerate(self.possible_agents):
                     infos[a]["final_observation"] = w.final_obs_f32[i]
+            if w.episode_return is not None:
+                for i, a in enumerate(self.possible_agents):
+                    infos[a]["episode"] = {"r": w.episode_return[:, i], "l": w.episode_length}
             v = (obs, rew, {a: term for a in self.possible_agents}, {a: trunc for a in self.possible_agents}, infos)
             self._cached_views = v
         return v
@@ -403,6 +414,19 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         """``critic()`` of the last step of every episode that ended, (N, 4, R) float32, valid where ``terminated``
         (None without ``final_observations``)."""
         return self._w.final_critic_f32
+
+    def episode_statistics(self, reset: bool = False, by_map: bool = False, group=None) -> Dict:
+        """What the episodes that ended since creation (or the last ``reset=True``) add up to, from the step kernel's
+        per-map totals (one copy to the host): ``episodes``, ``captures``, ``timeouts``, ``capture_rate``, ``length``
+        (mean / min / max) and per agent ``returns`` (mean / population std / min / max); None where no episode ended.
+        ``by_map``: ``{"overall": ..., "maps": [one entry per map slot with "slot" and "map" (its name)]}``.  ``group``:
+        a ``torch.distributed`` group whose ranks' totals are all-reduced first (collective: every rank calls it).
+        ``reset`` zeroes this rank's totals after reading them.  Needs ``episode_statistics=True``."""
+        from . import episodes
+        raw = self._w.episode_totals_raw(reset)
+        if group is not None:
+            raw = episodes.allreduce_totals(raw, group)
+        return episodes.summarize_maps(raw, self.possible_agents, self.map_names, by_map=by_map)
 
     def render(self, world: int = 0):
         """``rgb_array`` of one world, drawn on that world's own map (numpy (W, H, 3) uint8 of that map's window):

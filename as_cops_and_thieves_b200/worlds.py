@@ -14,8 +14,9 @@ from typing import Dict, Mapping, Optional, Sequence, Union
 import numpy as np
 import torch
 
-from . import _lib
-from ._lib import CatEnvInfo, CatMapDesc, CatParams, CatRecordLayout, CatStateView, CatStepIO, CAT_WALL_SLOTS
+from . import _lib, episodes
+from ._lib import (CatEnvInfo, CatEpisodeStatsIO, CatMapDesc, CatParams, CatRecordLayout, CatStateView, CatStepIO,
+                   CAT_WALL_SLOTS)
 from .maps import CompiledMap
 from .params import EnvParams
 
@@ -108,7 +109,8 @@ class CatWorlds:
                  gid0: int = 0, params: Optional[EnvParams] = None, want_f32: bool = True,
                  want_shared: bool = True, want_hits: bool = False, pinned_outputs: bool = False,
                  want_critic: bool = False, want_bf16: bool = False, want_final: bool = False,
-                 swappable_maps: bool = False, map_blob_capacity: Optional[int] = None, **overrides):
+                 swappable_maps: bool = False, map_blob_capacity: Optional[int] = None,
+                 want_episode_stats: bool = False, **overrides):
         """``pinned_outputs=True`` places every output tensor in mapped pinned HOST memory: the kernel stores its
         results there directly and the host reads them (``tensor.numpy()``) after one stream synchronisation —
         the layout for callers that consume every step on the CPU, like the single-world PettingZoo face.
@@ -135,7 +137,13 @@ class CatWorlds:
         of its maps later without invalidating its buffers or a captured CUDA graph.  Each map's blob is then allocated
         at ``map_blob_capacity`` bytes (a positive multiple of 16; default: the largest blob of the creation maps and the
         shipped maps, ``default_blob_capacity``), and the mixed-map kernels run even for one map.  Needs ray lists
-        (``ray_list_cell >= 0``)."""
+        (``ray_list_cell >= 0``).
+
+        ``want_episode_stats``: the step kernel keeps each world's running return ``episode_acc`` (N, A) and, for every
+        world that ends in a step, writes that episode's return ``episode_return`` (N, A) float32 and length
+        ``episode_length`` (N,) int32 (valid where ``terminated``) and adds it to its map slot's totals, read with
+        ``episode_totals`` (``cat_env_attach_episode_stats``; resets zero the running returns and never count an
+        episode).  A step stays one launch; it runs the full-output kernel."""
         if map_blob_capacity is not None and (int(map_blob_capacity) < 16 or int(map_blob_capacity) % 16):
             # the step kernel stages a blob with one bulk copy whose size must be a multiple of 16 bytes
             raise ValueError(f"map_blob_capacity must be a positive multiple of 16, got {map_blob_capacity}")
@@ -243,6 +251,17 @@ class CatWorlds:
         self._host = None
         self._io = self._make_io()
         self._ptr_table = (C.c_void_p * 8)()
+        self.want_episode_stats = bool(want_episode_stats)
+        self.episode_acc = self.episode_return = self.episode_length = self._episode_totals = None
+        if want_episode_stats:
+            # always device memory: the kernel updates the totals with atomics
+            self.episode_acc = torch.zeros((N, A), dtype=torch.float32, device=dev)
+            self.episode_return = torch.zeros((N, A), dtype=torch.float32, device=dev)
+            self.episode_length = torch.zeros(N, dtype=torch.int32, device=dev)
+            self._episode_totals = torch.zeros(len(cmaps) * episodes.TOTALS_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+            sio = CatEpisodeStatsIO(self.episode_acc.data_ptr(), self.episode_return.data_ptr(),
+                                    self.episode_length.data_ptr(), self._episode_totals.data_ptr())
+            _lib.check(self.L.cat_env_attach_episode_stats(self._h, C.byref(sio)), "cat_env_attach_episode_stats")
         _lib.check(self.L.cat_env_init_state(self._h, self.state.data_ptr(), self._stream()), "cat_env_init_state")
 
     # ------------------------------------------------------------------ plumbing
@@ -608,10 +627,33 @@ class CatWorlds:
                    "cat_env_set_state")
         torch.cuda.current_stream(self.device).synchronize()  # `keep` tensors must outlive the copy
 
+    def episode_totals_raw(self, reset: bool = False) -> np.ndarray:
+        """The per-map-slot ``CatEpisodeTotals`` as a numpy structured array (``episodes.TOTALS_DTYPE``), one copy to the
+        host (which waits for the launches enqueued so far).  ``reset`` zeroes them on the device afterwards."""
+        if self._episode_totals is None:
+            raise _lib.CatError("episode statistics are off (want_episode_stats=False)")
+        raw = np.frombuffer(self._episode_totals.cpu().numpy().tobytes(), dtype=episodes.TOTALS_DTYPE)
+        if reset:
+            self._episode_totals.zero_()
+        return raw.copy()
+
+    def episode_totals(self, reset: bool = False, agents: Optional[Sequence[str]] = None) -> list:
+        """Every map slot's totals decoded (``episodes.summarize``: episodes, captures, timeouts, length and per-agent
+        return moments); ``agents`` names the agents in index order (default ``0 .. A-1``)."""
+        raw = self.episode_totals_raw(reset)
+        agents = list(agents) if agents is not None else [str(i) for i in range(self.A)]
+        return [episodes.summarize(raw[m], agents) for m in range(len(raw))]
+
     def state_dict(self) -> Dict[str, torch.Tensor]:
-        """Checkpoint = the packed state buffer (everything else is recomputed by ``observe``)."""
-        return {"state": self.state.clone(), "seed": torch.tensor(self.params["seed"])}
+        """Checkpoint = the packed state buffer (everything else is recomputed by ``observe``), and the running returns
+        when episode statistics are on."""
+        sd = {"state": self.state.clone(), "seed": torch.tensor(self.params["seed"])}
+        if self.episode_acc is not None:
+            sd["episode_acc"] = self.episode_acc.clone()
+        return sd
 
     def load_state_dict(self, sd: Mapping[str, torch.Tensor]) -> None:
         self.state.copy_(sd["state"].to(self.device))
         self.set_seed(int(sd["seed"]))
+        if self.episode_acc is not None and "episode_acc" in sd:
+            self.episode_acc.copy_(sd["episode_acc"].to(self.device))

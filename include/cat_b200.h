@@ -160,6 +160,47 @@ typedef struct {
   float* final_critic_f32;
 } CatStepIO;
 
+/* EPISODE STATISTICS (cat_env_attach_episode_stats): the step kernel keeps each world's running return and reports
+ * every episode that ends, per world and summed per map, at the cost of a few stores and atomics of the worlds that end.
+ *
+ * Semantics.  While statistics are attached, every step launch adds each agent's emitted fp32 reward to the world's
+ * running return, acc = acc + reward (one fp32 add: bit for bit a cumulative_rewards += rewards on the same rewards).
+ * A world ENDS in a step when it reports terminated (captured or timed out); for such a world the kernel writes the
+ * episode's return per agent and its length (the step_count the step reached: steps since the world's last reset) to
+ * episode_return / episode_length, adds the episode to the totals of its map, and zeroes acc.  The per-world entries
+ * of other worlds are left untouched: valid where terminated, as the final outputs.  A reset never counts an episode:
+ * cat_env_reset zeroes acc of the worlds it resets, cat_env_init_state zeroes every acc; cat_env_set_state does not
+ * touch acc (a length follows whatever step_count it sets).  auto_reset = 0 follows the same rules.  cat_env_observe
+ * ignores the statistics.
+ *
+ * Totals are indexed by the world's map slot (0 for a single-map environment, the slot of cat_env_create_multi /
+ * _swappable otherwise); a zero-filled CatEpisodeTotals is the empty state.  Every field is updated by atomicAdd or
+ * atomicMax only.  Minima and maxima are u32 keys under atomicMax: the maximum is stored as an order-preserving key of
+ * the value, the minimum as the key's complement, so 0 = "no episode yet".  For lengths the key is the length itself;
+ * for an fp32 return r with bits b, key = b | 0x80000000 if its sign bit is clear and ~b if it is set, which is
+ * non-zero for every non-NaN value.  Counts, length sums and the minima and maxima are exact; the f64 sums depend on
+ * the order in which the atomics land, so they may differ between runs in the last bits. */
+typedef struct {
+  uint64_t episodes;                            /* episodes that ended */
+  uint64_t captures;                            /* ... by capture (cop win) */
+  uint64_t timeouts;                            /* ... by timeout (thief win) */
+  uint64_t length_sum;
+  uint32_t length_min_key;                      /* ~min(length) */
+  uint32_t length_max_key;                      /* max(length) */
+  double return_sum[CAT_MAX_AGENTS];            /* per agent, sum of episode returns */
+  double return_sq_sum[CAT_MAX_AGENTS];         /* per agent, sum of squared episode returns */
+  uint32_t return_min_key[CAT_MAX_AGENTS];      /* ~key(min return) */
+  uint32_t return_max_key[CAT_MAX_AGENTS];      /* key(max return) */
+} CatEpisodeTotals;
+
+/* caller-owned device pointers (N worlds, A agents) */
+typedef struct {
+  float* acc;                  /* f32 [N][A] running returns; required, zeroed by the caller before it is attached */
+  float* episode_return;       /* f32 [N][A] return of the episode a world ended in its last step; optional */
+  int32_t* episode_length;     /* i32 [N] its length; optional */
+  CatEpisodeTotals* totals;    /* [n_maps] per map slot; optional */
+} CatEpisodeStatsIO;
+
 /* byte offsets inside one world's output record (cat_env_record_layout / cat_env_packed_record_layout) */
 typedef struct {
   int32_t bytes;        /* record size = default world stride (multiple of 16) */
@@ -289,6 +330,12 @@ int cat_env_step_host(CatEnv* env, void* state_dev, const uint8_t* host_actions,
 /* Entity.get_observation + get_shared_observations of the current state (entity.py:159-220,
  * observation_spaces.py:67-131) without stepping */
 int cat_env_observe(CatEnv* env, void* state_dev, const CatStepIO* io, void* stream);
+/* Attach episode statistics (CatEpisodeStatsIO above) to an environment, or detach them with io = NULL.  Host only, no
+ * CUDA call: the pointers are stored, and every later launch of the environment (step, reset, init and the chunks of
+ * cat_env_step_host) carries them; such launches run the full-output kernel.  CAT_ERR_INVALID for a null env, outputs
+ * without acc, or a misaligned pointer (4 bytes for the arrays, 8 for totals); nothing is stored then.  A CUDA graph
+ * captured before this call keeps the parameters its launches were captured with. */
+int cat_env_attach_episode_stats(CatEnv* env, const CatEpisodeStatsIO* io);
 /* parity-test access to the hidden state */
 int cat_env_get_state(CatEnv* env, const void* state_dev, const CatStateView* view, void* stream);
 int cat_env_set_state(CatEnv* env, void* state_dev, const CatStateView* view, void* stream);

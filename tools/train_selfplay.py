@@ -6,10 +6,12 @@ all-reduced over NCCL per minibatch.
     python tools/train_selfplay.py --map agh-map --worlds 4096 --iterations 2 --timesteps 256
     python tools/train_selfplay.py --map squarinth,agh-map,labyrinth --worlds 4096   # one policy over three maps
     python tools/train_selfplay.py --map squarinth --procedural 2 --swap-every 4     # + 2 slots of fresh mazes
+    python tools/train_selfplay.py --map squarinth,agh-map --episode-stats            # + episode returns / lengths
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_selfplay.py ...
 
 Prints one JSON line per self-play iteration (rank 0): environment agent-steps/s inside training, GAE / update /
-all-reduce milliseconds per update, win rates.
+all-reduce milliseconds per update, win rates; with --episode-stats also "episodes": what the training episodes of the
+iteration added up to (all ranks), overall and per map slot (the evaluation's episodes are not counted).
 """
 import argparse
 import json
@@ -17,11 +19,12 @@ import sys
 import time
 from pathlib import Path
 
+import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
-from as_cops_and_thieves_b200 import selfplay  # noqa: E402
+from as_cops_and_thieves_b200 import episodes, selfplay  # noqa: E402
 from as_cops_and_thieves_b200.env import BatchedCopsThievesEnv  # noqa: E402
 from as_cops_and_thieves_b200.mappo import MAPPOConfig, MAPPOLearner  # noqa: E402
 from as_cops_and_thieves_b200.maps import free_space_regions, generate_maze, load_named_map  # noqa: E402
@@ -52,6 +55,8 @@ def main():
     ap.add_argument("--swap-every", type=int, default=0,
                     help="with --procedural: every this many updates, replace one maze slot (round robin) by a fresh maze")
     ap.add_argument("--maze-seed", type=int, default=0, help="seed of the first maze; later mazes take the next seeds")
+    ap.add_argument("--episode-stats", action="store_true",
+                    help="report the returns, lengths and capture rate of the training episodes, overall and per map")
     a = ap.parse_args()
 
     rank, local_rank, world_size = dist_env()
@@ -76,11 +81,12 @@ def main():
     swaps = {"updates": 0, "next": next_maze}
     if len(maps) == 1:
         env = BatchedCopsThievesEnv(maps[0], n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
-                                    spawn_override=spawn[0], final_observations=a.time_limit_bootstrap)
+                                    spawn_override=spawn[0], final_observations=a.time_limit_bootstrap,
+                                    episode_statistics=a.episode_stats)
     else:
         env = BatchedCopsThievesEnv(maps, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
                                     spawn_override=spawn, final_observations=a.time_limit_bootstrap,
-                                    swappable_maps=swappable)
+                                    swappable_maps=swappable, episode_statistics=a.episode_stats)
     # the reference's schedule (10 000 random / 15 000 before learning / 15 000 frozen policy) counts steps of ONE
     # environment; with thousands of lockstep worlds the same number of TRANSITIONS is reached in a few steps, so the
     # driver scales the durations by the world count unless told otherwise
@@ -92,6 +98,28 @@ def main():
                       opponent_freeze_duration=-(-15000 // scale) if a.schedule != "off" else 0)
     learner = MAPPOLearner(env, cfg, seed=0)
     archive = Path(a.archive) if rank == 0 else Path(a.archive + f".rank{rank}")
+    # training episodes of the current iteration: (slot, map name) -> totals, read (and cleared) from the environment
+    # before a slot is swapped and after training; the evaluation's episodes are cleared unread
+    ep_parts = {}
+
+    def take_episodes():
+        raw = env.worlds.episode_totals_raw(reset=True)
+        for m in range(len(raw)):
+            key = (m, env.map_names[m])
+            ep_parts[key] = episodes.merge_totals(np.stack([ep_parts[key], raw[m]]) if key in ep_parts else raw[m:m + 1])
+
+    def episode_report():
+        keys = list(ep_parts)        # the same keys in the same order on every rank: every rank swaps the same slots
+        tot = np.stack([ep_parts[k] for k in keys]) if keys else episodes.empty_totals(0)
+        if world_size > 1:
+            import torch.distributed as dist
+            tot = episodes.allreduce_totals(tot, dist.group.WORLD)
+        ep_parts.clear()
+        out = episodes.summarize_maps(tot, learner.agents, [name for _, name in keys], by_map=True)
+        for entry, (slot, _) in zip(out["maps"], keys):
+            entry["slot"] = slot
+        return out
+
     for it in range(a.iterations):
         agg = {"gae_ms": 0.0, "update_ms": 0.0, "allreduce_ms": 0.0, "updates": 0}
 
@@ -103,12 +131,16 @@ def main():
             if swappable and a.swap_every > 0 and swaps["updates"] % a.swap_every == 0:
                 seed = swaps["next"]
                 slot = len(names) + (seed - a.maze_seed) % a.procedural
+                if a.episode_stats:
+                    take_episodes()
                 learner.note_reset(env.set_map(slot, generate_maze(seed)))
                 swaps["next"] = seed + 1
         env_s0, t0 = learner.env_seconds, time.perf_counter()
         step0 = learner.timestep
         learner.train(learner.timestep + a.timesteps, callback=cb)
         train_s = time.perf_counter() - t0
+        if a.episode_stats:
+            take_episodes()
         tc = selfplay.TrainingConfig
         res_c = selfplay.evaluate_agent(env, learner, tc.cop_role_prefix, tc.thief_role_prefix, archive / "thief", tc)
         res_t = selfplay.evaluate_agent(env, learner, tc.thief_role_prefix, tc.cop_role_prefix, archive / "cop", tc)
@@ -118,6 +150,10 @@ def main():
         selfplay.add_policy_to_archive(str(ck), archive / "cop", it, "cop")
         selfplay.add_policy_to_archive(str(ck), archive / "thief", it, "thief")
         steps = learner.timestep - step0
+        extra = {}
+        if a.episode_stats:
+            env.worlds.episode_totals_raw(reset=True)        # the evaluation's episodes
+            extra["episodes"] = episode_report()
         if rank == 0:
             u = max(agg["updates"], 1)
             print(json.dumps({
@@ -127,7 +163,7 @@ def main():
                 "train_agent_steps_per_s": a.worlds * world_size * len(learner.agents) * steps / train_s,
                 "gae_ms_per_update": agg["gae_ms"] / u, "ppo_ms_per_update": agg["update_ms"] / u,
                 "allreduce_ms_per_update": agg["allreduce_ms"] / u,
-                "eval_vs_archive": {"cop_trained": res_c, "thief_trained": res_t}}), flush=True)
+                "eval_vs_archive": {"cop_trained": res_c, "thief_trained": res_t}, **extra}), flush=True)
     env.close()
     if world_size > 1:
         import torch.distributed as dist
