@@ -80,6 +80,19 @@ class CatEpisodeStatsIO(C.Structure):
     _fields_ = [("acc", C.c_void_p), ("episode_return", C.c_void_p), ("episode_length", C.c_void_p), ("totals", C.c_void_p)]
 
 
+class CatWorldParams(C.Structure):
+    _fields_ = [("unit_velocity", C.c_float * 2), ("max_speed", C.c_float * 2), ("termination_radius", C.c_float),
+                ("max_step_count", C.c_int32)]
+
+
+class CatWorldParamRanges(C.Structure):
+    _fields_ = [("lo", CatWorldParams), ("hi", CatWorldParams), ("draw", C.c_int32)]
+
+
+class CatWorldParamsIO(C.Structure):
+    _fields_ = [("params", C.c_void_p), ("ranges", C.c_void_p)]
+
+
 class CatRecordLayout(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("bytes", "off_dist", "off_type", "off_reward", "off_terminated",
                                          "off_truncated", "off_winner", "type_bits")]
@@ -113,7 +126,7 @@ EXPORTS = (
     "cat_env_map_info", "cat_env_create_swappable", "cat_env_set_map", "cat_map_blob_bytes", "cat_ray_lists_device",
     "cat_env_record_layout", "cat_env_packed_record_layout", "cat_env_overflow_counts", "cat_ray_lists_host",
     "cat_env_set_seed", "cat_env_state_bytes", "cat_env_init_state", "cat_env_reset", "cat_env_step", "cat_env_step_host", "cat_env_observe",
-    "cat_env_get_state", "cat_env_set_state", "cat_env_attach_episode_stats", "cat_gae", "cat_adv_normalize",
+    "cat_env_get_state", "cat_env_set_state", "cat_env_attach_episode_stats", "cat_env_attach_world_params", "cat_gae", "cat_adv_normalize",
     "cat_renderer_create", "cat_renderer_destroy", "cat_renderer_frame_size", "cat_render", "cat_ray_directions",
 )
 
@@ -167,6 +180,7 @@ def load():
     for fn in (L.cat_env_get_state, L.cat_env_set_state):
         fn.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(CatStateView), C.c_void_p]
     L.cat_env_attach_episode_stats.argtypes = [C.c_void_p, C.POINTER(CatEpisodeStatsIO)]
+    L.cat_env_attach_world_params.argtypes = [C.c_void_p, C.POINTER(CatWorldParamsIO)]
     L.cat_gae.argtypes = [C.c_void_p] * 7 + [C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_void_p]
     L.cat_adv_normalize.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
     L.cat_renderer_create.argtypes = [C.POINTER(CatMapDesc), C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int32,

@@ -195,11 +195,11 @@ static bool pick_launch_shape(CatEnv* env, int n_worlds, LaunchShape* out) {
 static int fill_map_table(const CatEnv* env, KParams& k, int w0, int w1, int grid, int wpc) {
   int len[CAT_MAX_MAPS], ctas[CAT_MAX_MAPS];
   int n = 0;
-  k.ep_map0 = -1;
+  k.map_slot0 = -1;
   for (const EnvMap& m : env->maps) {
     const int b = std::max(w0, m.world_begin), e = std::min(w1, m.world_begin + m.n_worlds);
     if (b >= e) continue;
-    if (k.ep_map0 < 0) k.ep_map0 = (int)(&m - env->maps.data());   // the maps of [w0, w1) are consecutive slots
+    if (k.map_slot0 < 0) k.map_slot0 = (int)(&m - env->maps.data());   // the maps of [w0, w1) are consecutive slots
     MapSlice& sl = k.maps[n];
     sl.blob = m.blob_dev; sl.blob_bytes = m.blob_bytes; sl.world_begin = b; sl.world_end = e;
     len[n++] = e - b;
@@ -947,7 +947,7 @@ static int prepare(CatEnv* env, void* state_dev, const CatStepIO* io, int mode, 
 static WorldKernel kernel_for(const CatEnv* env, const KParams& k) {
   const bool record_only = k.mode == MODE_STEP && k.record && !k.shared_dist && !k.shared_type && !k.team_pos && !k.obs_f32 && !k.state_f32 &&
                            !k.hit_point && !k.critic_f32 && !k.obs_bf16 && !k.critic_bf16 &&
-                           !k.final_record && !k.final_obs_f32 && !k.final_state_f32 && !k.final_critic_f32 && !k.ep_acc;
+                           !k.final_record && !k.final_obs_f32 && !k.final_state_f32 && !k.final_critic_f32 && !k.ep_acc && !k.wp;
   return record_only ? env->kernel_record : env->kernel;
 }
 
@@ -964,6 +964,20 @@ int cat_env_attach_episode_stats(CatEnv* env, const CatEpisodeStatsIO* io) {
     return fail(CAT_ERR_INVALID, "episode statistics: acc / episode_return / episode_length must be 4-byte aligned, totals 8-byte aligned");
   env->kp.ep_acc = io->acc; env->kp.ep_return = io->episode_return; env->kp.ep_length = io->episode_length;
   env->kp.ep_totals = io->totals;
+  return CAT_OK;
+}
+
+// Like the statistics, the table lives in env->kp.
+int cat_env_attach_world_params(CatEnv* env, const CatWorldParamsIO* io) {
+  if (!env) return fail(CAT_ERR_INVALID, "null env");
+  if (!io) {
+    env->kp.wp = nullptr; env->kp.wp_ranges = nullptr;
+    return CAT_OK;
+  }
+  if (!io->params) return fail(CAT_ERR_INVALID, "world parameters need params");
+  if ((reinterpret_cast<uintptr_t>(io->params) | reinterpret_cast<uintptr_t>(io->ranges)) & 3)
+    return fail(CAT_ERR_INVALID, "world parameters: params / ranges must be 4-byte aligned");
+  env->kp.wp = io->params; env->kp.wp_ranges = io->ranges;
   return CAT_OK;
 }
 

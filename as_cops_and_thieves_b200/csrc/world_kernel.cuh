@@ -202,7 +202,11 @@ struct KParams {
   float* ep_return;               // [N][A] return of the episode a world ended in this step
   int32_t* ep_length;             // [N]
   CatEpisodeTotals* ep_totals;    // [n_maps]
-  int ep_map0;                    // the environment's map slot of maps[0] (a host-path chunk's table starts at its first map)
+  int map_slot0;                  // the environment's map slot of maps[0] (a host-path chunk's table starts at its first map)
+  // Per-world parameters (cat_env_attach_world_params), carried like the statistics and read by the TX = true
+  // instantiations only (kernel_for never picks the record-only one while wp is set).
+  CatWorldParams* wp;                      // [N]
+  const CatWorldParamRanges* wp_ranges;    // [n_maps], by map slot like ep_totals; nullptr = never draw
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -1589,6 +1593,27 @@ __device__ __forceinline__ void reset_world(const KParams& k, const MapView& m, 
   __syncwarp();
 }
 
+// A re-spawned world's fresh parameters (cat_env_attach_world_params), when its map slot draws: one lane makes the two
+// Philox calls of cat_param_draws, keyed by the new episode number reset_world has just stored, and writes the entry.
+// The entry is next read by the world's next step.
+__device__ __forceinline__ void draw_world_params(const KParams& k, const Warp& w, long long world, int mi) {
+  if (w.lane != 0) return;
+  const CatWorldParamRanges* r = k.wp_ranges + k.map_slot0 + mi;
+  if (!r->draw) return;
+  const uint32_t episode = reinterpret_cast<const uint32_t*>(w.rec)[k.lay.o_ep];
+  uint32_t u[6];
+  cat_param_draws(k.seed, (unsigned long long)(k.gid0 + world), episode, u);
+  CatWorldParams p;
+#pragma unroll
+  for (int t = 0; t < 2; ++t) {
+    p.unit_velocity[t] = cat_param_float(u[t], r->lo.unit_velocity[t], r->hi.unit_velocity[t]);
+    p.max_speed[t] = cat_param_float(u[2 + t], r->lo.max_speed[t], r->hi.max_speed[t]);
+  }
+  p.termination_radius = cat_param_float(u[4], r->lo.termination_radius, r->hi.termination_radius);
+  p.max_step_count = cat_param_int(u[5], r->lo.max_step_count, r->hi.max_step_count);
+  k.wp[world] = p;
+}
+
 // Order-preserving u32 key of an fp32 value (CatEpisodeTotals): sign bit clear -> bits | 0x80000000, set -> ~bits.
 // Non-zero for every non-NaN value, and so is its complement, so 0 stays "empty" for both the maximum and the minimum.
 __device__ __forceinline__ uint32_t ep_key(float v) {
@@ -1603,7 +1628,7 @@ template <int TA, int TR>
 __device__ __forceinline__ void episode_stats(const KParams& k, const Warp& w, long long world, int mi, float acc, bool done,
                                               bool captured) {
   const int A = TA ? TA : k.A, lane = w.lane;
-  CatEpisodeTotals* t = k.ep_totals ? k.ep_totals + k.ep_map0 + mi : nullptr;
+  CatEpisodeTotals* t = k.ep_totals ? k.ep_totals + k.map_slot0 + mi : nullptr;
   if (lane < A) {
     const size_t i = (size_t)world * A + lane;
     const float ret = acc + w.rew[lane];   // one fp32 add: cumulative_rewards += rewards
@@ -1793,6 +1818,20 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
       if (mode == MODE_STEP) ep_acc = k.ep_acc[(size_t)world * A + lane];
       else if (mode == MODE_RESET) k.ep_acc[(size_t)world * A + lane] = 0.f;
     }
+    // Per-world parameters of a step, loaded here for the same reason: lanes < A take their team's thrust and top
+    // speed, every lane the capture radius and time limit (one broadcast load each).  The record-only instantiation
+    // reads the parameters where it always has (WORLD_PARAM): hoisted to here, they changed its SASS and stack frame.
+    float impulse = 0.f, max_speed = 0.f, term_r = 0.f;
+    int max_steps = 0;
+#define WORLD_PARAM(local, field) (TX ? local : k.field)
+    if (TX) { impulse = k.impulse; max_speed = k.max_speed; term_r = k.term_r; max_steps = k.max_steps; }
+    if (TX && k.wp && mode == MODE_STEP) {
+      const CatWorldParams* e = k.wp + world;
+      const int team = lane < k.nc ? 0 : 1;
+      if (lane < A) { impulse = e->unit_velocity[team]; max_speed = e->max_speed[team]; }
+      term_r = e->termination_radius;
+      max_steps = e->max_step_count;
+    }
 
     if (prefetched && world == first_world) {
       if (lane < LAY(rec_words)) w.rec[lane] = pf0;
@@ -1821,12 +1860,12 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
         for (int c = 0; c < k.nc && !captured; ++c) {
           const float tx = pos[2 * t], ty = pos[2 * t + 1], cx = pos[2 * c], cy = pos[2 * c + 1];
           const float dx = tx - cx, dy = ty - cy;
-          if (dx * dx + dy * dy < k.term_r * k.term_r) {
+          if (dx * dx + dy * dy < WORLD_PARAM(term_r, term_r) * WORLD_PARAM(term_r, term_r)) {
             const bool blocked = los_blocked(smem, lane, tx, ty, cx, cy, k.wall_r);
             if (!__any_sync(0xFFFFFFFFu, blocked)) captured = true;
           }
         }
-      timeout = !captured && step_count >= k.max_steps;
+      timeout = !captured && step_count >= WORLD_PARAM(max_steps, max_steps);
       // Entity._perform_action (entity.py:126-134)
       if (lane < A) {
         int act;
@@ -1836,11 +1875,13 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
         else if (k.actions_kind == 2) act = (int)reinterpret_cast<const long long*>(k.actions[0])[ai];
         else act = (int)reinterpret_cast<const long long*>(k.actions[lane])[world];
         float fx = 0.f, fy = 0.f;
-        if (act == 0) fx = -k.impulse; else if (act == 1) fy = k.impulse;
-        else if (act == 2) fx = k.impulse; else if (act == 3) fy = -k.impulse;
+        if (act == 0) fx = -WORLD_PARAM(impulse, impulse); else if (act == 1) fy = WORLD_PARAM(impulse, impulse);
+        else if (act == 2) fx = WORLD_PARAM(impulse, impulse); else if (act == 3) fy = -WORLD_PARAM(impulse, impulse);
         float vx = vel[2 * lane] + fx * k.inv_mass, vy = vel[2 * lane + 1] + fy * k.inv_mass;
         const float sp = sqrtf(vx * vx + vy * vy);
-        if (sp > k.max_speed) { vx = vx / sp * k.max_speed; vy = vy / sp * k.max_speed; }
+        if (sp > WORLD_PARAM(max_speed, max_speed)) {
+          vx = vx / sp * WORLD_PARAM(max_speed, max_speed); vy = vy / sp * WORLD_PARAM(max_speed, max_speed);
+        }
         vel[2 * lane] = vx; vel[2 * lane + 1] = vy;
       }
       __syncwarp();
@@ -1852,7 +1893,11 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
     //   OBSERVE : observe -> write
 #pragma unroll 1
     for (;;) {
-      if (do_reset) { reset_world(k, m, w, world); do_reset = false; staged = false; }
+      if (do_reset) {
+        reset_world(k, m, w, world);
+        if (TX && k.wp_ranges) draw_world_params(k, w, world, mi);
+        do_reset = false; staged = false;
+      }
       // entity.py:143 — observation of the pre-physics state (SURVEY.md C-1).  A world that ends on this step and
       // is re-spawned in it emits the NEW episode's observation (C-10) and a terminal reward that does not depend
       // on what is seen, so its terminal sensor sweep would be thrown away unless the launch asks for final outputs:
@@ -1903,4 +1948,5 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
 #undef CTA_CNT
 #undef W_BEGIN
 #undef W_END
+#undef WORLD_PARAM
 

@@ -277,6 +277,13 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
     launch.  ``infos[agent]["episode"]`` is ``{"r": (N,) returns of that agent, "l": (N,) lengths}`` of the episodes that
     ended in the step (gymnasium's ``RecordEpisodeStatistics`` shape, valid where ``terminated``), and
     ``episode_statistics()`` sums up every episode since the last read, overall or per map.
+
+    ``randomize``: domain randomisation of the dynamics, a spec for every map or a sequence of one spec (or None) per
+    map, e.g. ``{"max_speed": {"thief": (125, 175)}, "termination_radius": (15, 25), "max_step_count": (300, 500)}``
+    (a bare ``(lo, hi)`` applies to both teams; fields not named stay at the environment's values).  Every re-spawn
+    draws a world's thrust and top speed per team, capture radius and time limit for its next episode, inside the step
+    kernel.  ``world_params()``, ``set_world_params(...)`` and ``set_randomization(...)`` read and change them between
+    steps (a curriculum); observation and state spaces do not change.
     """
 
     def __init__(self, map: Union[Map, Sequence[Map]], num_envs: Union[int, Sequence[int]], *, max_step_count: int = 400,
@@ -284,7 +291,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
                  physical_params: Optional[dict] = None, stale_shape_cache: bool = True,
                  spawn_override: Optional[Union[dict, Sequence[Optional[dict]]]] = None, cell: Optional[float] = None,
                  render_mode=None, final_observations: bool = False, swappable_maps: bool = False,
-                 episode_statistics: bool = False):
+                 episode_statistics: bool = False,
+                 randomize: Union[None, Mapping, Sequence[Optional[Mapping]]] = None):
         params = _make_params(max_step_count, time_step, physical_params, auto_reset=1, seed=int(seed),
                               stale_shape_cache=int(stale_shape_cache))
         self._params = params
@@ -295,7 +303,7 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._setup_common(map, self._cmap, params)
             self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True,
                                 want_final=final_observations, swappable_maps=swappable_maps,
-                                want_episode_stats=episode_statistics)
+                                want_episode_stats=episode_statistics, param_ranges=randomize)
         else:
             self.maps = list(map)
             n = len(self.maps)
@@ -313,7 +321,7 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._setup_common(self.maps[0], self._cmap, params, window=window)
             self._w = CatWorlds(self._cmaps, counts, device=device, gid0=gid0, params=params, want_f32=True,
                                 want_critic=True, want_final=final_observations, swappable_maps=swappable_maps,
-                                want_episode_stats=episode_statistics)
+                                want_episode_stats=episode_statistics, param_ranges=randomize)
             num_envs = sum(counts)
         self._cell = cell
         self.map_names = [c.name for c in self._cmaps]
@@ -427,6 +435,21 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         if group is not None:
             raw = episodes.allreduce_totals(raw, group)
         return episodes.summarize_maps(raw, self.possible_agents, self.map_names, by_map=by_map)
+
+    def world_params(self) -> Dict[str, torch.Tensor]:
+        """Every world's current dynamics, named device views (``CatWorlds.world_params``).  Needs ``randomize``."""
+        return self._w.world_params()
+
+    def set_world_params(self, mask: Optional[torch.Tensor] = None, **values) -> None:
+        """Write worlds' dynamics directly (``CatWorlds.set_world_params``), e.g. ``termination_radius=15.0``."""
+        self._w.set_world_params(mask, **values)
+
+    def set_randomization(self, randomize: Union[None, Mapping, Sequence[Optional[Mapping]]]) -> None:
+        """Replace the randomisation spec (one for every map, or one per map; ``None`` stops drawing, leaving the current
+        values in place).  It applies from each world's next re-spawn.  Needs ``randomize`` at creation."""
+        from . import world_params as wparams
+        for slot, spec in enumerate(wparams.per_slot(randomize, len(self._cmaps))):
+            self._w.set_param_ranges(slot, draw=spec is not None, **(spec or {}))
 
     def render(self, world: int = 0):
         """``rgb_array`` of one world, drawn on that world's own map (numpy (W, H, 3) uint8 of that map's window):

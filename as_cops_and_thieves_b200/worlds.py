@@ -9,13 +9,13 @@ from __future__ import annotations
 
 import ctypes as C
 import functools
-from typing import Dict, Mapping, Optional, Sequence, Union
+from typing import Dict, Mapping, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
 
-from . import _lib, episodes
-from ._lib import (CatEnvInfo, CatEpisodeStatsIO, CatMapDesc, CatParams, CatRecordLayout, CatStateView, CatStepIO,
+from . import _lib, episodes, world_params as wparams
+from ._lib import (CatEnvInfo, CatEpisodeStatsIO, CatWorldParamsIO, CatMapDesc, CatParams, CatRecordLayout, CatStateView, CatStepIO,
                    CAT_WALL_SLOTS)
 from .maps import CompiledMap
 from .params import EnvParams
@@ -110,7 +110,8 @@ class CatWorlds:
                  want_shared: bool = True, want_hits: bool = False, pinned_outputs: bool = False,
                  want_critic: bool = False, want_bf16: bool = False, want_final: bool = False,
                  swappable_maps: bool = False, map_blob_capacity: Optional[int] = None,
-                 want_episode_stats: bool = False, **overrides):
+                 want_episode_stats: bool = False, want_world_params: bool = False,
+                 param_ranges: Union[None, Mapping, Sequence[Optional[Mapping]]] = None, **overrides):
         """``pinned_outputs=True`` places every output tensor in mapped pinned HOST memory: the kernel stores its
         results there directly and the host reads them (``tensor.numpy()``) after one stream synchronisation —
         the layout for callers that consume every step on the CPU, like the single-world PettingZoo face.
@@ -143,7 +144,13 @@ class CatWorlds:
         world that ends in a step, writes that episode's return ``episode_return`` (N, A) float32 and length
         ``episode_length`` (N,) int32 (valid where ``terminated``) and adds it to its map slot's totals, read with
         ``episode_totals`` (``cat_env_attach_episode_stats``; resets zero the running returns and never count an
-        episode).  A step stays one launch; it runs the full-output kernel."""
+        episode).  A step stays one launch; it runs the full-output kernel.
+
+        ``want_world_params``: every world reads its thrust and top speed per team, its capture radius and its time limit
+        from a device table (``cat_env_attach_world_params``), filled with this environment's values for both teams;
+        ``world_params()`` gives named views of it and ``set_world_params`` writes it.  ``param_ranges`` (implies
+        ``want_world_params``): a randomisation spec for every map slot, or one per slot (``set_param_ranges``), from
+        which every re-spawn of a world draws its next entry.  A step stays one launch; it runs the full-output kernel."""
         if map_blob_capacity is not None and (int(map_blob_capacity) < 16 or int(map_blob_capacity) % 16):
             # the step kernel stages a blob with one bulk copy whose size must be a multiple of 16 bytes
             raise ValueError(f"map_blob_capacity must be a positive multiple of 16, got {map_blob_capacity}")
@@ -262,6 +269,20 @@ class CatWorlds:
             sio = CatEpisodeStatsIO(self.episode_acc.data_ptr(), self.episode_return.data_ptr(),
                                     self.episode_length.data_ptr(), self._episode_totals.data_ptr())
             _lib.check(self.L.cat_env_attach_episode_stats(self._h, C.byref(sio)), "cat_env_attach_episode_stats")
+        self.want_world_params = bool(want_world_params) or param_ranges is not None
+        self._wp = self._wp_ranges = None
+        if self.want_world_params:
+            # [N] CatWorldParams and [n_maps] CatWorldParamRanges as 4-byte words, read and written in place
+            self._wp = torch.from_numpy(np.tile(wparams.defaults(p), N).view(np.int32).reshape(N, wparams.WORDS)).to(dev)
+            self._ranges_host = np.zeros(len(cmaps), wparams.RANGES_DTYPE)
+            self._ranges_host[:] = wparams.ranges_entry(None, p, draw=False)
+            self._wp_ranges = torch.zeros((len(cmaps), wparams.RANGE_WORDS), dtype=torch.int32, device=dev)
+            for slot, spec in enumerate(wparams.per_slot(param_ranges, len(cmaps))):
+                if spec is not None:
+                    self._ranges_host[slot] = wparams.ranges_entry(spec, p)
+            self._upload_ranges()
+            wio = CatWorldParamsIO(self._wp.data_ptr(), self._wp_ranges.data_ptr())
+            _lib.check(self.L.cat_env_attach_world_params(self._h, C.byref(wio)), "cat_env_attach_world_params")
         _lib.check(self.L.cat_env_init_state(self._h, self.state.data_ptr(), self._stream()), "cat_env_init_state")
 
     # ------------------------------------------------------------------ plumbing
@@ -650,6 +671,9 @@ class CatWorlds:
         sd = {"state": self.state.clone(), "seed": torch.tensor(self.params["seed"])}
         if self.episode_acc is not None:
             sd["episode_acc"] = self.episode_acc.clone()
+        if self._wp is not None:
+            sd["world_params"] = self._wp.clone()
+            sd["param_ranges"] = self._wp_ranges.clone()
         return sd
 
     def load_state_dict(self, sd: Mapping[str, torch.Tensor]) -> None:
@@ -657,3 +681,62 @@ class CatWorlds:
         self.set_seed(int(sd["seed"]))
         if self.episode_acc is not None and "episode_acc" in sd:
             self.episode_acc.copy_(sd["episode_acc"].to(self.device))
+        if self._wp is not None and "world_params" in sd:
+            self._wp.copy_(sd["world_params"].to(self.device))
+            self._ranges_host = sd["param_ranges"].cpu().numpy().copy().view(wparams.RANGES_DTYPE).reshape(-1)
+            self._upload_ranges()
+
+    # ------------------------------------------------------------------ per-world parameters
+    def world_params(self) -> Dict[str, torch.Tensor]:
+        """Named device views of the per-world parameter table (writes through them reach the kernel):
+        ``unit_velocity`` (N, 2) and ``max_speed`` (N, 2) float32 by team (``[:, 0]`` cops, ``[:, 1]`` thieves),
+        ``termination_radius`` (N,) float32 and ``max_step_count`` (N,) int32.  The kernel does not check what it
+        reads: ``set_world_params`` does."""
+        if self._wp is None:
+            raise _lib.CatError("per-world parameters are off (want_world_params=False)")
+        f = self._wp.view(torch.float32)
+        return dict(unit_velocity=f[:, 0:2], max_speed=f[:, 2:4], termination_radius=f[:, 4], max_step_count=self._wp[:, 5])
+
+    def set_world_params(self, mask: Optional[torch.Tensor] = None, **values) -> None:
+        """Write per-world parameters in place (a captured graph stays valid), for the worlds of the (N,) bool ``mask``
+        (all if None): ``field=value`` with a number or a tensor broadcastable to the selected worlds; ``unit_velocity``
+        and ``max_speed`` take one value for both teams or ``{"cop": .., "thief": ..}``.  Every value is checked
+        (``world_params.check_values``) before anything is written.  The new values apply from each world's next step;
+        a later re-spawn of a world whose map slot draws replaces them."""
+        views = self.world_params()
+        sel = slice(None) if mask is None else torch.as_tensor(mask, device=self.device).reshape(-1).bool()
+        if mask is not None and sel.numel() != self.n_worlds:
+            raise ValueError(f"mask needs {self.n_worlds} entries, got {sel.numel()}")
+        writes = []
+        for field, value in values.items():
+            for col, v in wparams.per_team(field, value):
+                wparams.check_values(field, v)
+                dst = views[field] if col is None else views[field][:, col]
+                writes.append((dst, torch.as_tensor(v, device=self.device).to(dst.dtype)))
+        for dst, t in writes:
+            dst[sel] = t
+
+    def set_param_ranges(self, slot: Optional[int] = None, draw: bool = True,
+                         **ranges: Union[float, Tuple[float, float], Mapping]) -> None:
+        """Set the randomisation of map slot ``slot`` (every slot if None): ``field=(lo, hi)`` or ``field=value`` (pinned),
+        per team for ``unit_velocity`` / ``max_speed`` (``max_speed={"thief": (125, 175)}``); fields and teams not named
+        are pinned to the environment's values.  With ``draw``, every later re-spawn of a world of the slot draws its
+        table entry from these ranges; ``draw=False`` leaves the table to the caller.  Written in place."""
+        if self._wp is None:
+            raise _lib.CatError("per-world parameters are off (want_world_params=False)")
+        entry = wparams.ranges_entry(ranges, self.params, draw)
+        slots = range(len(self.cmaps)) if slot is None else [int(slot)]
+        for s in slots:
+            if not 0 <= s < len(self.cmaps):
+                raise IndexError(f"map slot {s} out of range (0..{len(self.cmaps) - 1})")
+        for s in slots:
+            self._ranges_host[s] = entry
+        self._upload_ranges()
+
+    def param_ranges(self) -> np.ndarray:
+        """A copy of every map slot's ranges (``world_params.RANGES_DTYPE``)."""
+        return self._ranges_host.copy()
+
+    def _upload_ranges(self) -> None:
+        words = torch.from_numpy(self._ranges_host.view(np.int32).reshape(len(self.cmaps), wparams.RANGE_WORDS).copy())
+        self._wp_ranges.copy_(words)

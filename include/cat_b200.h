@@ -201,6 +201,42 @@ typedef struct {
   CatEpisodeTotals* totals;    /* [n_maps] per map slot; optional */
 } CatEpisodeStatsIO;
 
+/* PER-WORLD PHYSICS PARAMETERS (cat_env_attach_world_params): each world reads its thrust and top speed per team, its
+ * capture radius and its time limit from a caller-owned table instead of CatParams.
+ *
+ * Semantics.  While a table is attached, every step, reset and host-path chunk reads world w's entry params[w] in
+ * place of CatParams.unit_velocity, .max_speed, .termination_radius and .max_step_count.  Agent a uses team
+ * t = (a < n_cops ? 0 : 1): its action adds unit_velocity[t] * (1 / unit_mass) to its velocity (fp32, mass stays
+ * environment-wide) and clamps the speed to max_speed[t].  The capture test is dist^2 < termination_radius^2 and the
+ * timeout step_count >= max_step_count.
+ *
+ * Domain randomisation.  With ranges attached and ranges[slot].draw != 0 for the world's map slot, every re-spawn of
+ * the world (cat_env_reset, the in-kernel auto-reset, and so the resets after cat_env_set_map) writes a fresh draw
+ * into params[w]; the step in which a world ends used its old entry, the new one applies from its next step on.
+ * cat_env_init_state never draws, and with draw == 0 or no ranges the resets leave the table alone (the caller writes
+ * it: curriculum).  The draw is cat_param_draws (cat_philox.h) of (seed, gid, the new episode number): independent of
+ * sharding, chunking and launch shape.  lo == hi pins a field.
+ *
+ * The kernel does not validate the table: it expects finite values, thrust >= 0, top speeds > 0, radius >= 0,
+ * max_step_count >= 1 and lo <= hi (the Python setters check these). */
+typedef struct {
+  float unit_velocity[2];       /* impulse of one action: [0] cops, [1] thieves */
+  float max_speed[2];           /* [0] cops, [1] thieves */
+  float termination_radius;
+  int32_t max_step_count;
+} CatWorldParams;
+
+typedef struct {
+  CatWorldParams lo, hi;        /* floats fmaf(hi - lo, u, lo) with u in [0, 1), max_step_count in [lo, hi] */
+  int32_t draw;                 /* 0: re-spawns leave the table alone */
+} CatWorldParamRanges;
+
+/* caller-owned device pointers, 4-byte aligned */
+typedef struct {
+  CatWorldParams* params;              /* [N] one entry per world; required */
+  const CatWorldParamRanges* ranges;   /* [n_maps] one entry per map slot; optional */
+} CatWorldParamsIO;
+
 /* byte offsets inside one world's output record (cat_env_record_layout / cat_env_packed_record_layout) */
 typedef struct {
   int32_t bytes;        /* record size = default world stride (multiple of 16) */
@@ -336,6 +372,11 @@ int cat_env_observe(CatEnv* env, void* state_dev, const CatStepIO* io, void* str
  * without acc, or a misaligned pointer (4 bytes for the arrays, 8 for totals); nothing is stored then.  A CUDA graph
  * captured before this call keeps the parameters its launches were captured with. */
 int cat_env_attach_episode_stats(CatEnv* env, const CatEpisodeStatsIO* io);
+/* Attach a per-world parameter table (CatWorldParamsIO above), or detach it with io = NULL.  Host only, no CUDA call,
+ * like cat_env_attach_episode_stats: every later launch carries the pointers and runs the full-output kernel.
+ * CAT_ERR_INVALID for a null env, a missing params pointer or a pointer that is not 4-byte aligned; nothing is stored
+ * then.  The table's contents are not checked. */
+int cat_env_attach_world_params(CatEnv* env, const CatWorldParamsIO* io);
 /* parity-test access to the hidden state */
 int cat_env_get_state(CatEnv* env, const void* state_dev, const CatStateView* view, void* stream);
 int cat_env_set_state(CatEnv* env, void* state_dev, const CatStateView* view, void* stream);

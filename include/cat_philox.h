@@ -9,6 +9,7 @@
 #ifndef CAT_PHILOX_H
 #define CAT_PHILOX_H
 
+#include <math.h>
 #include <stdint.h>
 
 #if defined(__CUDACC__)
@@ -63,6 +64,29 @@ CAT_HD void cat_spawn_uniforms(uint64_t seed, uint64_t gid, uint32_t episode, ui
                                   (uint32_t)seed, (uint32_t)(seed >> 32));
   *ux = cat_u01_24(r.v[0]);
   *uy = cat_u01_24(r.v[1]);
+}
+
+/* Per-world parameter draws (CatWorldParams, cat_b200.h), at each re-spawn:
+ *   call j (0, 1) : counter = (gid_lo, gid_hi, episode, 0xFF00 | j)
+ *   fields 0..3 (unit_velocity[0..1], max_speed[0..1]) take the words of call 0, fields 4..5 (termination_radius,
+ *   max_step_count) the first two words of call 1.  Spawns use agent << 8 | try with agent < 8, so the two streams
+ *   never share a counter.
+ * words[6] receives the six words; cat_param_float / cat_param_int map one to its range. */
+CAT_HD void cat_param_draws(uint64_t seed, uint64_t gid, uint32_t episode, uint32_t words[6]) {
+  for (uint32_t j = 0; j < 2; ++j) {
+    cat_u32x4 r = cat_philox4x32_10((uint32_t)gid, (uint32_t)(gid >> 32), episode, 0xFF00u | j,
+                                    (uint32_t)seed, (uint32_t)(seed >> 32));
+    for (int i = 0; i < 4 && 4 * (int)j + i < 6; ++i) words[4 * j + i] = r.v[i];
+  }
+}
+
+/* a float field: uniform on [lo, hi) before the fp32 rounding, which can reach hi (one fma: the GPU and the oracle
+ * agree bit for bit) */
+CAT_HD float cat_param_float(uint32_t word, float lo, float hi) { return fmaf(hi - lo, cat_u01_24(word), lo); }
+
+/* an integer field in [lo, hi] */
+CAT_HD int32_t cat_param_int(uint32_t word, int32_t lo, int32_t hi) {
+  return lo + (int32_t)(((uint64_t)word * (uint64_t)(uint32_t)(hi - lo + 1)) >> 32);
 }
 
 #endif /* CAT_PHILOX_H */

@@ -7,6 +7,7 @@ all-reduced over NCCL per minibatch.
     python tools/train_selfplay.py --map squarinth,agh-map,labyrinth --worlds 4096   # one policy over three maps
     python tools/train_selfplay.py --map squarinth --procedural 2 --swap-every 4     # + 2 slots of fresh mazes
     python tools/train_selfplay.py --map squarinth,agh-map --episode-stats            # + episode returns / lengths
+    python tools/train_selfplay.py --episode-stats --randomize "max_speed.thief=125:175,termination_radius=15:25"
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_selfplay.py ...
 
 Prints one JSON line per self-play iteration (rank 0): environment agent-steps/s inside training, GAE / update /
@@ -24,7 +25,7 @@ import torch
 
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
-from as_cops_and_thieves_b200 import episodes, selfplay  # noqa: E402
+from as_cops_and_thieves_b200 import episodes, selfplay, world_params  # noqa: E402
 from as_cops_and_thieves_b200.env import BatchedCopsThievesEnv  # noqa: E402
 from as_cops_and_thieves_b200.mappo import MAPPOConfig, MAPPOLearner  # noqa: E402
 from as_cops_and_thieves_b200.maps import free_space_regions, generate_maze, load_named_map  # noqa: E402
@@ -57,7 +58,11 @@ def main():
     ap.add_argument("--maze-seed", type=int, default=0, help="seed of the first maze; later mazes take the next seeds")
     ap.add_argument("--episode-stats", action="store_true",
                     help="report the returns, lengths and capture rate of the training episodes, overall and per map")
+    ap.add_argument("--randomize", default="",
+                    help="domain randomisation drawn at every re-spawn, e.g. 'max_speed.thief=125:175,termination_radius="
+                         "15:25,max_step_count=300:500' (field[.cop|.thief]=lo:hi, or one number to pin it)")
     a = ap.parse_args()
+    randomize = world_params.parse_cli(a.randomize) if a.randomize else None
 
     rank, local_rank, world_size = dist_env()
     dev = torch.device(f"cuda:{local_rank}")
@@ -82,11 +87,11 @@ def main():
     if len(maps) == 1:
         env = BatchedCopsThievesEnv(maps[0], n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
                                     spawn_override=spawn[0], final_observations=a.time_limit_bootstrap,
-                                    episode_statistics=a.episode_stats)
+                                    episode_statistics=a.episode_stats, randomize=randomize)
     else:
         env = BatchedCopsThievesEnv(maps, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
                                     spawn_override=spawn, final_observations=a.time_limit_bootstrap,
-                                    swappable_maps=swappable, episode_statistics=a.episode_stats)
+                                    swappable_maps=swappable, episode_statistics=a.episode_stats, randomize=randomize)
     # the reference's schedule (10 000 random / 15 000 before learning / 15 000 frozen policy) counts steps of ONE
     # environment; with thousands of lockstep worlds the same number of TRANSITIONS is reached in a few steps, so the
     # driver scales the durations by the world count unless told otherwise
