@@ -13,7 +13,7 @@ import numpy as np
 
 from . import build as _build
 
-CAT_ABI_VERSION = 8
+CAT_ABI_VERSION = 9
 CAT_MAX_AGENTS = 8
 CAT_MAX_RAYS = 128
 CAT_MAX_MAPS = 8
@@ -55,11 +55,8 @@ class CatParams(C.Structure):
 class CatStepIO(C.Structure):
     _fields_ = [
         ("actions", C.c_void_p), ("actions_kind", C.c_int32), ("reset_mask", C.c_void_p),
-        ("obs_dist", C.c_void_p), ("obs_type", C.c_void_p), ("reward", C.c_void_p),
-        ("terminated", C.c_void_p), ("truncated", C.c_void_p), ("winner", C.c_void_p),
         ("shared_dist", C.c_void_p), ("shared_type", C.c_void_p), ("team_pos", C.c_void_p),
         ("obs_f32", C.c_void_p), ("state_f32", C.c_void_p), ("hit_point", C.c_void_p),
-        ("obs_dist_world_stride", C.c_int32), ("obs_type_world_stride", C.c_int32),
         ("record", C.c_void_p), ("record_world_stride", C.c_int32),
         ("critic_f32", C.c_void_p), ("obs_bf16", C.c_void_p), ("critic_bf16", C.c_void_p), ("record_packed_types", C.c_int32),
         ("final_record", C.c_void_p), ("final_record_world_stride", C.c_int32),

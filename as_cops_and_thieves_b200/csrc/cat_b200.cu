@@ -906,16 +906,7 @@ static int prepare(CatEnv* env, void* state_dev, const CatStepIO* io, int mode, 
       else k.actions[0] = io->actions;
     }
     k.reset_mask = io->reset_mask;
-    k.obs_dist = io->obs_dist; k.obs_type = io->obs_type; k.reward = io->reward;
-    k.dist_stride = io->obs_dist_world_stride ? io->obs_dist_world_stride : k.lay.nrays * 2;
-    k.type_stride = io->obs_type_world_stride ? io->obs_type_world_stride : k.lay.nrays;
-    if (k.dist_stride < k.lay.nrays * 2 || (k.dist_stride & 1) || k.type_stride < k.lay.nrays)
-      return fail(CAT_ERR_INVALID, "observation world strides are smaller than one world's block");
-    k.obs_vec = ((k.dist_stride | k.type_stride) & 15) == 0 &&
-                ((reinterpret_cast<uintptr_t>(io->obs_dist) | reinterpret_cast<uintptr_t>(io->obs_type)) & 15) == 0 &&
-                k.dist_stride >= (k.lay.nrays * 2 + 15) / 16 * 16 && k.type_stride >= (k.lay.nrays + 15) / 16 * 16;
-    k.terminated = io->terminated;
-    k.truncated = io->truncated; k.winner = io->winner; k.shared_dist = io->shared_dist; k.shared_type = io->shared_type;
+    k.shared_dist = io->shared_dist; k.shared_type = io->shared_type;
     k.team_pos = io->team_pos; k.obs_f32 = io->obs_f32; k.state_f32 = io->state_f32; k.hit_point = io->hit_point;
     k.critic_f32 = io->critic_f32; k.obs_bf16 = io->obs_bf16; k.critic_bf16 = io->critic_bf16;
     if (io->record) {
@@ -925,7 +916,6 @@ static int prepare(CatEnv* env, void* state_dev, const CatStepIO* io, int mode, 
       k.record_stride = io->record_world_stride ? io->record_world_stride : rec_bytes;
       if ((reinterpret_cast<uintptr_t>(io->record) & 15) || (k.record_stride & 15) || k.record_stride < rec_bytes)
         return fail(CAT_ERR_INVALID, "record output must be 16-byte aligned with a world stride that is a multiple of 16 and >= CatRecordLayout.bytes");
-      k.obs_dist = nullptr; k.obs_type = nullptr; k.reward = nullptr; k.terminated = nullptr; k.truncated = nullptr; k.winner = nullptr;
     }
     if (mode == MODE_STEP) {   // final outputs: step launches only (reset / observe share the caller's CatStepIO)
       if (io->final_record) {

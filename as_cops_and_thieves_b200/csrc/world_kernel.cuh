@@ -164,14 +164,6 @@ struct KParams {
   const void* actions[CAT_MAX_AGENTS];
   int actions_kind;
   const uint8_t* reset_mask;
-  uint16_t* obs_dist;
-  uint8_t* obs_type;
-  int dist_stride, type_stride;   // bytes between worlds
-  int obs_vec;                    // 1: both strides and bases are 16-byte aligned -> uint4 stores
-  float* reward;
-  uint8_t* terminated;
-  uint8_t* truncated;
-  int8_t* winner;
   uint16_t* shared_dist;
   uint8_t* shared_type;
   uint16_t* team_pos;
@@ -1058,64 +1050,12 @@ __device__ __noinline__ void write_flat_layouts(const KParams& k, const FlatOut 
   }
 }
 
-// Write the outputs of one world from shared memory (coalesced).  `flags_too`: the staged rewards / flags belong
-// to this launch (a step); reset / observe launches leave the caller's reward / flag arrays alone, except in record
-// mode, where the whole record is one block (their staged values are then 0 / 0 / 0 / -1).
+// Write the optional outputs of one world from shared memory (coalesced).  The record goes last, by write_record: its
+// packed form rewrites the staged types in place.
 template <int TA, int TR>
-__device__ __forceinline__ void write_optional_outputs(const KParams& k, const Warp& w, long long world, bool flags_too) {
-  const int A = TA ? TA : k.A, R = TR ? TR : k.R, lane = w.lane, nrays = A * R;
+__device__ __forceinline__ void write_optional_outputs(const KParams& k, const Warp& w, long long world) {
+  const int A = TA ? TA : k.A, R = TR ? TR : k.R, lane = w.lane;
   const float* pos = w.rec;
-  if (k.record) {
-    // (shipped last, by write_record: the packed form rewrites the staged types in place)
-  } else if (k.obs_vec) {
-    // 16-byte aligned world blocks (mapped pinned host memory): one or two 512-byte warp stores per array
-    if (k.obs_dist) {
-      uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(k.obs_dist) + (size_t)world * k.dist_stride);
-      const uint4* src = reinterpret_cast<const uint4*>(w.rdist);
-#pragma unroll 1
-      for (int i = lane; i < (nrays * 2 + 15) / 16; i += 32) dst[i] = src[i];
-    }
-    if (k.obs_type) {
-      uint4* dst = reinterpret_cast<uint4*>(k.obs_type + (size_t)world * k.type_stride);
-      const uint4* src = reinterpret_cast<const uint4*>(w.rtype);
-#pragma unroll 1
-      for (int i = lane; i < (nrays + 15) / 16; i += 32) dst[i] = src[i];
-    }
-  } else {
-    if (k.obs_dist) {
-      unsigned char* base = reinterpret_cast<unsigned char*>(k.obs_dist) + (size_t)world * k.dist_stride;
-      if (((nrays | (k.dist_stride >> 1)) & 1) == 0) {
-        uint32_t* dst = reinterpret_cast<uint32_t*>(base);
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(w.rdist);
-#pragma unroll 1
-        for (int i = lane; i < nrays / 2; i += 32) dst[i] = src[i];
-      } else {
-        uint16_t* dst = reinterpret_cast<uint16_t*>(base);
-#pragma unroll 1
-        for (int i = lane; i < nrays; i += 32) dst[i] = w.rdist[i];
-      }
-    }
-    if (k.obs_type) {
-      uint8_t* base = k.obs_type + (size_t)world * k.type_stride;
-      if (((nrays | k.type_stride) & 1) == 0) {
-        uint16_t* dst = reinterpret_cast<uint16_t*>(base);
-        const uint16_t* src = reinterpret_cast<const uint16_t*>(w.rtype);
-#pragma unroll 1
-        for (int i = lane; i < nrays / 2; i += 32) dst[i] = src[i];
-      } else {
-#pragma unroll 1
-        for (int i = lane; i < nrays; i += 32) base[i] = w.rtype[i];
-      }
-    }
-  }
-  if (!k.record && flags_too) {
-    if (lane < A && k.reward) k.reward[(size_t)world * A + lane] = w.rew[lane];
-    if (lane == 0) {
-      if (k.terminated) k.terminated[world] = w.flg[0];
-      if (k.truncated) k.truncated[world] = w.flg[1];
-      if (k.winner) k.winner[world] = (int8_t)w.flg[2];
-    }
-  }
   if (k.team_pos) {  // observation_spaces.py:92-95
 #pragma unroll 1
     for (int i = lane; i < 2 * A; i += 32)
@@ -1206,8 +1146,8 @@ __device__ __forceinline__ void write_record(const KParams& k, const Warp& w, lo
 // TX = false: the instantiation for launches that ask for the record and nothing else (the host picks it per launch) —
 // none of the optional outputs above is compiled in.
 template <int TA, int TR, bool TX>
-__device__ __forceinline__ void write_observation(const KParams& k, const Warp& w, long long world, bool flags_too) {
-  if (TX) write_optional_outputs<TA, TR>(k, w, world, flags_too);
+__device__ __forceinline__ void write_observation(const KParams& k, const Warp& w, long long world) {
+  if (TX) write_optional_outputs<TA, TR>(k, w, world);
   if (TX ? k.record != nullptr : true) write_record<TA, TR, false>(k, w, world);
 }
 
@@ -1661,7 +1601,7 @@ __device__ __forceinline__ void episode_stats(const KParams& k, const Warp& w, l
 // TA / TR: agents per world and rays per agent as compile-time constants (the 2 cops + 1 thief x 90 rays of every
 // shipped map: <3, 90>), or 0 = read them from the parameters (any other configuration: <0, 0>).  TL: the environment
 // has ray lists (the default) — the instantiation carries no rasteriser code at all.  TX = false: a STEP launch that wants the
-// output record only — none of the optional outputs (separate arrays, shared observations, fp32 / bf16 layouts, hit
+// output record only — none of the optional outputs (shared observations, team positions, fp32 / bf16 layouts, hit
 // points) and none of the init / reset / observe launch modes is compiled in.  TM: a mixed-map environment — each CTA
 // looks its map up in the launch's map table and reads the map-dependent values from the blob header it staged; the
 // single-map instantiations (TM = false) take them from the parameters, at no register cost (a run-time table lookup
@@ -1926,7 +1866,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
       }
       __syncwarp();
       if (final_out) write_final_outputs<TA, TR>(k, w, world);
-      if (!again) write_observation<TA, TR, TX>(k, w, world, mode == MODE_STEP);
+      if (!again) write_observation<TA, TR, TX>(k, w, world);
       __syncwarp();
       if (do_step) {
         physics_world<TA, TR>(k, m, w);  // base_env.py:392

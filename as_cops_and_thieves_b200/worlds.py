@@ -320,12 +320,13 @@ class CatWorlds:
         def dp(t):
             return None if t is None or not extras else t.data_ptr()
         rec = self._out if record is None else record
-        return CatStepIO(None, 0, None, None, None, None, None, None, None, dp(self.shared_dist), dp(self.shared_type),
-                         dp(self.team_pos), dp(self.obs_f32), dp(self.state_f32), dp(self.hit_point), 0, 0,
-                         rec.data_ptr(), self.packed_record_bytes if packed else self.record_bytes,
-                         dp(self.critic_f32), dp(self.obs_bf16), dp(self.critic_bf16), 1 if packed else 0,
-                         dp(self._final_out), self.record_bytes, dp(self.final_obs_f32), dp(self.final_state_f32),
-                         dp(self.final_critic_f32))
+        return CatStepIO(shared_dist=dp(self.shared_dist), shared_type=dp(self.shared_type), team_pos=dp(self.team_pos),
+                         obs_f32=dp(self.obs_f32), state_f32=dp(self.state_f32), hit_point=dp(self.hit_point),
+                         record=rec.data_ptr(), record_world_stride=self.packed_record_bytes if packed else self.record_bytes,
+                         critic_f32=dp(self.critic_f32), obs_bf16=dp(self.obs_bf16), critic_bf16=dp(self.critic_bf16),
+                         record_packed_types=1 if packed else 0, final_record=dp(self._final_out),
+                         final_record_world_stride=self.record_bytes, final_obs_f32=dp(self.final_obs_f32),
+                         final_state_f32=dp(self.final_state_f32), final_critic_f32=dp(self.final_critic_f32))
 
     def map_info(self, m: int) -> CatEnvInfo:
         """``cat_env_map_info``: the figures of map ``m`` alone (its worlds, hulls, edges, blob and ray-list bytes)."""

@@ -16,13 +16,14 @@
  *   - there is NO CPU fallback: every compute entry point fails with CAT_ERR_CUDA without a GPU.
  *
  * Layouts (N worlds, A = n_cops + n_thieves agents ordered cops then thieves
- * [base_env.py:91-96], R rays):
- *   obs_dist  f16 [N][A][R]   entity.py:200-210   (float16 chain reproduced bit-for-bit)
- *   obs_type  u8  [N][A][R]   entity.py:222-241   (WALL 0, COP 1, THIEF 2, EMPTY 4)
- *   reward    f32 [N][A]      cop.py:49-75, thief.py:48-69
- *   terminated u8 [N]         captured or timed out (entity.py:146)
- *   truncated  u8 [N]         timed out (base_env.py:397)
- *   winner     i8 [N]         -1 none, 0 cop, 1 thief (base_env.py:399-411)
+ * [base_env.py:91-96], R rays).  Fields of each world's output record (CatStepIO.record, CatRecordLayout):
+ *   distance  f16 [A][R]      entity.py:200-210   (float16 chain reproduced bit-for-bit)
+ *   type      u8  [A][R]      entity.py:222-241   (WALL 0, COP 1, THIEF 2, EMPTY 4)
+ *   reward    f32 [A]         cop.py:49-75, thief.py:48-69
+ *   terminated u8             captured or timed out (entity.py:146)
+ *   truncated  u8             timed out (base_env.py:397)
+ *   winner     i8             -1 none, 0 cop, 1 thief (base_env.py:399-411)
+ * Optional caller arrays:
  *   shared_dist f16 [N][2][R], shared_type u8 [N][2][R]   observation_spaces.py:97-121 (team 0 cops, 1 thieves)
  *   team_pos  f16 [N][A][2]   observation_spaces.py:92-95
  *   obs_f32   f32 [A][N][2R]  per-agent obs as skrl flattens it: [distance | object_type]
@@ -39,7 +40,7 @@
 extern "C" {
 #endif
 
-#define CAT_ABI_VERSION 8
+#define CAT_ABI_VERSION 9
 #define CAT_MAX_AGENTS 8
 #define CAT_MAX_RAYS 128
 #define CAT_MAX_MAPS 8 /* maps of one environment (cat_env_create_multi) */
@@ -109,29 +110,18 @@ typedef struct {
   /* input (reset only): u8 [N] device mask, NULL = every world */
   const uint8_t* reset_mask;
   /* outputs — device pointers, any may be NULL */
-  uint16_t* obs_dist;
-  uint8_t* obs_type;
-  float* reward;
-  uint8_t* terminated;
-  uint8_t* truncated;
-  int8_t* winner;
   uint16_t* shared_dist;
   uint8_t* shared_type;
   uint16_t* team_pos;
   float* obs_f32;
   float* state_f32;
   float* hit_point;
-  /* bytes between consecutive worlds in obs_dist / obs_type; 0 = dense (A*R*2 and A*R).  A stride that is a
-   * multiple of 16 (with a 16-byte aligned base) lets the kernel store each world's observation with 16-byte
-   * vector stores (the world's block is then written up to the next multiple of 16 bytes, padding included). */
-  int32_t obs_dist_world_stride;
-  int32_t obs_type_world_stride;
-  /* RECORD OUTPUT (preferred): one contiguous record per world, CatRecordLayout below —
+  /* RECORD OUTPUT: one contiguous record per world, CatRecordLayout below —
    *   [ f16 distance A*R | pad to 16 | u8 type A*R | pad to 4 | f32 reward A | u8 terminated | u8 truncated | i8 winner | pad to 16 ]
-   * written with 16-byte stores (device memory or mapped pinned host memory).  When `record` is non-NULL the six
-   * pointers obs_dist, obs_type, reward, terminated, truncated, winner above are ignored: one world = one block,
-   * so a host-facing caller moves a range of worlds with ONE copy.  record must be 16-byte aligned and
-   * record_world_stride a multiple of 16 that is >= CatRecordLayout.bytes (0 = exactly that). */
+   * written with 16-byte stores (device memory or mapped pinned host memory).  One world = one block, so a host-facing
+   * caller moves a range of worlds with ONE copy.  NULL = no record: the launch writes only the optional outputs it is
+   * given.  record must be 16-byte aligned and record_world_stride a multiple of 16 that is >= CatRecordLayout.bytes
+   * (0 = exactly that). */
   void* record;
   int32_t record_world_stride;
   /* critic front end (lstm_value_net.py:122-137): the 4 ray channels LSTMValue cuts from the first agent's block of

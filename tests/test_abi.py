@@ -39,30 +39,34 @@ def test_every_declared_symbol_is_exported_and_bound():
     assert sorted(_lib.EXPORTS) == decl, "the ctypes binding must cover exactly the declared ABI"
 
 
-def test_struct_layouts_match_what_a_c_compiler_sees(tmp_path):
-    """Compile a probe against include/cat_b200.h with gcc and compare sizeof/offsetof with ctypes."""
+def test_every_struct_field_matches_what_a_c_compiler_sees(tmp_path):
+    """Compile a probe against include/cat_b200.h with gcc, generated from the binding: every ``CAT_*`` constant, and for
+    every ctypes struct its size and alignment and every field's offset, size and alignment, compared with ctypes.  A
+    field the header does not have under the binding's name fails to compile."""
     import subprocess
+    structs = {n: T for n, T in vars(_lib).items()
+               if isinstance(T, type) and issubclass(T, C.Structure) and T.__module__ == _lib.__name__}
+    consts = {n: v for n, v in vars(_lib).items() if n.startswith("CAT_") and isinstance(v, int)}
+    assert len(structs) >= 12 and "CAT_ABI_VERSION" in consts
+    want, exprs = dict(consts), {n: n for n in consts}
+    for name, T in structs.items():
+        want[f"sizeof({name})"], want[f"alignof({name})"] = C.sizeof(T), C.alignment(T)
+        exprs[f"sizeof({name})"], exprs[f"alignof({name})"] = f"sizeof({name})", f"_Alignof({name})"
+        for f, ftype in T._fields_:
+            member = f"(({name}*)0)->{f}"
+            for what, expr, val in (("offsetof", f"offsetof({name}, {f})", getattr(T, f).offset),
+                                    ("sizeof", f"sizeof({member})", getattr(T, f).size),
+                                    ("alignof", f"__alignof__({member})", C.alignment(ftype))):
+                want[f"{what}({name}.{f})"], exprs[f"{what}({name}.{f})"] = val, expr
+    lines = "\n".join(f'  printf("%s %lld\\n", "{key}", (long long)({expr}));' for key, expr in exprs.items())
     probe = tmp_path / "probe.c"
-    probe.write_text(r"""
-#include <stdio.h>
-#include <stddef.h>
-#include "cat_b200.h"
-int main(void) {
-  printf("%zu %zu %zu %zu %zu %zu\n", sizeof(CatMapDesc), sizeof(CatParams), sizeof(CatStepIO), sizeof(CatEnvInfo), sizeof(CatStateView), sizeof(CatRecordLayout));
-  printf("%zu %zu %zu %zu\n", offsetof(CatMapDesc, grid_x0), offsetof(CatParams, seed), offsetof(CatStepIO, obs_dist), offsetof(CatStateView, pair_jn));
-  printf("%zu %zu %zu %zu %zu\n", offsetof(CatParams, ray_list_cell), offsetof(CatStepIO, record), offsetof(CatStepIO, critic_bf16), offsetof(CatEnvInfo, ray_list_bytes), offsetof(CatRecordLayout, off_winner));
-  return 0;
-}""")
+    probe.write_text(f'#include <stdio.h>\n#include <stddef.h>\n#include "cat_b200.h"\nint main(void) {{\n{lines}\n  return 0;\n}}\n')
     exe = tmp_path / "probe"
     subprocess.run(["/usr/bin/gcc", "-I", str(ROOT / "include"), str(probe), "-o", str(exe)], check=True)
-    out = subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.split()
-    got = [int(x) for x in out]
-    want = [C.sizeof(_lib.CatMapDesc), C.sizeof(_lib.CatParams), C.sizeof(_lib.CatStepIO), C.sizeof(_lib.CatEnvInfo),
-            C.sizeof(_lib.CatStateView), C.sizeof(_lib.CatRecordLayout), _lib.CatMapDesc.grid_x0.offset, _lib.CatParams.seed.offset,
-            _lib.CatStepIO.obs_dist.offset, _lib.CatStateView.pair_jn.offset, _lib.CatParams.ray_list_cell.offset,
-            _lib.CatStepIO.record.offset, _lib.CatStepIO.critic_bf16.offset, _lib.CatEnvInfo.ray_list_bytes.offset,
-            _lib.CatRecordLayout.off_winner.offset]
+    out = subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout
+    got = {key: int(v) for key, v in (line.split(" ") for line in out.splitlines())}
     assert got == want
+    assert _lib.CAT_ABI_VERSION == 9
 
 
 def _desc(cmap):
