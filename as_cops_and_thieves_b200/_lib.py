@@ -19,6 +19,10 @@ CAT_MAX_RAYS = 128
 CAT_MAX_MAPS = 8
 CAT_WALL_SLOTS = 4
 CAT_NEAR_SLOTS = 4
+CAT_SCRIPT_NONE = 0
+CAT_SCRIPT_RANDOM = 1
+CAT_SCRIPT_CHASE = 2
+CAT_SCRIPT_EVADE = 3
 
 
 class CatError(RuntimeError):
@@ -90,6 +94,10 @@ class CatWorldParamsIO(C.Structure):
     _fields_ = [("params", C.c_void_p), ("ranges", C.c_void_p)]
 
 
+class CatScriptIO(C.Structure):
+    _fields_ = [("mode", C.c_void_p), ("decisions", C.c_void_p)]
+
+
 class CatRecordLayout(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("bytes", "off_dist", "off_type", "off_reward", "off_terminated",
                                          "off_truncated", "off_winner", "type_bits")]
@@ -123,7 +131,8 @@ EXPORTS = (
     "cat_env_map_info", "cat_env_create_swappable", "cat_env_set_map", "cat_map_blob_bytes", "cat_ray_lists_device",
     "cat_env_record_layout", "cat_env_packed_record_layout", "cat_env_overflow_counts", "cat_ray_lists_host",
     "cat_env_set_seed", "cat_env_state_bytes", "cat_env_init_state", "cat_env_reset", "cat_env_step", "cat_env_step_host", "cat_env_observe",
-    "cat_env_get_state", "cat_env_set_state", "cat_env_attach_episode_stats", "cat_env_attach_world_params", "cat_gae", "cat_adv_normalize",
+    "cat_env_get_state", "cat_env_set_state", "cat_env_attach_episode_stats", "cat_env_attach_world_params",
+    "cat_env_attach_scripts", "cat_gae", "cat_adv_normalize",
     "cat_renderer_create", "cat_renderer_destroy", "cat_renderer_frame_size", "cat_render", "cat_ray_directions",
 )
 
@@ -178,6 +187,7 @@ def load():
         fn.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(CatStateView), C.c_void_p]
     L.cat_env_attach_episode_stats.argtypes = [C.c_void_p, C.POINTER(CatEpisodeStatsIO)]
     L.cat_env_attach_world_params.argtypes = [C.c_void_p, C.POINTER(CatWorldParamsIO)]
+    L.cat_env_attach_scripts.argtypes = [C.c_void_p, C.POINTER(CatScriptIO)]
     L.cat_gae.argtypes = [C.c_void_p] * 7 + [C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_void_p]
     L.cat_adv_normalize.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
     L.cat_renderer_create.argtypes = [C.POINTER(CatMapDesc), C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int32,

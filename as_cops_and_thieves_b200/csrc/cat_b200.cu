@@ -937,7 +937,8 @@ static int prepare(CatEnv* env, void* state_dev, const CatStepIO* io, int mode, 
 static WorldKernel kernel_for(const CatEnv* env, const KParams& k) {
   const bool record_only = k.mode == MODE_STEP && k.record && !k.shared_dist && !k.shared_type && !k.team_pos && !k.obs_f32 && !k.state_f32 &&
                            !k.hit_point && !k.critic_f32 && !k.obs_bf16 && !k.critic_bf16 &&
-                           !k.final_record && !k.final_obs_f32 && !k.final_state_f32 && !k.final_critic_f32 && !k.ep_acc && !k.wp;
+                           !k.final_record && !k.final_obs_f32 && !k.final_state_f32 && !k.final_critic_f32 && !k.ep_acc && !k.wp &&
+                           !k.script_mode;
   return record_only ? env->kernel_record : env->kernel;
 }
 
@@ -968,6 +969,18 @@ int cat_env_attach_world_params(CatEnv* env, const CatWorldParamsIO* io) {
   if ((reinterpret_cast<uintptr_t>(io->params) | reinterpret_cast<uintptr_t>(io->ranges)) & 3)
     return fail(CAT_ERR_INVALID, "world parameters: params / ranges must be 4-byte aligned");
   env->kp.wp = io->params; env->kp.wp_ranges = io->ranges;
+  return CAT_OK;
+}
+
+// Like the statistics, the tables live in env->kp.
+int cat_env_attach_scripts(CatEnv* env, const CatScriptIO* io) {
+  if (!env) return fail(CAT_ERR_INVALID, "null env");
+  if (!io) {
+    env->kp.script_mode = nullptr; env->kp.script_dec = nullptr;
+    return CAT_OK;
+  }
+  if (!io->mode || !io->decisions) return fail(CAT_ERR_INVALID, "scripts need mode and decisions");
+  env->kp.script_mode = io->mode; env->kp.script_dec = io->decisions;
   return CAT_OK;
 }
 

@@ -199,6 +199,10 @@ struct KParams {
   // instantiations only (kernel_for never picks the record-only one while wp is set).
   CatWorldParams* wp;                      // [N]
   const CatWorldParamRanges* wp_ranges;    // [n_maps], by map slot like ep_totals; nullptr = never draw
+  // Scripted agents (cat_env_attach_scripts), carried like the statistics and read by the TX = true instantiations only
+  // (kernel_for never picks the record-only one while script_mode is set).  Both set or both null.
+  const uint8_t* script_mode;     // [N][A] CAT_SCRIPT_*
+  uint8_t* script_dec;            // [N][A] the controllers' decisions from the last emitted observation
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -1554,6 +1558,48 @@ __device__ __forceinline__ void draw_world_params(const KParams& k, const Warp& 
   k.wp[world] = p;
 }
 
+// Scripted agents (cat_env_attach_scripts): the three controllers' next actions from the observation the warp has
+// staged and is about to emit, one byte per agent (random | chase << 2 | evade << 4, cat_b200.h).  Lanes are rays: for
+// each agent an argmin of (d << 16 | i) over the rays that see its target, by warp reduction; lane a then owns agent a's
+// decision (four axis-ray reads for evade, one Philox call).  Kept out of line, like los_blocked, so that it stays off
+// the register budget of the full-output kernels.  Reads the staged record only; the caller syncs the warp after it.
+__device__ __noinline__ void write_script_decisions(uint8_t* dec, const uint16_t* rdist, const uint8_t* rtype,
+                                                    unsigned long long seed, unsigned long long gid, uint32_t episode,
+                                                    uint32_t step_count, int lane, int A, int nc, int R) {
+  uint32_t mine = kEmpty;   // lane a: the (d << 16 | i) key of the closest target agent a sees
+#pragma unroll 1
+  for (int a = 0; a < A; ++a) {
+    const uint8_t target = a < nc ? TYPE_THIEF : TYPE_COP;
+    uint32_t best = kEmpty;
+#pragma unroll 1
+    for (int i = lane; i < R; i += 32)
+      if (rtype[a * R + i] == target) best = min(best, (uint32_t)rdist[a * R + i] << 16 | (uint32_t)i);
+    best = __reduce_min_sync(0xFFFFFFFFu, best);
+    if (lane == a) mine = best;
+  }
+  if (lane >= A) return;
+  const int a = lane;
+  const uint32_t rnd = cat_script_random(seed, gid, episode, step_count, (uint32_t)a);
+  uint32_t chase = rnd, evade = rnd;
+  if (mine != kEmpty) {
+    constexpr uint32_t kAct = 2u | 1u << 2 | 0u << 4 | 3u << 6;   // ACT[q] = (kAct >> 2 q) & 3: +x, +y, -x, -y
+    const uint8_t target = a < nc ? TYPE_THIEF : TYPE_COP;
+    const int qs = ((8 * (int)(mine & 0xFFFFu) + R) / (2 * R)) & 3;
+    chase = (kAct >> (2 * qs)) & 3u;
+    int best_q = 0;
+    uint32_t best_c = 0;
+#pragma unroll
+    for (int t = 0; t < 3; ++t) {
+      const int q = (qs + (t == 0 ? 2 : t == 1 ? 1 : 3)) & 3;
+      const int j = ((q * R + 2) / 4) % R;
+      const uint32_t c = rtype[a * R + j] == target ? 0u : (uint32_t)rdist[a * R + j];
+      if (t == 0 || c > best_c) { best_c = c; best_q = q; }
+    }
+    evade = (kAct >> (2 * best_q)) & 3u;
+  }
+  dec[a] = (uint8_t)(rnd | chase << 2 | evade << 4);
+}
+
 // Order-preserving u32 key of an fp32 value (CatEpisodeTotals): sign bit clear -> bits | 0x80000000, set -> ~bits.
 // Non-zero for every non-NaN value, and so is its complement, so 0 stays "empty" for both the maximum and the minimum.
 __device__ __forceinline__ uint32_t ep_key(float v) {
@@ -1747,6 +1793,7 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
         grec[i] = v;
       }
       if (TX && k.ep_acc && lane < A) k.ep_acc[(size_t)world * A + lane] = 0.f;   // no episode is running yet
+      if (TX && k.script_mode && lane < A) k.script_dec[(size_t)world * A + lane] = 0;   // nothing observed yet
       continue;
     }
     if (mode == MODE_RESET && k.reset_mask && !k.reset_mask[world]) continue;
@@ -1814,6 +1861,10 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
         else if (k.actions_kind == 1) act = reinterpret_cast<const int32_t*>(k.actions[0])[ai];
         else if (k.actions_kind == 2) act = (int)reinterpret_cast<const long long*>(k.actions[0])[ai];
         else act = (int)reinterpret_cast<const long long*>(k.actions[lane])[world];
+        if (TX && k.script_mode) {   // a scripted agent: its controller's decision from the last emitted observation
+          const int sm = k.script_mode[ai];
+          if (sm) act = (k.script_dec[ai] >> (2 * (sm - 1))) & 3;
+        }
         float fx = 0.f, fy = 0.f;
         if (act == 0) fx = -WORLD_PARAM(impulse, impulse); else if (act == 1) fy = WORLD_PARAM(impulse, impulse);
         else if (act == 2) fx = WORLD_PARAM(impulse, impulse); else if (act == 3) fy = -WORLD_PARAM(impulse, impulse);
@@ -1866,7 +1917,18 @@ __global__ void __launch_bounds__(kMaxThreads, 1) cat_world_kernel(const __grid_
       }
       __syncwarp();
       if (final_out) write_final_outputs<TA, TR>(k, w, world);
-      if (!again) write_observation<TA, TR, TX>(k, w, world);
+      if (!again) {
+        // the controllers decide on the observation this launch emits (before write_observation: the packed record
+        // form rewrites the staged types); observe launches leave the decisions alone
+        if (TX && k.script_mode && mode != MODE_OBSERVE) {
+          const uint32_t* recu = reinterpret_cast<const uint32_t*>(w.rec);
+          write_script_decisions(k.script_dec + (size_t)world * A, w.rdist, w.rtype, k.seed,
+                                 (unsigned long long)(k.gid0 + world), recu[LAY(o_ep)], recu[LAY(o_sc)], lane, A, k.nc,
+                                 TR ? TR : k.R);
+          __syncwarp();
+        }
+        write_observation<TA, TR, TX>(k, w, world);
+      }
       __syncwarp();
       if (do_step) {
         physics_world<TA, TR>(k, m, w);  // base_env.py:392

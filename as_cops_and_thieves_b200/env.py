@@ -284,6 +284,12 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
     draws a world's thrust and top speed per team, capture radius and time limit for its next episode, inside the step
     kernel.  ``world_params()``, ``set_world_params(...)`` and ``set_randomization(...)`` read and change them between
     steps (a curriculum); observation and state spaces do not change.
+
+    ``scripted``: built-in controllers play chosen agents inside the step kernel, e.g. ``{"thief_0": "evade"}``
+    (modes ``random``, ``chase``, ``evade``, ``none``; ``scripts.py``).  An empty dict turns them on with nobody
+    scripted.  A controller decides from the agent's own observation that the last step or reset emitted, and the next
+    step uses that decision instead of the caller's action.  ``set_scripted(spec, mask)`` changes the modes between steps
+    (in place, graph-safe); ``step`` takes a mapping without the agents in ``scripted_agents``.
     """
 
     def __init__(self, map: Union[Map, Sequence[Map]], num_envs: Union[int, Sequence[int]], *, max_step_count: int = 400,
@@ -292,7 +298,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
                  spawn_override: Optional[Union[dict, Sequence[Optional[dict]]]] = None, cell: Optional[float] = None,
                  render_mode=None, final_observations: bool = False, swappable_maps: bool = False,
                  episode_statistics: bool = False,
-                 randomize: Union[None, Mapping, Sequence[Optional[Mapping]]] = None):
+                 randomize: Union[None, Mapping, Sequence[Optional[Mapping]]] = None,
+                 scripted: Optional[Mapping[str, Union[str, int]]] = None):
         params = _make_params(max_step_count, time_step, physical_params, auto_reset=1, seed=int(seed),
                               stale_shape_cache=int(stale_shape_cache))
         self._params = params
@@ -303,7 +310,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._setup_common(map, self._cmap, params)
             self._w = CatWorlds(self._cmap, num_envs, device=device, gid0=gid0, params=params, want_f32=True, want_critic=True,
                                 want_final=final_observations, swappable_maps=swappable_maps,
-                                want_episode_stats=episode_statistics, param_ranges=randomize)
+                                want_episode_stats=episode_statistics, param_ranges=randomize,
+                                want_scripts=scripted is not None)
         else:
             self.maps = list(map)
             n = len(self.maps)
@@ -321,7 +329,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
             self._setup_common(self.maps[0], self._cmap, params, window=window)
             self._w = CatWorlds(self._cmaps, counts, device=device, gid0=gid0, params=params, want_f32=True,
                                 want_critic=True, want_final=final_observations, swappable_maps=swappable_maps,
-                                want_episode_stats=episode_statistics, param_ranges=randomize)
+                                want_episode_stats=episode_statistics, param_ranges=randomize,
+                                want_scripts=scripted is not None)
             num_envs = sum(counts)
         self._cell = cell
         self.map_names = [c.name for c in self._cmaps]
@@ -334,6 +343,10 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         self.max_step_count = max_step_count
         self.state_spaces = {a: self.shared_observation_spaces for a in self.possible_agents}
         self.state_dim = self._w.S
+        # the slot of a scripted agent a mapping leaves out of step(): the kernel never reads it
+        self._script_zero = torch.zeros(self.num_envs, dtype=torch.int64, device=self.device)
+        if scripted:
+            self.set_scripted(scripted)
 
     @property
     def worlds(self) -> CatWorlds:
@@ -396,7 +409,8 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
 
     def step(self, actions: Union[Mapping[str, torch.Tensor], torch.Tensor]):
         if isinstance(actions, Mapping):
-            acts = [actions[a].reshape(-1) for a in self.possible_agents]
+            acts = [actions[a].reshape(-1) if a in actions or a not in self.scripted_agents else self._script_zero
+                    for a in self.possible_agents]
             if all(t.dtype == torch.int64 and t.is_contiguous() and t.device == self.device for t in acts):
                 self._w.step(acts)
             else:
@@ -450,6 +464,22 @@ class BatchedCopsThievesEnv(_EnvCommon, _ParallelEnvBase):
         from . import world_params as wparams
         for slot, spec in enumerate(wparams.per_slot(randomize, len(self._cmaps))):
             self._w.set_param_ranges(slot, draw=spec is not None, **(spec or {}))
+
+    def set_scripted(self, spec: Mapping[str, Union[str, int]], mask=None) -> None:
+        """Set agents' modes, ``{"thief_0": "evade", "cop_0": "none"}``, in the worlds of the (N,) bool ``mask`` (all if
+        None); agents not named keep theirs.  Checked before anything is written, then written in place (a captured
+        graph stays valid).  Needs ``scripted`` at creation."""
+        from . import scripts
+        self._w.set_scripts(scripts.agent_modes(spec, self.possible_agents), mask)
+
+    @property
+    def scripted_agents(self) -> List[str]:
+        """The agents scripted in every world (from the host mirror of the modes: no device sync)."""
+        return [a for i, a in enumerate(self.possible_agents) if self._w.scripted_in(i) == "all"]
+
+    def scripted_in(self, agent: str) -> str:
+        """``"all"``, ``"none"`` or ``"some"``: in which worlds ``agent`` is scripted."""
+        return self._w.scripted_in(self.possible_agents.index(agent))
 
     def render(self, world: int = 0):
         """``rgb_array`` of one world, drawn on that world's own map (numpy (W, H, 3) uint8 of that map's window):

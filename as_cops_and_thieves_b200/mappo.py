@@ -273,13 +273,26 @@ def build_models(agents: Iterable[str], n_obs: int, n_state: int, kind: str, dev
 
 # ------------------------------------------------------------------ the learner
 class MAPPOLearner:
-    """Collect ``rollouts`` lockstep steps with the current policies, then one MAPPO update per agent."""
+    """Collect ``rollouts`` lockstep steps with the current policies, then one MAPPO update per agent.
+
+    Agents that the environment scripts in every world (``BatchedCopsThievesEnv(scripted=...)``) are played by the step
+    kernel's controllers: the learner gives them no models, no memory and no update, and ``agents`` lists only the
+    learned ones.  An agent scripted in some worlds but not all is refused, and so is a rollout after the set of scripted
+    agents has changed."""
 
     def __init__(self, env, cfg: Optional[MAPPOConfig] = None, seed: int = 0):
         self.env = env
         self.cfg = cfg or MAPPOConfig()
         self.device = env.device
-        self.agents: List[str] = list(env.possible_agents)
+        self._scripts = self._script_signature()
+        partial = [a for a, where in zip(env.possible_agents, self._scripts) if where == "some"]
+        if partial:
+            raise ValueError(f"agents {partial} are scripted in some worlds but not all: a learner needs each agent "
+                             "either scripted everywhere or nowhere")
+        self.scripted_agents: List[str] = [a for a, where in zip(env.possible_agents, self._scripts) if where == "all"]
+        self.agents: List[str] = [a for a in env.possible_agents if a not in self.scripted_agents]
+        if not self.agents:
+            raise ValueError("every agent is scripted: there is nothing to learn")
         self.n_obs = 2 * env.worlds.R
         self.n_state = env.state_dim
         if self.cfg.rollouts % self.cfg.sequence_length:
@@ -334,6 +347,11 @@ class MAPPOLearner:
         self._graphs: Dict[bool, object] = {}
         self.timestep = 0
         self.env_seconds = 0.0
+
+    def _script_signature(self) -> Tuple[str, ...]:
+        """Per agent, where the environment scripts it ("all", "none" or "some"), from the host mirror of the modes."""
+        where = getattr(self.env, "scripted_in", None)
+        return tuple(where(a) if where is not None else "none" for a in self.env.possible_agents)
 
     # -------------------------------------------------------------- parameters / checkpoints
     def parameters(self, agent: str) -> List[nn.Parameter]:
@@ -496,6 +514,9 @@ class MAPPOLearner:
         replay ONE CUDA graph holding every network launch and every environment-step launch of the rollout,
         so the host issues a single graph launch instead of ~10^4 kernel launches."""
         env, cfg = self.env, self.cfg
+        if self._script_signature() != self._scripts:
+            raise RuntimeError("the environment's scripted agents changed since this learner was built (it learns "
+                               f"{self.agents}); build a new learner for the new set")
         if self._obs is None:
             self._obs, _ = env.reset()
         uniform = self.timestep < cfg.random_timesteps

@@ -187,6 +187,35 @@ def evaluate_agents(env, learner, n_episodes: int = 5, cop_prefix: str = "cop", 
     return int(cop_wins.item()) / total, int(thief_wins.item()) / total, per_map
 
 
+def evaluate_vs_scripted(env, learner, role_prefix: str, controller: str = "evade", n_episodes: int = 5,
+                         by_map: bool = False, greedy: bool = False, cop_prefix: str = "cop", thief_prefix: str = "thief"):
+    """Win rate of the learned role ``role_prefix`` against the step kernel's ``controller`` (``"evade"``, ``"chase"``
+    or ``"random"``) playing every agent of the other role: a yardstick that does not move when the learner's own
+    opponents change.  Needs ``BatchedCopsThievesEnv(scripted=...)``; the agents of ``role_prefix`` must have models in
+    the learner.  The other role is scripted in every world, ``evaluate_agents`` runs (the kernel ignores the learner's
+    actions for scripted agents), and the modes found are restored.  Returns the rate, or with ``by_map``
+    ``(rate, [{"map", "rate", "episodes"} per map])``."""
+    if role_prefix not in (cop_prefix, thief_prefix):
+        raise ValueError(f"role_prefix must be {cop_prefix!r} or {thief_prefix!r}, got {role_prefix!r}")
+    learned = [a for a in env.possible_agents if a.startswith(role_prefix)]
+    missing = [a for a in learned if a not in learner.agents]
+    if missing:
+        raise ValueError(f"the learner has no models for {missing}")
+    other = [a for a in env.possible_agents if not a.startswith(role_prefix)]
+    w = env.worlds
+    saved = w.script_modes.clone()
+    try:
+        env.set_scripted({a: controller for a in other})
+        out = evaluate_agents(env, learner, n_episodes, cop_prefix, thief_prefix, greedy=greedy, by_map=by_map)
+    finally:
+        w.set_script_table(saved)
+    key = "cop" if role_prefix == cop_prefix else "thief"
+    rate = out[0] if key == "cop" else out[1]
+    if not by_map:
+        return rate
+    return rate, [{"map": m["map"], "rate": m[key], "episodes": m["episodes"]} for m in out[2]]
+
+
 def evaluate_agent(env, learner, learned_role_prefix: str, opponent_role_prefix: str, opponent_role_archive_path: Path,
                    training_config=TrainingConfig, num_additional_opponents_to_evaluate: int = 5,
                    rng: Optional[random.Random] = None) -> Dict[str, Tuple[float, float]]:

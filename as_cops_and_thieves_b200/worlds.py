@@ -14,8 +14,8 @@ from typing import Dict, Mapping, Optional, Sequence, Tuple, Union
 import numpy as np
 import torch
 
-from . import _lib, episodes, world_params as wparams
-from ._lib import (CatEnvInfo, CatEpisodeStatsIO, CatWorldParamsIO, CatMapDesc, CatParams, CatRecordLayout, CatStateView, CatStepIO,
+from . import _lib, episodes, scripts as cscripts, world_params as wparams
+from ._lib import (CatEnvInfo, CatEpisodeStatsIO, CatScriptIO, CatWorldParamsIO, CatMapDesc, CatParams, CatRecordLayout, CatStateView, CatStepIO,
                    CAT_WALL_SLOTS)
 from .maps import CompiledMap
 from .params import EnvParams
@@ -111,7 +111,8 @@ class CatWorlds:
                  want_critic: bool = False, want_bf16: bool = False, want_final: bool = False,
                  swappable_maps: bool = False, map_blob_capacity: Optional[int] = None,
                  want_episode_stats: bool = False, want_world_params: bool = False,
-                 param_ranges: Union[None, Mapping, Sequence[Optional[Mapping]]] = None, **overrides):
+                 param_ranges: Union[None, Mapping, Sequence[Optional[Mapping]]] = None,
+                 want_scripts: bool = False, scripts: Optional[Mapping[int, Union[str, int]]] = None, **overrides):
         """``pinned_outputs=True`` places every output tensor in mapped pinned HOST memory: the kernel stores its
         results there directly and the host reads them (``tensor.numpy()``) after one stream synchronisation —
         the layout for callers that consume every step on the CPU, like the single-world PettingZoo face.
@@ -150,7 +151,13 @@ class CatWorlds:
         from a device table (``cat_env_attach_world_params``), filled with this environment's values for both teams;
         ``world_params()`` gives named views of it and ``set_world_params`` writes it.  ``param_ranges`` (implies
         ``want_world_params``): a randomisation spec for every map slot, or one per slot (``set_param_ranges``), from
-        which every re-spawn of a world draws its next entry.  A step stays one launch; it runs the full-output kernel."""
+        which every re-spawn of a world draws its next entry.  A step stays one launch; it runs the full-output kernel.
+
+        ``want_scripts``: built-in controllers can act for chosen agents inside the step kernel (``cat_env_attach_scripts``,
+        ``scripts.py``): ``script_modes`` (N, A) uint8 holds each agent's mode (0 none, 1 random, 2 chase, 3 evade),
+        written with ``set_scripts``, and ``script_decisions`` (N, A) uint8 what the controllers decided from the last
+        emitted observation.  ``scripts`` (implies ``want_scripts``): initial ``{agent index: mode}`` for every world.
+        A step stays one launch; it runs the full-output kernel."""
         if map_blob_capacity is not None and (int(map_blob_capacity) < 16 or int(map_blob_capacity) % 16):
             # the step kernel stages a blob with one bulk copy whose size must be a multiple of 16 bytes
             raise ValueError(f"map_blob_capacity must be a positive multiple of 16, got {map_blob_capacity}")
@@ -283,6 +290,16 @@ class CatWorlds:
             self._upload_ranges()
             wio = CatWorldParamsIO(self._wp.data_ptr(), self._wp_ranges.data_ptr())
             _lib.check(self.L.cat_env_attach_world_params(self._h, C.byref(wio)), "cat_env_attach_world_params")
+        self.want_scripts = bool(want_scripts) or scripts is not None
+        self._script_mode = self._script_dec = self._script_mode_host = None
+        if self.want_scripts:
+            self._script_mode = torch.zeros((N, A), dtype=torch.uint8, device=dev)
+            self._script_dec = torch.zeros((N, A), dtype=torch.uint8, device=dev)
+            self._script_mode_host = np.zeros((N, A), np.uint8)   # mirror of the modes, kept by set_scripts
+            if scripts:
+                self.set_scripts(scripts)
+            scio = CatScriptIO(self._script_mode.data_ptr(), self._script_dec.data_ptr())
+            _lib.check(self.L.cat_env_attach_scripts(self._h, C.byref(scio)), "cat_env_attach_scripts")
         _lib.check(self.L.cat_env_init_state(self._h, self.state.data_ptr(), self._stream()), "cat_env_init_state")
 
     # ------------------------------------------------------------------ plumbing
@@ -675,6 +692,8 @@ class CatWorlds:
         if self._wp is not None:
             sd["world_params"] = self._wp.clone()
             sd["param_ranges"] = self._wp_ranges.clone()
+        if self._script_mode is not None:
+            sd["script_mode"] = self._script_mode.clone()
         return sd
 
     def load_state_dict(self, sd: Mapping[str, torch.Tensor]) -> None:
@@ -686,6 +705,8 @@ class CatWorlds:
             self._wp.copy_(sd["world_params"].to(self.device))
             self._ranges_host = sd["param_ranges"].cpu().numpy().copy().view(wparams.RANGES_DTYPE).reshape(-1)
             self._upload_ranges()
+        if self._script_mode is not None and "script_mode" in sd:
+            self.set_script_table(sd["script_mode"])
 
     # ------------------------------------------------------------------ per-world parameters
     def world_params(self) -> Dict[str, torch.Tensor]:
@@ -741,3 +762,65 @@ class CatWorlds:
     def _upload_ranges(self) -> None:
         words = torch.from_numpy(self._ranges_host.view(np.int32).reshape(len(self.cmaps), wparams.RANGE_WORDS).copy())
         self._wp_ranges.copy_(words)
+
+    # ------------------------------------------------------------------ scripted agents
+    def _require_scripts(self) -> None:
+        if self._script_mode is None:
+            raise _lib.CatError("scripted agents are off (want_scripts=False)")
+
+    @property
+    def script_modes(self) -> torch.Tensor:
+        """(N, A) uint8 device table of every agent's mode, read by each step (``scripts.MODES``).  Write it with
+        ``set_scripts``, which checks the values and keeps the host mirror that ``scripted_in`` answers from."""
+        self._require_scripts()
+        return self._script_mode
+
+    @property
+    def script_decisions(self) -> torch.Tensor:
+        """(N, A) uint8 device table: what the random, chase and evade controllers decided (bits 0-1, 2-3, 4-5) from
+        the observation the last step or reset emitted.  Written by the kernel."""
+        self._require_scripts()
+        return self._script_dec
+
+    def scripted_actions(self) -> torch.Tensor:
+        """(N, A) int64 next actions of the scripted agents (``scripts.decode``; -1 where an agent is not scripted)."""
+        self._require_scripts()
+        return cscripts.decode(self._script_dec, self._script_mode)
+
+    def set_scripts(self, modes: Mapping[int, Union[str, int]], mask=None) -> None:
+        """Set the mode of agents ``{agent index: mode}`` (a name of ``scripts.MODES`` or its code) in the worlds of the
+        (N,) bool ``mask`` (all if None).  Everything is checked before anything is written; the table is written in
+        place, so a captured graph stays valid, and the next step acts on the new modes."""
+        self._require_scripts()
+        codes = {}
+        for a, mode in modes.items():
+            if isinstance(a, bool) or not isinstance(a, (int, np.integer)) or not 0 <= int(a) < self.A:
+                raise ValueError(f"agent index must be in 0..{self.A - 1}, got {a!r}")
+            codes[int(a)] = cscripts.mode_code(mode)
+        sel = None if mask is None else cscripts.check_mask(mask, self.n_worlds)
+        for a, code in codes.items():
+            if sel is None:
+                self._script_mode[:, a] = code
+                self._script_mode_host[:, a] = code
+            else:
+                self._script_mode[:, a].masked_fill_(sel.to(self.device), code)
+                self._script_mode_host[sel.numpy(), a] = code
+
+    def set_script_table(self, modes: torch.Tensor) -> None:
+        """Replace the whole (N, A) mode table (codes 0..3, checked), in place, e.g. to restore a saved copy."""
+        self._require_scripts()
+        modes = torch.as_tensor(modes)
+        cscripts.check_modes(modes)
+        if tuple(modes.shape) != (self.n_worlds, self.A):
+            raise ValueError(f"script modes must be ({self.n_worlds}, {self.A}), got {tuple(modes.shape)}")
+        host = modes.to(torch.uint8).cpu()
+        self._script_mode.copy_(host.to(self.device))
+        self._script_mode_host[:] = host.numpy()
+
+    def scripted_in(self, agent: int) -> str:
+        """``"all"``, ``"none"`` or ``"some"``: in which worlds agent ``agent`` is scripted, from the host mirror of the
+        modes (no device sync).  ``"none"`` without scripts."""
+        if self._script_mode_host is None:
+            return "none"
+        col = self._script_mode_host[:, int(agent)] != 0
+        return "all" if col.all() else "some" if col.any() else "none"

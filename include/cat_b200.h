@@ -227,6 +227,50 @@ typedef struct {
   const CatWorldParamRanges* ranges;   /* [n_maps] one entry per map slot; optional */
 } CatWorldParamsIO;
 
+/* SCRIPTED AGENTS (cat_env_attach_scripts): built-in controllers that act for chosen agents inside the step kernel, as
+ * fixed opponents and as a yardstick that does not move when the learner changes.
+ *
+ * Modes.  mode[w][a] selects what agent a of world w does at a step:
+ *   CAT_SCRIPT_NONE    the caller's action, exactly as without scripts;
+ *   CAT_SCRIPT_RANDOM  a uniform draw (cat_script_random, cat_philox.h);
+ *   CAT_SCRIPT_CHASE   move along the axis nearest to the closest opponent the agent sees, otherwise random;
+ *   CAT_SCRIPT_EVADE   move away from the closest opponent it sees, towards open space, otherwise random.
+ * Values above 3 are undefined: the kernel does not validate the table (the Python setters do).
+ *
+ * Decisions.  A policy picks its next action from the observation the last launch emitted, and a controller sees
+ * exactly that observation: the launch that emits a world's observation also writes, into decisions[w][a], the action
+ * each controller would take next, random in bits 0-1, chase in bits 2-3 and evade in bits 4-5.  All three are stored,
+ * so a mode may change between steps (in place, graph-safe) and the next step still acts on the latest observation.
+ * A step uses (decisions[w][a] >> 2 (mode - 1)) & 3 for every agent whose mode is non-zero and does not read the
+ * caller's action for it.
+ *   - Step launches (every cat_env_step_host chunk included) and reset launches (so the resets after cat_env_set_map)
+ *     write the decisions of every world whose observation they emit, from that observation: a world that auto-resets
+ *     decides from its re-spawned observation; final outputs are never used.
+ *   - cat_env_init_state zeroes every entry.  cat_env_observe and cat_env_set_state leave them alone (observing into
+ *     another buffer, as the renderer does, must not change what the next step does).
+ *
+ * Controllers.  Agent a reads only its own observation, the f16 distance bits d[i] and types ty[i] of its rays
+ * i < R.  Its target type is THIEF (2) for a cop and COP (1) for a thief.  Integer rules only:
+ *   quadrant of ray i   q(i) = ((8 i + R) / (2 R)) mod 4, i.e. round(4 i / R) with halves going up;
+ *   action of quadrant  ACT = {2 (+x), 1 (+y), 0 (-x), 3 (-y)};  axis ray of quadrant q: j(q) = ((q R + 2) / 4) mod R;
+ *   seen                some ray has ty[i] == target; i* = the ray with the smallest (d[i], i), d compared as u16 bits;
+ *   random              cat_script_random(seed, gid, episode, step_count, a), episode and step_count being the world's
+ *                       values when the observation is emitted (0 and the new episode right after a re-spawn);
+ *   chase               seen: ACT[q(i*)]; otherwise random;
+ *   evade               seen: with q* = q(i*), score the quadrants (q*+2, q*+1, q*+3) mod 4 in that order by
+ *                       c(q) = (ty[j(q)] == target ? 0 : d[j(q)]) and take ACT of the first with the strictly largest
+ *                       score; otherwise random. */
+#define CAT_SCRIPT_NONE 0
+#define CAT_SCRIPT_RANDOM 1
+#define CAT_SCRIPT_CHASE 2
+#define CAT_SCRIPT_EVADE 3
+
+/* caller-owned device pointers, both required */
+typedef struct {
+  const uint8_t* mode;          /* u8 [N][A] CAT_SCRIPT_* per agent */
+  uint8_t* decisions;           /* u8 [N][A] the controllers' next actions, written by the kernel */
+} CatScriptIO;
+
 /* byte offsets inside one world's output record (cat_env_record_layout / cat_env_packed_record_layout) */
 typedef struct {
   int32_t bytes;        /* record size = default world stride (multiple of 16) */
@@ -367,6 +411,10 @@ int cat_env_attach_episode_stats(CatEnv* env, const CatEpisodeStatsIO* io);
  * CAT_ERR_INVALID for a null env, a missing params pointer or a pointer that is not 4-byte aligned; nothing is stored
  * then.  The table's contents are not checked. */
 int cat_env_attach_world_params(CatEnv* env, const CatWorldParamsIO* io);
+/* Attach scripted agents (CatScriptIO above), or detach them with io = NULL.  Host only, no CUDA call, like
+ * cat_env_attach_episode_stats: every later launch carries the pointers and runs the full-output kernel.
+ * CAT_ERR_INVALID for a null env or a missing pointer; nothing is stored then.  The modes are not checked. */
+int cat_env_attach_scripts(CatEnv* env, const CatScriptIO* io);
 /* parity-test access to the hidden state */
 int cat_env_get_state(CatEnv* env, const void* state_dev, const CatStateView* view, void* stream);
 int cat_env_set_state(CatEnv* env, void* state_dev, const CatStateView* view, void* stream);

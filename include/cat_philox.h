@@ -89,4 +89,16 @@ CAT_HD int32_t cat_param_int(uint32_t word, int32_t lo, int32_t hi) {
   return lo + (int32_t)(((uint64_t)word * (uint64_t)(uint32_t)(hi - lo + 1)) >> 32);
 }
 
+/* The random controller's next action (CAT_SCRIPT_RANDOM, cat_b200.h) for agent a (< 8) of a world whose observation
+ * is emitted at (episode, step_count):
+ *   counter = (gid_lo, gid_hi, episode, 0x80000000 | (step_count & 0x0FFFFFFF) << 3 | a)  -> mulhi(word 0, 4)
+ * Bit 31 keeps this stream apart from the spawn stream (agent << 8 | try, below 0x800) and from the parameter draws
+ * (0xFF00 | j), so attaching scripts moves neither spawns nor parameter draws. */
+CAT_HD uint32_t cat_script_random(uint64_t seed, uint64_t gid, uint32_t episode, uint32_t step_count, uint32_t a) {
+  cat_u32x4 r = cat_philox4x32_10((uint32_t)gid, (uint32_t)(gid >> 32), episode,
+                                  0x80000000u | (step_count & 0x0FFFFFFFu) << 3 | a,
+                                  (uint32_t)seed, (uint32_t)(seed >> 32));
+  return (uint32_t)(((uint64_t)r.v[0] * 4u) >> 32);
+}
+
 #endif /* CAT_PHILOX_H */

@@ -8,11 +8,14 @@ all-reduced over NCCL per minibatch.
     python tools/train_selfplay.py --map squarinth --procedural 2 --swap-every 4     # + 2 slots of fresh mazes
     python tools/train_selfplay.py --map squarinth,agh-map --episode-stats            # + episode returns / lengths
     python tools/train_selfplay.py --episode-stats --randomize "max_speed.thief=125:175,termination_radius=15:25"
+    python tools/train_selfplay.py --map squarinth --scripted thief_0=evade --eval-scripted 2   # cops vs a scripted thief
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_selfplay.py ...
 
 Prints one JSON line per self-play iteration (rank 0): environment agent-steps/s inside training, GAE / update /
 all-reduce milliseconds per update, win rates; with --episode-stats also "episodes": what the training episodes of the
-iteration added up to (all ranks), overall and per map slot (the evaluation's episodes are not counted).
+iteration added up to (all ranks), overall and per map slot (the evaluation's episodes are not counted); with
+--eval-scripted also "eval_vs_scripted": the cops' win rate against an evading thief and the thief's against chasing
+cops (the step kernel's controllers), overall and per map, on this rank's worlds.
 """
 import argparse
 import json
@@ -25,7 +28,7 @@ import torch
 
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
-from as_cops_and_thieves_b200 import episodes, selfplay, world_params  # noqa: E402
+from as_cops_and_thieves_b200 import episodes, scripts, selfplay, world_params  # noqa: E402
 from as_cops_and_thieves_b200.env import BatchedCopsThievesEnv  # noqa: E402
 from as_cops_and_thieves_b200.mappo import MAPPOConfig, MAPPOLearner  # noqa: E402
 from as_cops_and_thieves_b200.maps import free_space_regions, generate_maze, load_named_map  # noqa: E402
@@ -61,8 +64,15 @@ def main():
     ap.add_argument("--randomize", default="",
                     help="domain randomisation drawn at every re-spawn, e.g. 'max_speed.thief=125:175,termination_radius="
                          "15:25,max_step_count=300:500' (field[.cop|.thief]=lo:hi, or one number to pin it)")
+    ap.add_argument("--scripted", default="",
+                    help="agents played by the step kernel's controllers, e.g. 'thief_0=evade' (random, chase, evade): "
+                         "the learner trains the remaining agents against them")
+    ap.add_argument("--eval-scripted", type=int, default=0, metavar="K",
+                    help="after each iteration, K episodes per world of the cops against an evading thief and of the "
+                         "thief against chasing cops (a role the learner does not train is skipped)")
     a = ap.parse_args()
     randomize = world_params.parse_cli(a.randomize) if a.randomize else None
+    scripted = scripts.parse_spec(a.scripted) if a.scripted or a.eval_scripted > 0 else None
 
     rank, local_rank, world_size = dist_env()
     dev = torch.device(f"cuda:{local_rank}")
@@ -87,11 +97,13 @@ def main():
     if len(maps) == 1:
         env = BatchedCopsThievesEnv(maps[0], n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
                                     spawn_override=spawn[0], final_observations=a.time_limit_bootstrap,
-                                    episode_statistics=a.episode_stats, randomize=randomize)
+                                    episode_statistics=a.episode_stats, randomize=randomize,
+                                    scripted=scripted)
     else:
         env = BatchedCopsThievesEnv(maps, n_local, device=dev, seed=0, gid0=gid0, max_step_count=a.max_step_count,
                                     spawn_override=spawn, final_observations=a.time_limit_bootstrap,
-                                    swappable_maps=swappable, episode_statistics=a.episode_stats, randomize=randomize)
+                                    swappable_maps=swappable, episode_statistics=a.episode_stats, randomize=randomize,
+                                    scripted=scripted)
     # the reference's schedule (10 000 random / 15 000 before learning / 15 000 frozen policy) counts steps of ONE
     # environment; with thousands of lockstep worlds the same number of TRANSITIONS is reached in a few steps, so the
     # driver scales the durations by the world count unless told otherwise
@@ -120,7 +132,7 @@ def main():
             import torch.distributed as dist
             tot = episodes.allreduce_totals(tot, dist.group.WORLD)
         ep_parts.clear()
-        out = episodes.summarize_maps(tot, learner.agents, [name for _, name in keys], by_map=True)
+        out = episodes.summarize_maps(tot, env.possible_agents, [name for _, name in keys], by_map=True)
         for entry, (slot, _) in zip(out["maps"], keys):
             entry["slot"] = slot
         return out
@@ -159,13 +171,24 @@ def main():
         if a.episode_stats:
             env.worlds.episode_totals_raw(reset=True)        # the evaluation's episodes
             extra["episodes"] = episode_report()
+        if a.eval_scripted > 0:
+            vs = {}
+            mixed = len(env.map_names) > 1
+            for key, role, controller in (("cop_vs_evade", tc.cop_role_prefix, "evade"),
+                                          ("thief_vs_chase", tc.thief_role_prefix, "chase")):
+                if not all(ag in learner.agents for ag in env.possible_agents if ag.startswith(role)):
+                    vs[key] = None       # the role is scripted: the learner has no policy for it
+                    continue
+                r = selfplay.evaluate_vs_scripted(env, learner, role, controller, n_episodes=a.eval_scripted, by_map=mixed)
+                vs[key] = r if not mixed else {"overall": r[0], "maps": r[1]}
+            extra["eval_vs_scripted"] = vs
         if rank == 0:
             u = max(agg["updates"], 1)
             print(json.dumps({
                 "iteration": it, "n_gpus": world_size, "map": a.map, "worlds_per_gpu": a.worlds, "model": a.model,
                 "parameters": learner.n_parameters(), "rollouts": a.rollouts, "lockstep_steps": steps,
-                "rollout_agent_steps_per_s": a.worlds * world_size * len(learner.agents) * steps / max(learner.env_seconds - env_s0, 1e-9),
-                "train_agent_steps_per_s": a.worlds * world_size * len(learner.agents) * steps / train_s,
+                "rollout_agent_steps_per_s": a.worlds * world_size * len(env.possible_agents) * steps / max(learner.env_seconds - env_s0, 1e-9),
+                "train_agent_steps_per_s": a.worlds * world_size * len(env.possible_agents) * steps / train_s,
                 "gae_ms_per_update": agg["gae_ms"] / u, "ppo_ms_per_update": agg["update_ms"] / u,
                 "allreduce_ms_per_update": agg["allreduce_ms"] / u,
                 "eval_vs_archive": {"cop_trained": res_c, "thief_trained": res_t}, **extra}), flush=True)
